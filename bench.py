@@ -4,6 +4,7 @@ QM9-shape synthetic batches) — see DESIGN.md §Measurement for every definitio
 
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = one training step over one batch of 1024 synthetic QM9-shaped molecules per GPU
 (index build + forward + backward of the energy MSE loss + gradient all-reduce for N > 1 + fused
@@ -318,15 +319,22 @@ def run_ours(args):
         h2d = sum(v.numel() * v.element_size() for v in host.values() if torch.is_tensor(v))
         get_batch = lambda: (GraphClone(resident), y_dev)  # noqa: E731
 
+    # --dump-outputs: the outputs of the latest step, detached (a reference to the graph would keep it alive)
+    last = {} if args.dump_outputs else None
+
     def step(batch, y):
         bucket.zero()
         out = model(batch)
+        if last is not None:
+            last["out"] = tuple(t.detach() for t in out) if isinstance(out, tuple) else out.detach()
         if isinstance(out, tuple):  # (energy, forces): the forces are evaluated, the loss is on the energy
             out = out[0]
         loss = torch.nn.functional.mse_loss(out, y)
         loss.backward()
         bucket.all_reduce_mean()
         opt.step()
+        if last is not None:
+            last["loss"] = loss.detach()
         return loss
 
     def barrier():
@@ -362,6 +370,8 @@ def run_ours(args):
     l0 = _lib.launch_count()
     ms_dev = timed(lambda: step(*get_batch()), args.steps)
     launches = (_lib.launch_count() - l0) // max(args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, last["out"], last["loss"])
     # CPU time to enqueue ONE step into an empty stream (median of 5): if it approaches ms_per_step the host is the limit
     hs = []
     for _ in range(5):
@@ -485,6 +495,33 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS_BYTES = 16 << 20  # per model output: energies and forces together stay well inside 64 MB with the parameters
+
+
+def dump_outputs(path, model, out, loss):
+    """Write what one training step computed as float32 DIR/<name>.npy: the model outputs (`energy`, and `forces` for
+    the crystal workload), the `loss`, every parameter's gradient (`grad.<name>`), every parameter after the optimizer
+    step (`param.<name>`) and the floating-point buffers the step updates (`buffer.<name>`, BatchNorm statistics).  A
+    model output larger than DUMP_ROWS_BYTES is replaced by the same rows every run (sorted, drawn with seed 0), so that
+    two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+
+    outputs = dict(zip(("energy", "forces"), out)) if isinstance(out, tuple) else {"energy": out}
+    arrays = {"loss": loss}
+    for name, t in outputs.items():
+        rows = max(1, DUMP_ROWS_BYTES // (4 * max(1, t[0].numel())))
+        if t.shape[0] > rows:
+            keep = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values
+            t = t[keep.to(t.device)]
+        arrays[name] = t
+    arrays.update((f"grad.{n}", p.grad) for n, p in model.named_parameters() if p.grad is not None)
+    arrays.update((f"param.{n}", p) for n, p in model.named_parameters())
+    arrays.update((f"buffer.{n}", b) for n, b in model.named_buffers() if b.is_floating_point())
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 class GraphClone(dict):
     """Fresh shallow copy of the resident batch per step (forward writes side-effect keys into it)."""
 
@@ -569,7 +606,13 @@ def main():
                     help="also time the oracle port with PyTorch eager on the GPU at these batch sizes and quote the best "
                          "(empty string = skip)")
     ap.add_argument("--profile-host", action="store_true", help="cProfile of 5 steps (host side) to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -9,7 +9,7 @@ Only `tests/`, `__graft_entry__.smoke()` and `bench.py`'s `cpu_baseline` / `--im
 may import this module, and only as the checker / the timed CPU baseline.  `lcaonet_b200/` never
 imports it.
 
-Parity pinning (see tests/test_oracle_vs_reference.py, tests/test_oracle_golden.py):
+Parity pinning (see tests/test_oracle_golden.py):
   * against the UNMODIFIED reference imported in the build container through `oracle/_shims`
     (all interaction / embedding / output numerics, triplet indices) -> committed golden vectors
     in tests/golden/ made by oracle/make_golden.py;

@@ -85,9 +85,11 @@ def _cases():
 
 @pytest.mark.parametrize("idx", range(7))
 def test_wrapper_through_emulator(idx, monkeypatch):
+    # imported before the emulator is installed: the module binds `call`, `require_cuda` and `stream_ptr` at import, and
+    # bound to the emulator's stand-ins they would outlive this test and route the CUDA tests below to the emulator
+    from lcaonet_b200 import neighbors
     from tests import cpu_abi
     cpu_abi.install(monkeypatch)
-    from lcaonet_b200 import neighbors
     monkeypatch.setattr(neighbors, "require_cuda", lambda *a: None)
     monkeypatch.setattr(neighbors, "stream_ptr", lambda: 0)
     monkeypatch.setattr(neighbors, "call", lambda name, *a: cpu_abi._TABLE[name](*a))
