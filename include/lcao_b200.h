@@ -138,6 +138,22 @@ int lcao_geom_basis_bwd(const float* dist, const float* unit, const float* drb, 
                         const float* d_unit, const float* d_rb, int64_t E, int64_t N, int32_t O,
                         const int32_t* in_ptr, const int32_t* in_edge, const int32_t* out_ptr,
                         const int32_t* out_edge, float* dvec_scratch, float* d_pos, void* stream);
+/* Cell derivatives of the energy, per graph g, from the dvec (E,3) = d E / d vec that lcao_geom_basis_bwd wrote, with
+ * vec_e = pos[t] - pos[s] + shift_e . L_g (row vectors; the rows of L_g = lattice[g] are the cell vectors):
+ *   d_lattice[g][i][j] = sum_{e in g} shift_e[i] dvec_e[j]              d E / d L_g          (B,3,3), nullable
+ *   virial[g][i][j]    = sum_{e in g} vec_e[i]   dvec_e[j]              d E / d eps_g        (B,3,3), nullable
+ * where eps_g is a strain acting as pos' = pos (I + eps), L' = L (I + eps); stress = virial / |det L_g|.  An edge belongs
+ * to the graph of its source.  vec is recomputed in FP64 from pos / shift / lattice / batch exactly as the forward forms
+ * it; both sums are accumulated in FP64 and rounded once, without atomics (bitwise reproducible): per-chunk partials
+ * over the out-edges of LCAO_CELL_CHUNK nodes, then a per-graph sum in chunk order.  Graphs without nodes or edges get
+ * zeros.  (seg_ptr (B+1), seg_perm (N, nullable = identity)) lists the nodes of each graph (lcao_bucket_sort of batch);
+ * batch (N, nullable = all graph 0) selects the lattice row as in the forward.
+ * scratch: (N / LCAO_CELL_CHUNK + B) * 18 doubles.  The gradient w.r.t. edge_shift is not computed. */
+#define LCAO_CELL_CHUNK 128
+int lcao_geom_cell_bwd(const float* pos, const float* shift, const float* lattice, const int64_t* batch,
+                       const int32_t* dst32, const float* dvec, int64_t E, int64_t N, const int32_t* out_ptr,
+                       const int32_t* out_edge, const int32_t* seg_ptr, const int32_t* seg_perm, int64_t B,
+                       double* scratch, float* d_lattice, float* virial, void* stream);
 
 /* ---- orbital contraction (the einsum "ed,edh->eh" sites lcaonet.py:180-183,200-203) ----------- */
 /* B[e,l,:]  = sum_{o: l(o)=l} rb[e,o] * (A[e,o,:] + m[e,o] V[e,o,:])        l = 0..NL-1

@@ -20,6 +20,7 @@ ACT_NONE, ACT_SILU = 0, 1
 ACT = {"none": 0, "silu": 1, "shiftedsoftplus": 2, "softplus": 3, "relu": 4, "tanh": 5, "sigmoid": 6, "gelu": 7, "elu": 8,
        "leakyrelu": 9}
 GEMM_FP32, GEMM_TF32X3, GEMM_TF32 = 0, 1, 2
+CELL_CHUNK = 128  # LCAO_CELL_CHUNK: nodes per partial of lcao_geom_cell_bwd (its scratch is (N // 128 + B) * 18 doubles)
 
 
 class BasisSpec(C.Structure):
@@ -46,6 +47,7 @@ SIGNATURES = {
     "lcao_neighbor_fill": [_p, _p, _p, _p, _p, _p, _p, _i64, _i64, C.c_double, _i32, _p, _p, _p, _p],
     "lcao_geom_basis_fwd": [_p, _p, _p, _p, _p, _p, _i64, C.POINTER(BasisSpec), _p, _p, _p, _p, _p],
     "lcao_geom_basis_bwd": [_p, _p, _p, _p, _p, _p, _i64, _i64, _i32, _p, _p, _p, _p, _p, _p, _p],
+    "lcao_geom_cell_bwd": [_p, _p, _p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p, _i64, _p, _p, _p, _p],
     "lcao_coeff_contract_fwd": [_p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32, _p, _p],
     "lcao_coeff_contract_bwd": [_p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32, _p, _p, _p],
     "lcao_pair_contract_fwd": [_p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32, _p, _p, _p, _p],

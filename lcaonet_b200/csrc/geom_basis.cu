@@ -112,6 +112,109 @@ __global__ void k_geom_node_bwd(const float* __restrict__ dvec, const int32_t* _
   d_pos[idx] = acc;
 }
 
+// ---- cell derivatives: d E / d lattice and the virial, per graph (lcao_geom_cell_bwd).
+// A graph's nodes (seg_perm[seg_ptr[g] .. seg_ptr[g+1]), or that range itself when seg_perm is NULL) are cut into chunks of
+// LCAO_CELL_CHUNK; chunk j of graph g owns partial slot  seg_ptr[g] / LCAO_CELL_CHUNK + g + j.  These ranges are disjoint
+// (the slots of g end at or before the first slot of g + 1), their union lies in [0, N / LCAO_CELL_CHUNK + B), and a slot
+// finds its graph by a binary search over seg_ptr: no scan kernel, no atomics.
+constexpr int kCellWarps = 8;
+constexpr int kCellVals = 18;  // 9 of d E / d L, then 9 of the virial
+
+__device__ __forceinline__ int64_t cell_slot_base(const int32_t* seg_ptr, int g) {
+  return seg_ptr[g] / LCAO_CELL_CHUNK + g;
+}
+
+// Stage 1: CTA = one chunk; warp w takes the chunk's nodes w, w + 8, ...; lane l the out-edges l, l + 32, ... of each
+// node in out-CSR order.  Every lane accumulates shift (x) dvec and vec (x) dvec in FP64; the lanes are combined by a
+// fixed xor butterfly and the warps in warp order: the partial is a fixed function of the inputs (bitwise reproducible).
+// vec is recomputed in FP64 exactly as k_geom_basis_fwd forms it (not dist * unit: that would carry the FP32 rounding of
+// unit into the virial).
+__global__ void __launch_bounds__(kCellWarps * 32) k_geom_cell_partial(
+    const float* __restrict__ pos, const float* __restrict__ shift, const float* __restrict__ lattice,
+    const int64_t* __restrict__ batch, const int32_t* __restrict__ dst32, const float* __restrict__ dvec,
+    const int32_t* __restrict__ out_ptr, const int32_t* __restrict__ out_edge, const int32_t* __restrict__ seg_ptr,
+    const int32_t* __restrict__ seg_perm, int B, double* __restrict__ partial) {
+  pdl_trigger();  // (programmatic dependent launch: the next kernel may start its set-up; common.cuh)
+  pdl_wait();     // launched through launch_pdl: nothing of the stream's earlier work is touched before this
+  __shared__ double s_red[kCellWarps][kCellVals];
+  const int64_t slot = blockIdx.x;
+  int lo = 0, hi = B;  // the graph: last g with cell_slot_base(g) <= slot (strictly increasing in g)
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (cell_slot_base(seg_ptr, mid) <= slot) lo = mid; else hi = mid;
+  }
+  const int g = lo;
+  const int64_t j0 = seg_ptr[g] + (slot - cell_slot_base(seg_ptr, g)) * LCAO_CELL_CHUNK;
+  const int64_t j1 = min(j0 + LCAO_CELL_CHUNK, (int64_t)seg_ptr[g + 1]);
+  if (j0 >= j1) return;  // a slot no chunk owns: never read
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double acc[kCellVals];
+#pragma unroll
+  for (int k = 0; k < kCellVals; ++k) acc[k] = 0.0;
+  for (int64_t j = j0 + warp; j < j1; j += kCellWarps) {
+    const int32_t n = seg_perm ? seg_perm[j] : (int32_t)j;
+    const int32_t p0 = out_ptr[n], p1 = out_ptr[n + 1];
+    if (p0 >= p1) continue;
+    const float* L = lattice + 9 * (batch ? batch[n] : 0);
+    const double ps0 = pos[3 * n], ps1 = pos[3 * n + 1], ps2 = pos[3 * n + 2];
+    for (int32_t p = p0 + lane; p < p1; p += 32) {
+      const int64_t e = out_edge[p];
+      const int32_t t = dst32[e];
+      const double sh[3] = {shift[3 * e], shift[3 * e + 1], shift[3 * e + 2]};
+      const double ps[3] = {ps0, ps1, ps2};
+      const double dv[3] = {dvec[3 * e], dvec[3 * e + 1], dvec[3 * e + 2]};
+      double v[3];
+#pragma unroll
+      for (int c = 0; c < 3; ++c)
+        v[c] = ((double)pos[3 * t + c] - ps[c]) + (sh[0] * L[c] + sh[1] * L[3 + c] + sh[2] * L[6 + c]);
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          acc[3 * a + c] = fma(sh[a], dv[c], acc[3 * a + c]);
+          acc[9 + 3 * a + c] = fma(v[a], dv[c], acc[9 + 3 * a + c]);
+        }
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < kCellVals; ++k) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+  }
+  if (lane == 0) {
+#pragma unroll
+    for (int k = 0; k < kCellVals; ++k) s_red[warp][k] = acc[k];
+  }
+  __syncthreads();
+  if (threadIdx.x < kCellVals) {
+    double s = 0.0;
+#pragma unroll
+    for (int w = 0; w < kCellWarps; ++w) s += s_red[w][threadIdx.x];
+    partial[slot * kCellVals + threadIdx.x] = s;
+  }
+}
+
+// Stage 2: warp = graph; lane k < 18 adds component k of the graph's chunk partials in chunk order and rounds once.
+// Graphs without nodes or without edges get zeros.
+__global__ void __launch_bounds__(kCellWarps * 32) k_geom_cell_final(const int32_t* __restrict__ seg_ptr, int B,
+                                                                     const double* __restrict__ partial,
+                                                                     float* __restrict__ d_lattice,
+                                                                     float* __restrict__ virial) {
+  pdl_trigger();
+  pdl_wait();  // the partials come from the kernel before this one
+  const int g = blockIdx.x * kCellWarps + (threadIdx.x >> 5), k = threadIdx.x & 31;
+  if (g >= B || k >= kCellVals) return;
+  const int64_t base = cell_slot_base(seg_ptr, g);
+  const int64_t chunks = ((int64_t)seg_ptr[g + 1] - seg_ptr[g] + LCAO_CELL_CHUNK - 1) / LCAO_CELL_CHUNK;
+  double s = 0.0;
+  for (int64_t c = 0; c < chunks; ++c) s += partial[(base + c) * kCellVals + k];
+  if (k < 9) {
+    if (d_lattice) d_lattice[9 * (int64_t)g + k] = (float)s;
+  } else if (virial) {
+    virial[9 * (int64_t)g + k - 9] = (float)s;
+  }
+}
+
 }  // namespace
 
 extern "C" int lcao_geom_basis_fwd(const float* pos, const float* shift, const float* lattice, const int64_t* batch,
@@ -147,5 +250,25 @@ extern "C" int lcao_geom_basis_bwd(const float* dist, const float* unit, const f
     k_geom_node_bwd<<<(unsigned)ceil_div64(N * 3, 256), 256, 0, st>>>(dvec, in_ptr, in_edge, out_ptr, out_edge, N, d_pos);
     LCAO_LAUNCH_CHECK();
   }
+  return LCAO_OK;
+}
+
+extern "C" int lcao_geom_cell_bwd(const float* pos, const float* shift, const float* lattice, const int64_t* batch,
+                                  const int32_t* dst32, const float* dvec, int64_t E, int64_t N, const int32_t* out_ptr,
+                                  const int32_t* out_edge, const int32_t* seg_ptr, const int32_t* seg_perm, int64_t B,
+                                  double* scratch, float* d_lattice, float* virial, void* stream) {
+  if (B == 0 || (!d_lattice && !virial)) return LCAO_OK;
+  LCAO_REQUIRE(B > 0 && B < (1 << 30) && N >= 0 && N < ((int64_t)1 << 31), "lcao_geom_cell_bwd: bad sizes (N=%lld, B=%lld)",
+               (long long)N, (long long)B);
+  LCAO_REQUIRE(lattice && out_ptr && seg_ptr && scratch, "lcao_geom_cell_bwd: null buffer");
+  LCAO_REQUIRE(E == 0 || (pos && shift && dst32 && dvec && out_edge), "lcao_geom_cell_bwd: null edge buffer");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t slots = N / LCAO_CELL_CHUNK + B;
+  LCAO_CUDA(launch_pdl(k_geom_cell_partial, (unsigned)slots, kCellWarps * 32, 0, st, pos, shift, lattice, batch, dst32, dvec,
+                       out_ptr, out_edge, seg_ptr, seg_perm, (int)B, scratch));
+  LCAO_LAUNCH_CHECK();
+  LCAO_CUDA(launch_pdl(k_geom_cell_final, (unsigned)ceil_div64(B, kCellWarps), kCellWarps * 32, 0, st, seg_ptr, (int)B,
+                       (const double*)scratch, d_lattice, virial));
+  LCAO_LAUNCH_CHECK();
   return LCAO_OK;
 }

@@ -412,7 +412,7 @@ class LCAOOut(nn.Module):
                                                Dense(emb_size, emb_size // 2, True, weight_init), activation,
                                                Dense(emb_size // 2, 1, False, weight_init))
 
-    def forward(self, x, seg, gi, unit, pos):
+    def forward(self, x, seg, gi, unit, pos, strain=None, lattice=None):
         prop = ops.segment_reduce(_mlp(self.out_lin, x), *seg, mean=not self.is_extensive)
         if not self.regress_forces:
             return prop
@@ -437,10 +437,21 @@ class LCAOOut(nn.Module):
         # pass: the backward kernels skip every parameter gradient inside it (ops.positions_only).
         graph = self.training if self.force_training is None else bool(self.force_training)
         graph = graph and torch.is_grad_enabled()
+        if strain is None:
+            with ops.positions_only():
+                cols = [-torch.autograd.grad(prop[:, i].sum(), pos, create_graph=graph, retain_graph=True)[0]
+                        for i in range(self.out_size)]
+            return prop, (cols[0] if len(cols) == 1 else torch.stack(cols, dim=1).squeeze(1))
+        # stress (LCAONet.regress_stress): the same backward pass also yields d E / d strain = the virial W (ops.geom_basis)
         with ops.positions_only():
-            cols = [-torch.autograd.grad(prop[:, i].sum(), pos, create_graph=graph, retain_graph=True)[0]
-                    for i in range(self.out_size)]
-        return prop, (cols[0] if len(cols) == 1 else torch.stack(cols, dim=1).squeeze(1))
+            grads = [torch.autograd.grad(prop[:, i].sum(), [pos, strain], create_graph=graph, retain_graph=True)
+                     for i in range(self.out_size)]
+        cols = [-g[0] for g in grads]
+        L = lattice[: strain.shape[0]].double()
+        vol = (L[:, 0] * torch.linalg.cross(L[:, 1], L[:, 2], dim=-1)).sum(-1).abs().to(grads[0][1].dtype)
+        sig = [g[1] / vol.view(-1, 1, 1) for g in grads]
+        return (prop, (cols[0] if len(cols) == 1 else torch.stack(cols, dim=1).squeeze(1)),
+                (sig[0] if len(sig) == 1 else torch.stack(sig, dim=1)))
 
 
 class PostProcess(nn.Module):
@@ -453,7 +464,7 @@ class PostProcess(nn.Module):
         self.register_buffer("mean", mean)
 
     def forward(self, out, z, seg):
-        out, force = out if isinstance(out, tuple) else (out, None)
+        out, *rest = out if isinstance(out, tuple) else (out,)
         if self.atomref is not None:
             out = out + ops.segment_reduce(self.atomref[z].to(torch.float32), *seg, mean=not self.is_extensive)
         if self.mean is not None:
@@ -462,7 +473,7 @@ class PostProcess(nn.Module):
                 cnt = (seg[0][1:] - seg[0][:-1]).to(m.dtype).unsqueeze(1)
                 m = cnt * m
             out = out + m
-        return out if force is None else (out, force)
+        return (out, *rest) if rest else out
 
 
 # ----------------------------------------------------------------------------------------------
@@ -602,6 +613,11 @@ class LCAONet(nn.Module):
         # range-check z / batch / edge_index on the device before they index anything (IndexError like the reference's
         # nn.Embedding / index_select); costs one host sync per forward — set False when the caller vouches for the batch
         self.validate_inputs = True
+        # also return the stress  sigma_g = (1 / |det L_g|) d E / d eps_g  (B,3,3) (ASE's get_stress convention before Voigt
+        # packing; eps_g a strain of cell g acting as pos (I + eps), L (I + eps)), computed in the same backward pass as the
+        # autograd forces: forward returns (energy, forces, stress), stress in energy units per A^3, not symmetrised; a cell
+        # of zero volume gives non-finite rows.  Needs regress_forces=True, direct_forces=False.
+        self.regress_stress = False
 
         elec_info = ElecInfo(max_z, max_orb, min_orb, n_per_orb)
         if elec_info.n_orb > 64:
@@ -655,6 +671,9 @@ class LCAONet(nn.Module):
     # -- forward ------------------------------------------------------------------------------------
     def forward(self, graph):
         autograd_forces = self.regress_forces and not self.direct_forces
+        if self.regress_stress and not autograd_forces:
+            raise ValueError("regress_stress needs autograd forces: construct the model with regress_forces=True, "
+                             "direct_forces=False")
         if autograd_forces:
             graph[GraphKeys.Pos].requires_grad_(True)
         batch_idx = graph.get(GraphKeys.Batch_idx)
@@ -669,23 +688,26 @@ class LCAONet(nn.Module):
 
         # indices: CSR by target / by source built on the GPU (replaces torch_sparse, lcaonet.py:462-477)
         gi = ops.GraphIndex(edge_index, N)
-        # geometry + radial basis in one kernel (base.py:27-43, rbf.py:129-142)
-        dist, unit, rb = ops.geom_basis(pos, shift, lattice, batch_idx, gi, self.rbf.spec, self.rbf.n_orb)
-        graph[GraphKeys.Edge_dist], graph[GraphKeys.Edge_vec_st] = dist, unit
-        if self.side_effect_keys:
-            k, e_ks, e_st, cos = gi.triplets(unit.detach())
-            graph[GraphKeys.Idx_k_3b], graph[GraphKeys.Edge_idx_ks_3b], graph[GraphKeys.Edge_idx_st_3b] = k, e_ks, e_st
-            graph[GraphKeys.Angles_3b] = cos
         # nodes -> graphs segments
         if batch_idx is None:
             seg = (torch.tensor([0, N], dtype=torch.int32, device=z.device), None,
                    torch.zeros(N, dtype=torch.int64, device=z.device))
         else:
             seg = (*ops.bucket_sort(batch_idx, n_graph), batch_idx)
+        # stress: a zero strain per graph whose gradient is the virial (ops.geom_basis)
+        strain = (torch.zeros(seg[0].numel() - 1, 3, 3, device=pos.device, requires_grad=True) if self.regress_stress
+                  else None)
+        # geometry + radial basis in one kernel (base.py:27-43, rbf.py:129-142)
+        dist, unit, rb = ops.geom_basis(pos, shift, lattice, batch_idx, gi, self.rbf.spec, self.rbf.n_orb, strain, seg[:2])
+        graph[GraphKeys.Edge_dist], graph[GraphKeys.Edge_vec_st] = dist, unit
+        if self.side_effect_keys:
+            k, e_ks, e_st, cos = gi.triplets(unit.detach())
+            graph[GraphKeys.Idx_k_3b], graph[GraphKeys.Edge_idx_ks_3b], graph[GraphKeys.Edge_idx_st_3b] = k, e_ks, e_st
+            graph[GraphKeys.Angles_3b] = cos
 
         x, cst = self.emb_layer(z, idx_s, idx_t)
         vmask = self.valence_mask(z, idx_t) if self.add_valence else None
         for layer in self.int_layers:
             x = layer(x, cst, vmask, rb, unit, gi, self._lgrp, self._n_l)
-        out = self.out_layer(x, seg, gi, unit, pos)
+        out = self.out_layer(x, seg, gi, unit, pos, strain, lattice)
         return self.pp_layer(out, z, seg)

@@ -164,33 +164,36 @@ def histogram(keys: Tensor, n_buckets: int) -> Tensor:
 # ------------------------------------------------------------------------------------------------
 class _GeomBasis(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, pos, shift, lattice, batch, gi: GraphIndex, spec, n_orb: int):
+    def forward(ctx, pos, shift, lattice, batch, gi: GraphIndex, spec, n_orb: int, strain=None, seg=None):
         require_cuda(pos, shift, lattice)
         pos_c, shift_c, lat_c = pos.contiguous().float(), shift.contiguous().float(), lattice.contiguous().float()
         E, dev = gi.E, pos.device
         dist = torch.empty(E, device=dev)
         unit = torch.empty(E, 3, device=dev)
         rb = torch.empty(E, n_orb, device=dev)
-        need_grad = ctx.needs_input_grad[0]
+        ni = ctx.needs_input_grad
+        need_grad = ni[0] or ni[2] or ni[7]
         drb = torch.empty(E, n_orb, device=dev) if need_grad else None
         _call("lcao_geom_basis_fwd", ptr(pos_c), ptr(shift_c), ptr(lat_c), ptr(batch), ptr(gi.src32), ptr(gi.dst32), E,
               ctypes.byref(spec), ptr(dist), ptr(unit), ptr(rb), ptr(drb), stream_ptr())
-        ctx.gi, ctx.n_orb, ctx.spec = gi, n_orb, spec
-        ctx.save_for_backward(dist, unit, drb, pos, shift, lattice, batch)
+        ctx.gi, ctx.n_orb, ctx.spec, ctx.seg = gi, n_orb, spec, seg
+        ctx.save_for_backward(dist, unit, drb, pos, shift, lattice, batch, strain)
         return dist, unit, rb
 
     @staticmethod
     def backward(ctx, d_dist, d_unit, d_rb):
-        dist, unit, drb, pos, shift, lattice, batch = ctx.saved_tensors
+        dist, unit, drb, pos, shift, lattice, batch, strain = ctx.saved_tensors
         gi = ctx.gi
         if drb is None:
-            return (None,) * 7
+            return (None,) * 9
+        ni = ctx.needs_input_grad
         if torch.is_grad_enabled():  # create_graph=True: this backward is itself differentiated (training on autograd forces)
             with torch.enable_grad():
-                (pos_,) = second_order.aliases([pos])
-                outs = second_order.geom_basis(pos_, shift, lattice, batch, gi.src32, gi.dst32, ctx.spec, ctx.n_orb)
-                (d_pos,) = second_order.grads_with_graph(outs, [pos_], [d_dist, d_unit, d_rb], [True])
-            return d_pos, None, None, None, None, None, None
+                pos_, lat_, strain_ = second_order.aliases([pos, lattice, strain])
+                outs = second_order.geom_basis(pos_, shift, lat_, batch, gi.src32, gi.dst32, ctx.spec, ctx.n_orb, strain_)
+                d_pos, d_lat, d_strain = second_order.grads_with_graph(outs, [pos_, lat_, strain_], [d_dist, d_unit, d_rb],
+                                                                       [ni[0], ni[2], ni[7]])
+            return d_pos, None, d_lat, None, None, None, None, d_strain, None
         dev = dist.device
         dvec = torch.empty(gi.E, 3, device=dev)
         d_pos = torch.empty(gi.N, 3, device=dev)
@@ -199,11 +202,44 @@ class _GeomBasis(torch.autograd.Function):
         _call("lcao_geom_basis_bwd", ptr(dist), ptr(unit), ptr(drb), ptr(d_dist), ptr(d_unit), ptr(d_rb), gi.E, gi.N,
               ctx.n_orb, ptr(gi.in_ptr), ptr(gi.in_edge), ptr(gi.out_ptr), ptr(gi.out_edge), ptr(dvec), ptr(d_pos),
               stream_ptr())
-        return d_pos, None, None, None, None, None, None
+        d_lat = d_strain = None
+        if ni[2] or ni[7]:
+            d_lat, d_strain = _cell_grads(dvec, pos, shift, lattice, batch, gi, ctx.seg, ni[2], ni[7])
+        return d_pos if ni[0] else None, None, d_lat, None, None, None, None, d_strain, None
 
 
-def geom_basis(pos, shift, lattice, batch, gi, spec, n_orb):
-    return _GeomBasis.apply(pos, shift, lattice, batch, gi, spec, n_orb)
+def _cell_grads(dvec, pos, shift, lattice, batch, gi, seg, want_lattice: bool, want_virial: bool):
+    """(d E / d lattice, virial) per graph from dvec = d E / d vec (lcao_geom_cell_bwd); None where not wanted.
+    `seg` = (seg_ptr, seg_perm) groups the nodes by graph; built from `batch` here when the caller has none."""
+    dev = dvec.device
+    if seg is None:
+        seg = (torch.tensor([0, gi.N], dtype=torch.int32, device=dev), None) if batch is None else \
+            bucket_sort(batch, lattice.shape[0])
+    seg_ptr, seg_perm = seg[0], seg[1]
+    B = seg_ptr.numel() - 1
+    d_lat = torch.empty(B, 3, 3, device=dev) if want_lattice else None
+    virial = torch.empty(B, 3, 3, device=dev) if want_virial else None
+    scratch = torch.empty((gi.N // _lib.CELL_CHUNK + B) * 18, dtype=torch.float64, device=dev)
+    pos_c, shift_c, lat_c = pos.contiguous().float(), shift.contiguous().float(), lattice.contiguous().float()
+    _call("lcao_geom_cell_bwd", ptr(pos_c), ptr(shift_c), ptr(lat_c), ptr(batch), ptr(gi.dst32), ptr(dvec), gi.E, gi.N,
+          ptr(gi.out_ptr), ptr(gi.out_edge), ptr(seg_ptr), ptr(seg_perm), B, ptr(scratch), ptr(d_lat), ptr(virial),
+          stream_ptr())
+    if d_lat is not None:
+        if lattice.shape[0] > B:  # batch=None: the forward reads lattice[0] only
+            d_lat = torch.cat([d_lat, d_lat.new_zeros(lattice.shape[0] - B, 3, 3)])
+        d_lat = d_lat.to(lattice.dtype)
+    return d_lat, virial
+
+
+def geom_basis(pos, shift, lattice, batch, gi, spec, n_orb, strain=None, seg=None):
+    """(dist, unit, rb) of every edge, vec_e = pos[t] - pos[s] + shift_e . lattice[batch[s]] (row vectors, base.py:27-43).
+    Differentiable with respect to `pos` and `lattice` (d E / d L_g[i][j] = sum_{e in g} shift_e[i] dvec_e[j]); the
+    gradient with respect to `shift` is not computed (None).
+    `strain` (internal, not public API: LCAONet.regress_stress creates it) is a (B,3,3) gradient probe: zeros with
+    requires_grad whose value the forward never reads, standing for eps_g in pos' = pos (I + eps), L' = L (I + eps).  Its
+    gradient is the virial W_g = sum_{e in g} vec_e (x) dvec_e.  `seg` = (seg_ptr, seg_perm), the nodes grouped by
+    graph (optional: built from `batch` when a cell gradient is wanted and it is missing)."""
+    return _GeomBasis.apply(pos, shift, lattice, batch, gi, spec, n_orb, strain, seg)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -704,7 +740,7 @@ class _InteractionLayer(torch.autograd.Function):
         # B = pair_contract(tab, rb) ; tab = f_coeffs(table)
         need_tab = wg and (ctx.needs_input_grad[1] or any(ctx.needs_input_grad[6:8]))
         d_rb = torch.empty(E, O, device=dev) if need_rb else None
-        if need_tab or need_rb:
+        if need_tab or (need_rb and E > 0):  # (an edge-less batch has no d rb to write)
             kptr, kperm = _grouping(grouping, pair, P)
             d_tab = torch.empty(P, O, Cp, device=dev) if need_tab else None
             scratch = None

@@ -83,14 +83,19 @@ def _cutoff(kind: int, r: Tensor, rc: float) -> Tensor:
     return torch.where(r <= rc, f, torch.zeros_like(f))
 
 
-def geom_basis(pos: Tensor, shift: Tensor, lattice: Tensor, batch: Tensor | None, src: Tensor, dst: Tensor, spec, n_orb: int):
-    """(dist, unit, rb) as functions of `pos` (base.py:27-43, rbf.py:92-142, cutoff.py:32-67), evaluated in float64
-    (edge-sized work) and rounded to float32 like the kernel's outputs."""
+def geom_basis(pos: Tensor, shift: Tensor, lattice: Tensor, batch: Tensor | None, src: Tensor, dst: Tensor, spec, n_orb: int,
+               strain: Tensor | None = None):
+    """(dist, unit, rb) as functions of `pos`, `lattice` and the strain probe (base.py:27-43, rbf.py:92-142,
+    cutoff.py:32-67), evaluated in float64 (edge-sized work) and rounded to float32 like the kernel's outputs.
+    With `strain` (B,3,3): vec = ((pos[t] - pos[s]) + shift . L) (I + strain[g]); its value is zero, so the result is
+    unchanged and only the derivative (the virial) differs from the plain form."""
     s, t = src.long(), dst.long()
     P = pos.double()
     b = batch[s] if batch is not None else torch.zeros_like(s)
     L = lattice.double()[b]
     v = (P[t] - P[s]) + (shift.double().unsqueeze(-1) * L).sum(1)
+    if strain is not None:
+        v = v + (v.unsqueeze(-1) * strain.double()[b]).sum(1)
     r = v.norm(dim=1)
     unit = v / r.unsqueeze(-1)
     fc = _cutoff(spec.cutoff_kind, r, float(spec.rc))
