@@ -6,25 +6,23 @@
 // (3 MMAs, error ~2^-21 per product: FP32-equivalent, which the 1e-5 parity bar needs); LCAO_GEMM_TF32
 // issues hi*hi only.
 //
-// Operands never go through TMA: "transform" warps stream the FP32 rows from HBM with coalesced 128-bit
-// loads, apply the fused prologue (identity, or dY * SiLU'(H) for the backward passes), split hi/lo in
-// registers and write both halves straight into the UMMA canonical NO-SWIZZLE K-major shared-memory
-// layout (the weight-gradient kernel transposes 4x4 blocks in registers on the way).  The leading byte
-// offset is padded by 16 B so those 128-bit shared stores are bank-conflict free.
+// Operands never go through TMA: loader warps stream the FP32 rows from HBM with 16-byte cp.async copies into
+// SWIZZLE_128B K-major shared-memory tiles, and transform warps split them into hi / lo for the MMAs (the weight-gradient
+// kernel transposes 4x4 blocks in registers on the way).  The row kernels keep the layer's weight resident in shared
+// memory, split once per CTA.
 //
-// Warp roles (288 threads): warps 0-3 epilogue (TMEM lanes 32w..32w+31 -> registers -> HBM),
-// warps 4-7 transform/producer, warp 8 MMA issuer (one elected lane) + TMEM allocator.
-// Pipelines: smem stages full/empty (producer <-> MMA), TMEM accumulator full/empty (MMA <-> epilogue),
-// persistent loop over 128-row blocks (grid = #SMs).  All mbarrier waits are bounded (trap on timeout)
-// so a protocol bug aborts the kernel instead of hanging the GPU.
-#include <stdlib.h>
-
+// Kernels (warp roles and pipelines are described at each kernel):
+//   k_tc_rows<EPI8>  Y = epi(A W^T) or epi(A W), 128-row tiles, persistent over the row blocks (grid <= #SMs);
+//                    EPI8 adds four epilogue warps for grids with one tile per CTA.
+//   k_tc_rows_ta     the same product in 3xTF32 mode with the A operand in tensor memory, for many tiles per CTA.
+//   k_tc_wgrad       dW += dY^T X (and db += colsum dY) as per-CTA partial tiles, summed in a fixed order by
+//                    k_wgrad_reduce / k_wgrad_reduce_batch (deterministic, no atomics).
+// All mbarrier waits are bounded (trap on timeout) so a protocol bug aborts the kernel instead of hanging the GPU.
 #include "common.cuh"
 
 namespace {
 
-constexpr int kEpiWarps = 4, kProdWarps = 4;
-constexpr int kThreadsTC = (kEpiWarps + kProdWarps + 1) * 32;  // 288
+constexpr int kEpiWarps = 4;
 constexpr int kBlockM = 128;                                   // rows per tile (UMMA M)
 constexpr int kChunkK = 32;                                    // contraction elements per smem stage
 constexpr uint32_t kSpinLimit = 1u << 28;  // (several seconds: under programmatic dependent launch a CTA may poll while the previous kernel drains)
@@ -106,17 +104,9 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
   for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
 
-// UMMA shared-memory descriptor, SWIZZLE_NONE (cute::UMMA::SmemDescriptor: start>>4 [0,14), LBO>>4 [16,30),
-// SBO>>4 [32,46), version=1 [46,48), layout_type=0 [61,64))
-__device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32;
-  d |= (uint64_t)1 << 46;
-  return d;
-}
-// SWIZZLE_128B K-major tile: rows of 128 bytes (32 tf32), 16-byte chunk c of row r stored at chunk (c ^ (r & 7));
+// UMMA shared-memory descriptor (cute::UMMA::SmemDescriptor: start>>4 [0,14), LBO>>4 [16,30), SBO>>4 [32,46),
+// version=1 [46,48), layout_type [61,64)) of a SWIZZLE_128B K-major tile:
+// rows of 128 bytes (32 tf32), 16-byte chunk c of row r stored at chunk (c ^ (r & 7));
 // 8-row groups are 1024 B apart (SBO), LBO is unused (=1), layout_type = 2, tile base 1024-byte aligned.
 // One MMA consumes K = 8 tf32 = 32 bytes: the start address advances by 32 B inside the swizzled row.
 __device__ __forceinline__ uint64_t make_desc_sw128(uint32_t smem_addr) {
@@ -130,10 +120,9 @@ __device__ __forceinline__ uint64_t make_desc_sw128(uint32_t smem_addr) {
 }
 __device__ __forceinline__ uint32_t sw128_off(int row, int chunk) { return row * 128 + ((chunk ^ (row & 7)) << 4); }
 // instruction descriptor (cute::UMMA::InstrDescriptor): c_format F32=1 [4,6), a/b_format TF32=2 [7,10)/[10,13),
-// a_major [15], b_major [16] (0 = K-major, 1 = MN-major), N>>3 [17,23), M>>4 [24,29)
-__host__ __device__ constexpr uint32_t make_idesc(int M, int N, int a_mn_major, int b_mn_major) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
-         ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+// a_major [15] = b_major [16] = 0 (both operands K-major), N>>3 [17,23), M>>4 [24,29)
+__host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
 __device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
@@ -189,8 +178,6 @@ struct RowsArgs {
   int64_t M; int Kc; int Nb;
   int b_trans, act, accumulate, x3, stages, lo_stages;
   int wide_store;  // Y / pre rows are 32-byte aligned: 256-bit stores
-  int one_acc;  // 3xTF32 corrections accumulate into the same TMEM accumulator as hi*hi (LCAO_TC_ONEACC, experiment)
-  int debug;  // ablation bits for tuning runs (LCAO_TC_DEBUG): 1 = no output stores, 2 = no input copies, 4 = no MMAs
 };
 
 constexpr int kLoadWarps = 4;
@@ -207,10 +194,9 @@ __device__ __forceinline__ void cp_async_arrive(uint64_t* bar) {
 }
 
 // EPI8: four more epilogue warps (13-16); the two warps of a TMEM lane quadrant take 64 output columns each
-template <bool RP, bool EPI8>
+template <bool EPI8>
 __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k_tc_rows(const RowsArgs g) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  if (g.debug & 32) return;  // (ablation: launch cost only)
   pdl_trigger();  // the next kernel of the stream may start its own set-up while this one runs
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t blockB = g.Nb * 128;                 // bytes of one 32-k column block of the weight
@@ -240,7 +226,7 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
   if (threadIdx.x == 0) {
     for (int s = 0; s < R; ++s) {
       mbar_init(&raw_full[s], kLoadWarps * 32);
-      mbar_init(&full[s], RP ? 8 * 32 : 4 * 32);
+      mbar_init(&full[s], 4 * 32);
       mbar_init(&hi_empty[s], 1);
     }
     for (int s = 0; s < L; ++s) mbar_init(&lo_empty[s], 1);
@@ -255,42 +241,6 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
   __syncthreads();  // barriers initialised, TMEM address published
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (g.debug & 64) {  // (ablation: launch + TMEM/barrier set-up only)
-    __syncthreads();
-    if (warp == 8) tmem_dealloc(tmem_base, tmem_cols);
-    return;
-  }
-
-  // ---- RP (register-prefetch producers): the 8 warps 4-7 and 9-12 stream A with plain 128-bit loads into REGISTERS,
-  //      three 16 KB chunks ahead of the one they split and store, so the bytes in flight (48 KB per SM) live in the
-  //      register file and a shared-memory stage is only occupied from its store to the commit of its MMAs.  The
-  //      cp.async path below keeps the in-flight bytes in the stages themselves (3 x 16 KB beside the 128 KB weight).
-  const bool is_prod = RP && ((warp >= 9 && warp < 13) || (warp >= 4 && warp < 8));
-  const int pidx = ((warp >= 9 ? warp - 5 : warp - 4) << 5) | lane;  // 0..255 among the producers
-  const int pc = pidx & 7, pr = pidx >> 3;                           // 16-byte column / row (+ 32 j) inside a chunk
-  float4 rbuf[4][4];
-  int64_t ld_mb = blockIdx.x;
-  int ld_kc = 0;
-  uint32_t ld_q = 0, rp_total = 0;
-  auto issue_load = [&](float4 (&b)[4]) {
-    if (ld_q < rp_total) {
-      const int64_t row0 = ld_mb * kBlockM + pr;
-      const float* src = g.A + row0 * g.lda + ld_kc * kChunkK + pc * 4;
-#pragma unroll
-      for (int j = 0; j < 4; ++j)
-        b[j] = (row0 + 32 * j < g.M && !(g.debug & 2)) ? ldg4(src + (int64_t)32 * j * g.lda) : make_float4(0.f, 0.f, 0.f, 0.f);
-      if (++ld_kc == nchunk) { ld_kc = 0; ld_mb += gridDim.x; }
-      ++ld_q;
-    }
-  };
-  if (is_prod) {
-    pdl_wait();
-    const int64_t my_tiles = nblocks > (int64_t)blockIdx.x ? (nblocks - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-    rp_total = (uint32_t)(my_tiles * nchunk);
-    issue_load(rbuf[0]);
-    issue_load(rbuf[1]);
-    issue_load(rbuf[2]);
-  }
 
   // ---- resident B operand (the layer's weight), split hi/lo once per CTA by the 9 non-loader warps while the
   //      loader warps already stream the first A stages; kWB loads in flight per thread (the weights come from L2 /
@@ -336,38 +286,7 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
   // Everything above (barriers, TMEM, the split of the resident weight: parameters, never written by a kernel that triggers
   // early) may overlap the tail of the previous kernel (programmatic dependent launch); the activations may not.
   pdl_wait();
-  if (is_prod) {
-    // ============================== producers: registers -> hi / lo stages ==============================
-    uint32_t it = 0;
-    for (uint32_t q = 0; q < rp_total; q += 4) {
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        if (q + u < rp_total) {
-          issue_load(rbuf[(u + 3) & 3]);  // chunk q + u + 3
-          const int s = it % R, l = it % L;
-          mbar_wait(&hi_empty[s], ((it / R) & 1) ^ 1);
-          if (g.x3) mbar_wait(&lo_empty[l], ((it / L) & 1) ^ 1);
-          uint8_t* ph = sHi + (size_t)s * kStageBytes;
-          uint8_t* pl = sLo + (size_t)l * kStageBytes;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const uint32_t off = sw128_off(pr + 32 * j, pc);
-            if (g.x3 && !(g.debug & 16)) {
-              float4 hi, lo;
-              split4(rbuf[u][j], hi, lo);
-              *reinterpret_cast<float4*>(ph + off) = hi;
-              *reinterpret_cast<float4*>(pl + off) = lo;
-            } else {
-              *reinterpret_cast<float4*>(ph + off) = rbuf[u][j];  // (the tensor core ignores the low mantissa bits)
-            }
-          }
-          fence_proxy_async();
-          mbar_arrive(&full[s]);
-          ++it;
-        }
-      }
-    }
-  } else if (!RP && warp >= 9 && warp < 13) {
+  if (warp >= 9 && warp < 13) {
     // ============================== loader warps ==============================
     // warp lw streams rows [32 lw, 32 lw + 32) of the tile: 8 copies per lane and stage; lanes 0-7 / 8-15 / ...
     // cover one 128-byte row each (global) and write its 8 chunks into one swizzled 128-byte smem line
@@ -381,17 +300,15 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
         mbar_wait(&hi_empty[s], ((it / R) & 1) ^ 1);
         const uint32_t dst = hi_base + s * kStageBytes;
         const float* src = g.A + mrow * g.lda + kc * kChunkK + c * 4;
-        if (!(g.debug & 2)) {
 #pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const bool ok = mrow + 4 * j < g.M;
-            cp_async16(dst + sw128_off(32 * lw + 4 * j + row_in, c), ok ? src + (int64_t)4 * j * g.lda : g.A, ok ? 16u : 0u);
-          }
+        for (int j = 0; j < 8; ++j) {
+          const bool ok = mrow + 4 * j < g.M;
+          cp_async16(dst + sw128_off(32 * lw + 4 * j + row_in, c), ok ? src + (int64_t)4 * j * g.lda : g.A, ok ? 16u : 0u);
         }
         cp_async_arrive(&raw_full[s]);
       }
     }
-  } else if (!RP && warp >= 4 && warp < 8) {
+  } else if (warp >= 4 && warp < 8) {
     // ============================== split warps: hi in place, lo into the short ring =================
     const int t = threadIdx.x - 128;              // 0..127
     uint32_t it = 0;
@@ -401,8 +318,6 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
         mbar_wait(&raw_full[s], (it / R) & 1);
         if (g.x3) {
           mbar_wait(&lo_empty[l], ((it / L) & 1) ^ 1);
-        }
-        if (g.x3 && !(g.debug & 16)) {
           uint8_t* ph = sHi + (size_t)s * kStageBytes + t * 16;
           uint8_t* pl = sLo + (size_t)l * kStageBytes + t * 16;
 #pragma unroll
@@ -420,31 +335,29 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
   } else if (warp == 8) {
     // ============================== MMA issuer (all lanes run the loop; one is elected per instruction) ==============
     {
-      const uint32_t idesc = make_idesc(kBlockM, g.Nb, 0, 0);
+      const uint32_t idesc = make_idesc(kBlockM, g.Nb);
       const uint32_t hiBase = smem_u32(sHi), loBase = smem_u32(sLo), bBase = smem_u32(sB);
       uint32_t it = 0, tile = 0;
       for (int64_t mb = blockIdx.x; mb < nblocks; mb += gridDim.x, ++tile) {
         const int acc = tile & 1;
         mbar_wait(&tempty[acc], ((tile >> 1) & 1) ^ 1);
         tc_fence_after();
-        const uint32_t d = tmem_base + acc * acc_cols, dc = g.one_acc ? d : d + g.Nb;
+        const uint32_t d = tmem_base + acc * acc_cols, dc = d + g.Nb;
         for (int kc = 0; kc < nchunk; ++kc, ++it) {
           const int s = it % R, l = it % L;
           mbar_wait(&full[s], (it / R) & 1);
           tc_fence_after();
           const uint32_t a_hi = hiBase + s * kStageBytes, a_lo = loBase + l * kStageBytes;
           const uint32_t b_hi = bBase + kc * blockB, b_lo = b_hi + halfB;
-          if (!(g.debug & 4)) {
-            const uint64_t dAh0 = make_desc_sw128(a_hi), dBh0 = make_desc_sw128(b_hi), dAl0 = make_desc_sw128(a_lo), dBl0 = make_desc_sw128(b_lo);
+          const uint64_t dAh0 = make_desc_sw128(a_hi), dBh0 = make_desc_sw128(b_hi), dAl0 = make_desc_sw128(a_lo), dBl0 = make_desc_sw128(b_lo);
 #pragma unroll
-            for (int kk = 0; kk < kChunkK / 8; ++kk) {
-              const uint64_t dAh = dAh0 + 2 * kk, dBh = dBh0 + 2 * kk, dAl = dAl0 + 2 * kk, dBl = dBl0 + 2 * kk;
-              if (elect_one()) {
-                umma_tf32(d, dAh, dBh, idesc, (kc | kk) != 0);
-                if (g.x3) {
-                  umma_tf32(dc, dAl, dBh, idesc, g.one_acc ? 1 : (kc | kk) != 0);
-                  umma_tf32(dc, dAh, dBl, idesc, 1);
-                }
+          for (int kk = 0; kk < kChunkK / 8; ++kk) {
+            const uint64_t dAh = dAh0 + 2 * kk, dBh = dBh0 + 2 * kk, dAl = dAl0 + 2 * kk, dBl = dBl0 + 2 * kk;
+            if (elect_one()) {
+              umma_tf32(d, dAh, dBh, idesc, (kc | kk) != 0);
+              if (g.x3) {
+                umma_tf32(dc, dAl, dBh, idesc, (kc | kk) != 0);
+                umma_tf32(dc, dAh, dBl, idesc, 1);
               }
             }
           }
@@ -480,7 +393,7 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
       }
       mbar_wait(&tfull[acc], (tile >> 1) & 1);
       tc_fence_after();
-      for (int c0 = c_begin; c0 < ((g.debug & 8) ? 0 : c_end); c0 += 32) {
+      for (int c0 = c_begin; c0 < c_end; c0 += 32) {
         float4 gn[8];
         if (g.G && m < g.M && c0 + 32 < c_end) {
 #pragma unroll
@@ -489,7 +402,7 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
         }
         float v[32];
         tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + acc * acc_cols + c0, v);
-        if (g.x3 && !g.one_acc) {
+        if (g.x3) {
           float w[32];
           tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + acc * acc_cols + g.Nb + c0, w);
 #pragma unroll
@@ -520,7 +433,7 @@ __global__ void __launch_bounds__(EPI8 ? kRowsThreads + 128 : kRowsThreads, 1) k
                 o[0] *= silu_grad_fast(h0.x); o[1] *= silu_grad_fast(h0.y); o[2] *= silu_grad_fast(h0.z); o[3] *= silu_grad_fast(h0.w);
                 o[4] *= silu_grad_fast(h1.x); o[5] *= silu_grad_fast(h1.y); o[6] *= silu_grad_fast(h1.z); o[7] *= silu_grad_fast(h1.w);
               }
-              if (!(g.debug & 1)) store8(g.Y + m * g.ldy + c0 + j, o, wide);
+              store8(g.Y + m * g.ldy + c0 + j, o, wide);
             }
           }
         }
@@ -591,17 +504,13 @@ __device__ __forceinline__ void tmem_ld32_nw(uint32_t taddr, float (&v)[32]) {
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
-// CPS = 32-column chunks per pipeline stage (1 or 2).  Every stage costs one round of mbarrier hand-shakes between the
-// loaders, the split warps and the MMA issuer (~0.35 us: with nothing but the hand-shakes left the kernel takes 29 us
-// at M = 252 798 with one chunk per stage, 20 us with two), but the hand-shakes are not the critical path: the full
-// kernel does not get faster with CPS = 2, nor with a second group of split warps taking the odd chunks.  What set
-// the pace after the operand moved to tensor memory was the epilogue (see below); profiles/r02_notes.md.
-template <int CPS>
+// One 32-column chunk per pipeline stage.  Every stage costs one round of mbarrier hand-shakes between the loaders, the
+// split warps and the MMA issuer (~0.35 us), but the hand-shakes are not the critical path: two chunks per stage, or a
+// second group of split warps taking the odd chunks, did not make the kernel faster.  What set the pace after the
+// operand moved to tensor memory was the epilogue (see below); profiles/r02_notes.md.
 __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) {
   // warps: 0-3 epilogue (columns 0-63), 4-7 split, 8 MMA issuer, 9-10 loaders (64 rows each), 11-14 epilogue (columns 64-127)
   constexpr int kLd = 2;
-  constexpr uint32_t kStB = CPS * kStageBytes;         // bytes of one raw stage
-  constexpr int kTaSt = kTaStages / CPS;               // TMEM ring depth (stage = CPS x (32 hi + 32 lo) columns)
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   pdl_trigger();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -610,7 +519,7 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
   const int R = g.stages;
   uint8_t* sB = smem_raw;
   uint8_t* sRaw = sB + 2 * halfB;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sRaw + (size_t)R * kStB);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sRaw + (size_t)R * kStageBytes);
   uint64_t* raw_full = bars;               // [R] loaders (cp.async completion) -> split warps
   uint64_t* raw_empty = raw_full + R;      // [R] split warps -> loaders
   uint64_t* a_full = raw_empty + R;        // [kTaStages] split warps -> MMA
@@ -619,7 +528,7 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
   uint64_t* tempty = tfull + 2;            // [2] epilogue -> MMA
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
   const int64_t nblocks = (g.M + kBlockM - 1) / kBlockM;
-  const int nchunk = g.Kc / (kChunkK * CPS);  // pipeline stages per tile
+  const int nchunk = g.Kc / kChunkK;
   constexpr uint32_t tmem_cols = 512;
 
   if (threadIdx.x == 0) {
@@ -627,7 +536,7 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
       mbar_init(&raw_full[s], kLd * 32);
       mbar_init(&raw_empty[s], 4 * 32);
     }
-    for (int s = 0; s < kTaSt; ++s) {
+    for (int s = 0; s < kTaStages; ++s) {
       mbar_init(&a_full[s], 4 * 32);
       mbar_init(&a_empty[s], 1);
     }
@@ -694,16 +603,12 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
       for (int kc = 0; kc < nchunk; ++kc, ++it) {
         const int s = it % R;
         mbar_wait(&raw_empty[s], ((it / R) & 1) ^ 1);
-        if (!(g.debug & 2))
+        const uint32_t dst = raw_base + s * kStageBytes;
+        const float* src = g.A + mrow * g.lda + kc * kChunkK + c * 4;
 #pragma unroll
-        for (int sub = 0; sub < CPS; ++sub) {
-          const uint32_t dst = raw_base + s * kStB + sub * kStageBytes;
-          const float* src = g.A + mrow * g.lda + (kc * CPS + sub) * kChunkK + c * 4;
-#pragma unroll
-          for (int j = 0; j < kRowsPerLd / 4; ++j) {
-            const bool ok = mrow + 4 * j < g.M;
-            cp_async16(dst + sw128_off(kRowsPerLd * lw + 4 * j + row_in, c), ok ? src + (int64_t)4 * j * g.lda : g.A, ok ? 16u : 0u);
-          }
+        for (int j = 0; j < kRowsPerLd / 4; ++j) {
+          const bool ok = mrow + 4 * j < g.M;
+          cp_async16(dst + sw128_off(kRowsPerLd * lw + 4 * j + row_in, c), ok ? src + (int64_t)4 * j * g.lda : g.A, ok ? 16u : 0u);
         }
         cp_async_arrive(&raw_full[s]);
       }
@@ -715,32 +620,23 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
     uint32_t it = 0;
     for (int64_t mb = blockIdx.x; mb < nblocks; mb += gridDim.x) {
       for (int kc = 0; kc < nchunk; ++kc, ++it) {
-        const int s = it % R, ts = it % kTaSt;
+        const int s = it % R, ts = it % kTaStages;
         mbar_wait(&raw_full[s], (it / R) & 1);
-        if (g.debug & 16) {  // (ablation: no split work, no TMEM stores)
-          mbar_arrive(&raw_empty[s]);
-          mbar_wait(&a_empty[ts], ((it / kTaSt) & 1) ^ 1);
-          mbar_arrive(&a_full[ts]);
-          continue;
-        }
-        mbar_wait(&a_empty[ts], ((it / kTaSt) & 1) ^ 1);
+        mbar_wait(&a_empty[ts], ((it / kTaStages) & 1) ^ 1);
         tc_fence_after();
+        const uint8_t* pr = sRaw + (size_t)s * kStageBytes;
+        uint32_t hi[32], lo[32];
 #pragma unroll
-        for (int sub = 0; sub < CPS; ++sub) {
-          const uint8_t* pr = sRaw + (size_t)s * kStB + sub * kStageBytes;
-          uint32_t hi[32], lo[32];
-#pragma unroll
-          for (int c = 0; c < 8; ++c) {
-            const float4 v = *reinterpret_cast<const float4*>(pr + sw128_off(row, c));
-            float4 h, l;
-            split4(v, h, l);
-            hi[4 * c] = __float_as_uint(h.x); hi[4 * c + 1] = __float_as_uint(h.y); hi[4 * c + 2] = __float_as_uint(h.z); hi[4 * c + 3] = __float_as_uint(h.w);
-            lo[4 * c] = __float_as_uint(l.x); lo[4 * c + 1] = __float_as_uint(l.y); lo[4 * c + 2] = __float_as_uint(l.z); lo[4 * c + 3] = __float_as_uint(l.w);
-          }
-          const uint32_t ta = tmem_base + lane_base + kTaCol0 + (ts * CPS + sub) * 64;
-          tmem_st32(ta, hi);
-          tmem_st32(ta + 32, lo);
+        for (int c = 0; c < 8; ++c) {
+          const float4 v = *reinterpret_cast<const float4*>(pr + sw128_off(row, c));
+          float4 h, l;
+          split4(v, h, l);
+          hi[4 * c] = __float_as_uint(h.x); hi[4 * c + 1] = __float_as_uint(h.y); hi[4 * c + 2] = __float_as_uint(h.z); hi[4 * c + 3] = __float_as_uint(h.w);
+          lo[4 * c] = __float_as_uint(l.x); lo[4 * c + 1] = __float_as_uint(l.y); lo[4 * c + 2] = __float_as_uint(l.z); lo[4 * c + 3] = __float_as_uint(l.w);
         }
+        const uint32_t ta = tmem_base + lane_base + kTaCol0 + ts * 64;
+        tmem_st32(ta, hi);
+        tmem_st32(ta + 32, lo);
         mbar_arrive(&raw_empty[s]);  // the stage is in registers / tensor memory: it can take the next copies
         tmem_wait_st();
         tc_fence_before();
@@ -750,7 +646,7 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
   } else if (warp == 8) {
     // ============================== MMA issuer (all lanes run the loop; one is elected per instruction) ==============
     {
-      const uint32_t idesc = make_idesc(kBlockM, g.Nb, 0, 0);
+      const uint32_t idesc = make_idesc(kBlockM, g.Nb);
       const uint32_t bBase = smem_u32(sB);
       uint32_t it = 0, tile = 0;
       for (int64_t mb = blockIdx.x; mb < nblocks; mb += gridDim.x, ++tile) {
@@ -759,22 +655,19 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
         tc_fence_after();
         const uint32_t d = tmem_base + acc * g.Nb;
         for (int kc = 0; kc < nchunk; ++kc, ++it) {
-          const int ts = it % kTaSt;
-          mbar_wait(&a_full[ts], (it / kTaSt) & 1);
+          const int ts = it % kTaStages;
+          mbar_wait(&a_full[ts], (it / kTaStages) & 1);
           tc_fence_after();
+          const uint32_t a_hi = tmem_base + kTaCol0 + ts * 64, a_lo = a_hi + 32;
+          const uint32_t b_hi = bBase + kc * blockB, b_lo = b_hi + halfB;
+          const uint64_t dBh0 = make_desc_sw128(b_hi), dBl0 = make_desc_sw128(b_lo);
 #pragma unroll
-          for (int sub = 0; sub < CPS; ++sub) {
-            const uint32_t a_hi = tmem_base + kTaCol0 + (ts * CPS + sub) * 64, a_lo = a_hi + 32;
-            const uint32_t b_hi = bBase + (kc * CPS + sub) * blockB, b_lo = b_hi + halfB;
-            const uint64_t dBh0 = make_desc_sw128(b_hi), dBl0 = make_desc_sw128(b_lo);
-#pragma unroll
-            for (int kk = 0; kk < ((g.debug & 4) ? 0 : kChunkK / 8); ++kk) {
-              const uint64_t dBh = dBh0 + 2 * kk, dBl = dBl0 + 2 * kk;  // (+ 32 B per K step: + 2 in the address field)
-              if (elect_one()) {
-                umma_tf32_ts(d, a_hi + kk * 8, dBh, idesc, (kc | sub | kk) != 0);
-                umma_tf32_ts(d, a_lo + kk * 8, dBh, idesc, 1);
-                umma_tf32_ts(d, a_hi + kk * 8, dBl, idesc, 1);
-              }
+          for (int kk = 0; kk < kChunkK / 8; ++kk) {
+            const uint64_t dBh = dBh0 + 2 * kk, dBl = dBl0 + 2 * kk;  // (+ 32 B per K step: + 2 in the address field)
+            if (elect_one()) {
+              umma_tf32_ts(d, a_hi + kk * 8, dBh, idesc, (kc | kk) != 0);
+              umma_tf32_ts(d, a_lo + kk * 8, dBh, idesc, 1);
+              umma_tf32_ts(d, a_hi + kk * 8, dBl, idesc, 1);
             }
           }
           if (elect_one()) umma_commit(&a_empty[ts]);
@@ -794,14 +687,11 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
     const int quad = warp & 3;
     const int c_begin = warp >= 9 + kLd ? 64 : 0, c_end = min(g.Nb, c_begin + 64);
     uint32_t tile = 0;
-    long long t_wait = 0, t_work = 0;  // (LCAO_TC_DEBUG & 64: cycles spent waiting for a finished tile / draining it)
     for (int64_t mb = blockIdx.x; mb < nblocks; mb += gridDim.x, ++tile) {
       const int acc = tile & 1;
-      const long long tq0 = clock64();
       const int64_t m = mb * kBlockM + quad * 32 + lane;
       mbar_wait(&tfull[acc], (tile >> 1) & 1);
       tc_fence_after();
-      const long long tq1 = clock64();
       float v[2][32];
       const uint32_t t0 = tmem_base + ((uint32_t)(quad * 32) << 16) + acc * g.Nb;
       if (c_begin < c_end) tmem_ld32_nw(t0 + c_begin, v[0]);
@@ -809,7 +699,7 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
       tmem_wait_ld();
       tc_fence_before();
       mbar_arrive(&tempty[acc]);
-      if (m < g.M && !(g.debug & 8)) {
+      if (m < g.M) {
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
           const int c0 = c_begin + 32 * h;
@@ -838,18 +728,12 @@ __global__ void __launch_bounds__(kTaThreads, 1) k_tc_rows_ta(const RowsArgs g) 
                   o[0] *= silu_grad_fast(h0.x); o[1] *= silu_grad_fast(h0.y); o[2] *= silu_grad_fast(h0.z); o[3] *= silu_grad_fast(h0.w);
                   o[4] *= silu_grad_fast(h1.x); o[5] *= silu_grad_fast(h1.y); o[6] *= silu_grad_fast(h1.z); o[7] *= silu_grad_fast(h1.w);
                 }
-                if (!(g.debug & 1)) store8(g.Y + m * g.ldy + c0 + j, o, wide);
+                store8(g.Y + m * g.ldy + c0 + j, o, wide);
               }
             }
           }
         }
       }
-      t_wait += tq1 - tq0;
-      t_work += clock64() - tq1;
-    }
-    if ((g.debug & 64) && threadIdx.x == 0) {
-      g.Y[2 * blockIdx.x] = (float)t_wait / (float)max(1u, tile);
-      g.Y[2 * blockIdx.x + 1] = (float)t_work / (float)max(1u, tile);
     }
   }
   tc_fence_before();
@@ -877,8 +761,6 @@ struct WgradArgs {
   float* db;
   float* part;     // per-CTA partial sums: [grid][Kx][128] then [grid][128] column sums (deterministic two-stage reduction)
   int64_t M; int Kx; int x3, raw_stages, op_stages;
-  int one_acc;  // 3xTF32 corrections accumulate into the same TMEM chain as hi*hi (LCAO_TC_ONEACC, experiment)
-  int debug_timing;  // LCAO_TC_DEBUG & 64: CTA 0 prints where its transform warps / MMA issuer wait
 };
 
 __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g) {
@@ -973,15 +855,10 @@ __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g)
     const int ngB = g.Kx / 4;
     float4 colsum[2] = {make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f)};
     uint32_t it = 0;
-    long long tw_raw = 0, tw_op = 0, tw_work = 0;  // (LCAO_TC_DEBUG & 64: where the transform stage spends its cycles)
     for (int64_t c = c_beg; c < c_end; ++c, ++it) {
       const int r = it % Rr, s = it % S;
-      const long long q0 = clock64();
       mbar_wait(&raw_full[r], (it / Rr) & 1);
-      const long long q1 = clock64();
       mbar_wait(&op_empty[s], ((it / S) & 1) ^ 1);
-      const long long q2 = clock64();
-      tw_raw += q1 - q0; tw_op += q2 - q1;
       const uint8_t* rA = sRaw + (size_t)r * (rawA + rawB);
       const uint8_t* rB = rA + rawA;
       uint8_t* oA = sOp + (size_t)s * op_stage;
@@ -1025,11 +902,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g)
       fence_proxy_async();
       mbar_arrive(&op_full[s]);
       mbar_arrive(&raw_empty[r]);
-      tw_work += clock64() - q2;
     }
-    if (g.debug_timing && blockIdx.x == 0 && t == 0)
-      printf("wgrad transform (CTA 0, %d chunks): per chunk waits raw %lld, waits op stage %lld, works %lld cycles\n", (int)it,
-             tw_raw / max(1u, it), tw_op / max(1u, it), tw_work / max(1u, it));
     if (g.db) {  // the 8 row-group threads (kg = lane & 7) of a column group are adjacent lanes
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
@@ -1046,24 +919,18 @@ __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g)
   } else if (warp == 8) {
     // ============================== MMA issuer (all lanes run the loop; one is elected per instruction) ==============
     {
-      const uint32_t idesc = make_idesc(kBlockM, g.Kx, 0, 0);
+      const uint32_t idesc = make_idesc(kBlockM, g.Kx);
       const uint32_t base = smem_u32(sOp);
       uint32_t it = 0, fl = 0;
-      long long tm_wait = 0, tm_acc = 0;
-      const long long tm0 = clock64();
       for (int64_t c = c_beg; c < c_end; ++fl) {
         const int acc = fl & 1;
-        const long long qa = clock64();
         mbar_wait(&tempty[acc], ((fl >> 1) & 1) ^ 1);
-        tm_acc += clock64() - qa;
         tc_fence_after();
-        const uint32_t d = tmem_base + acc * acc_cols, dc = g.one_acc ? d : d + g.Kx;
+        const uint32_t d = tmem_base + acc * acc_cols, dc = d + g.Kx;
         const int64_t c_stop = min(c_end, c + kFlush);
         for (int first = 1; c < c_stop; ++c, ++it) {
           const int s = it % S;
-          const long long qb = clock64();
           mbar_wait(&op_full[s], (it / S) & 1);
-          tm_wait += clock64() - qb;
           tc_fence_after();
           const uint32_t a_hi = base + s * op_stage, a_lo = a_hi + opA, b_hi = a_hi + (g.x3 ? 2 : 1) * opA, b_lo = b_hi + opB;
           // (a K step of 8 tf32 = 32 B inside the swizzled row: + 2 in the descriptor's 16-byte address field)
@@ -1074,7 +941,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g)
             if (elect_one()) {
               umma_tf32(d, dAh, dBh, idesc, !first);
               if (g.x3) {
-                umma_tf32(dc, dAl, dBh, idesc, g.one_acc ? 1 : !first);
+                umma_tf32(dc, dAl, dBh, idesc, !first);
                 umma_tf32(dc, dAh, dBl, idesc, 1);
               }
             }
@@ -1084,8 +951,6 @@ __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g)
         }
         if (elect_one()) umma_commit(&tfull[acc]);
       }
-      if (g.debug_timing && blockIdx.x == 0 && lane == 0)
-        printf("wgrad MMA issuer (CTA 0): %lld cycles in all, waits for operands %lld, for a free accumulator %lld\n", clock64() - tm0, tm_wait, tm_acc);
     }
     __syncwarp();
   } else {
@@ -1107,7 +972,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g)
           tmem_ld32(t0 + c0, v);
 #pragma unroll
           for (int j = 0; j < 32; ++j) sum[c0 + j] += v[j];
-          if (g.x3 && !g.one_acc) {
+          if (g.x3) {
             tmem_ld32(t0 + g.Kx + c0, v);
 #pragma unroll
             for (int j = 0; j < 32; ++j) sum[c0 + j] += v[j];
@@ -1119,242 +984,6 @@ __global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad(const WgradArgs g)
     }
     const int n = warp * 32 + lane;
     float* pp = g.part + (size_t)blockIdx.x * g.Kx * 128 + n;   // [cta][j][n]: coalesced over the 128 rows n
-#pragma unroll
-    for (int j = 0; j < kMaxCols; ++j)
-      if (j < g.Kx) pp[(size_t)j * 128] = sum[j];
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 8) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, tmem_cols);
-  }
-}
-
-// =================================================================================================
-// Kernel 2b: the weight gradient with MN-MAJOR operands (3xTF32 mode).
-// tcgen05 accepts MN-major shared-memory operands for TF32 (instruction descriptor bits 15 / 16), and both operands of
-// dW = dY^T X are MN-major as they lie in HBM: A[n, m] = dY[m, n] has n contiguous, B[k, m] = X[m, k] has k contiguous.
-// So the loaders write every 32-row chunk straight into the canonical MN-major SWIZZLE_128B layout
-//   [32-column block][4-row group][row in group: 128 B, 32-byte chunks XOR-swizzled by the row]   (LBO = 4096, SBO = 512)
-// and the MMAs read that raw tile as the `hi` operand (the tensor core ignores the 13 low mantissa bits: exactly the
-// hi = trunc(x) of the split).  The transform warps only compute lo = trunc(x - trunc(x)) — an elementwise pass into a
-// second ring — and the column sums of dY: no register transposes, no `hi` stores, and the per-chunk latency of the
-// transform stage (the bottleneck of k_tc_wgrad: ~1.5 us x 53 chunks per CTA at E rows) drops accordingly.
-// Shared memory: Rr raw stages (dY + X chunk, in flight / being multiplied) + S lo stages.
-// =================================================================================================
-// MN-major 32-bit operands take the 32-byte-base 128 B swizzle (cute::UMMA::LayoutType::SWIZZLE_128B_BASE32B = 1,
-// Layout_MN_SW128_32B_Atom): atom = 4 K-rows of 128 B (32 elements along M / N), the 32-byte chunk q of row r stored at
-// chunk q ^ (r & 3); 4-row groups SBO = 512 B apart, 32-element blocks LBO apart.
-__device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)(4096 >> 4) << 16;  // leading byte offset: next 32-element block along M / N
-  d |= (uint64_t)(512 >> 4) << 32;   // stride byte offset: next 4-row group along K
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)1 << 61;
-  return d;
-}
-// byte offset of the 16-byte piece `pc` (4 columns) of row m (0..31) inside a 32-row MN-major chunk tile
-__device__ __forceinline__ uint32_t mn_off(int m, int pc) {
-  const int p = pc & 7;
-  return (uint32_t)(pc >> 3) * 4096u + (uint32_t)(m >> 2) * 512u + (uint32_t)(m & 3) * 128u + (uint32_t)(((p >> 1) ^ (m & 3)) << 5) +
-         (uint32_t)(p & 1) * 16u;
-}
-
-__global__ void __launch_bounds__(kRowsThreads, 1) k_tc_wgrad_mn(const WgradArgs g) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rawA = kChunkK * 512, rawB = kChunkK * g.Kx * 4;  // chunk tile bytes (dY: 128 cols, X: Kx cols)
-  const uint32_t raw_stage = rawA + rawB;
-  const int Rr = g.raw_stages, S = g.op_stages;
-  uint8_t* sRaw = smem_raw;
-  uint8_t* sLo = sRaw + (size_t)Rr * raw_stage;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sLo + (size_t)S * raw_stage);
-  uint64_t* raw_full = bars;             // [Rr] loaders -> transform
-  uint64_t* raw_empty = raw_full + Rr;   // [Rr] MMA (commit) -> loaders
-  uint64_t* op_full = raw_empty + Rr;    // [S]  transform -> MMA  (lo written; implies the raw stage has landed)
-  uint64_t* op_empty = op_full + S;      // [S]  MMA (commit) -> transform
-  uint64_t* tfull = op_empty + S;        // [2]
-  uint64_t* tempty = tfull + 2;          // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
-  float* s_cs = reinterpret_cast<float*>(tmem_slot + 4);  // [4][128] column-sum partials of the transform warps
-  constexpr int kFlush = 8;
-  const uint32_t acc_cols = 2 * g.Kx;
-  const uint32_t need_cols = 2 * acc_cols;
-  const uint32_t tmem_cols = need_cols <= 32 ? 32 : need_cols <= 64 ? 64 : need_cols <= 128 ? 128 : need_cols <= 256 ? 256 : 512;
-  const int64_t nchunks = (g.M + kChunkK - 1) / kChunkK;
-  const int64_t per = (nchunks + gridDim.x - 1) / gridDim.x;
-  const int64_t c_beg = min(nchunks, (int64_t)blockIdx.x * per), c_end = min(nchunks, c_beg + per);
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < Rr; ++s) {
-      mbar_init(&raw_full[s], kLoadWarps * 32);
-      mbar_init(&raw_empty[s], 1);
-    }
-    for (int s = 0; s < S; ++s) {
-      mbar_init(&op_full[s], 4 * 32);
-      mbar_init(&op_empty[s], 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(&tfull[a], 1);
-      mbar_init(&tempty[a], kEpiWarps * 32);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, tmem_cols);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  pdl_trigger();
-  pdl_wait();  // (set-up above overlaps the previous kernel's tail)
-  if (c_beg >= c_end) {  // more CTAs than row chunks: nothing to do but to zero this CTA's partial slot
-    for (int i = threadIdx.x; i < g.Kx * 128; i += kRowsThreads) g.part[(size_t)blockIdx.x * g.Kx * 128 + i] = 0.f;
-    if (g.db && threadIdx.x < 128) g.part[(size_t)gridDim.x * g.Kx * 128 + (size_t)blockIdx.x * 128 + threadIdx.x] = 0.f;
-    __syncthreads();
-    if (warp == 8) tmem_dealloc(tmem_base, tmem_cols);
-    return;
-  }
-
-  if (warp >= 9) {
-    // ============================== loader warps ==============================
-    // lanes 0-7 of an instruction copy 8 consecutive 16-byte pieces of one row (one 128-byte line of HBM) into the 128-byte
-    // row (m & 7) of one 32-column block: conflict free on both sides
-    const int lw = warp - 9, r_in = lane >> 3, pl = lane & 7;
-    const uint32_t raw_base = smem_u32(sRaw);
-    const int pgB = g.Kx / 32;  // 32-column blocks per X row
-    uint32_t it = 0;
-    for (int64_t c = c_beg; c < c_end; ++c, ++it) {
-      const int s = it % Rr;
-      mbar_wait(&raw_empty[s], ((it / Rr) & 1) ^ 1);
-      const uint32_t dA = raw_base + s * raw_stage, dB = dA + rawA;
-      const int64_t m0 = c * kChunkK;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {   // dY: 32 rows x 4 blocks; this warp: rows 8 lw .. 8 lw + 7
-        const int r = 8 * lw + (j & 1) * 4 + r_in, pg = j >> 1;
-        const bool ok = m0 + r < g.M;
-        cp_async16(dA + mn_off(r, pg * 8 + pl), ok ? g.dY + (m0 + r) * g.ldy + (pg * 8 + pl) * 4 : g.dY, ok ? 16u : 0u);
-      }
-      for (int j = 0; j < 2 * pgB; ++j) {
-        const int r = 8 * lw + (j & 1) * 4 + r_in, pg = j >> 1;
-        const bool ok = m0 + r < g.M;
-        cp_async16(dB + mn_off(r, pg * 8 + pl), ok ? g.X + (m0 + r) * g.ldx + (pg * 8 + pl) * 4 : g.X, ok ? 16u : 0u);
-      }
-      cp_async_arrive(&raw_full[s]);
-    }
-  } else if (warp >= 4 && warp < 8) {
-    // ============================== transform warps: lo = trunc(x - trunc(x)), column sums of dY ==============
-    // thread t: 4-column piece pc = t % 32 (+ 32 j for X), rows m = t / 32 + 4 i  ->  every thread sums the same four
-    // dY columns over its rows; the four warps' partials meet once at the end
-    const int t = threadIdx.x - 128;
-    const int pc0 = t & 31, mrow = t >> 5;
-    const int pgB = g.Kx / 32;
-    float4 colsum = make_float4(0.f, 0.f, 0.f, 0.f);
-    uint32_t it = 0;
-    for (int64_t c = c_beg; c < c_end; ++c, ++it) {
-      const int r = it % Rr, s = it % S;
-      mbar_wait(&raw_full[r], (it / Rr) & 1);
-      mbar_wait(&op_empty[s], ((it / S) & 1) ^ 1);
-      const uint8_t* rA = sRaw + (size_t)r * raw_stage;
-      const uint8_t* rB = rA + rawA;
-      uint8_t* lA = sLo + (size_t)s * raw_stage;
-      uint8_t* lB = lA + rawA;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const uint32_t off = mn_off(mrow + 4 * i, pc0);
-        const float4 v = *reinterpret_cast<const float4*>(rA + off);
-        colsum = make_float4(colsum.x + v.x, colsum.y + v.y, colsum.z + v.z, colsum.w + v.w);
-        float4 hi, lo;
-        split4(v, hi, lo);
-        *reinterpret_cast<float4*>(lA + off) = lo;
-      }
-      for (int jb = 0; jb < pgB / 4 + (pgB % 4 != 0); ++jb) {  // X: Kx / 4 pieces per row, 32 per pass
-        const int pc = pc0 + 32 * jb;
-        if (pc < g.Kx / 4) {
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const uint32_t off = mn_off(mrow + 4 * i, pc);
-            float4 hi, lo;
-            split4(*reinterpret_cast<const float4*>(rB + off), hi, lo);
-            *reinterpret_cast<float4*>(lB + off) = lo;
-          }
-        }
-      }
-      fence_proxy_async();
-      mbar_arrive(&op_full[s]);
-    }
-    if (g.db) {
-      *reinterpret_cast<float4*>(s_cs + mrow * 128 + pc0 * 4) = colsum;
-      asm volatile("bar.sync 2, 128;" ::: "memory");
-      if (t < 32) {
-        const float4 a = *reinterpret_cast<const float4*>(s_cs + t * 4), b = *reinterpret_cast<const float4*>(s_cs + 128 + t * 4);
-        const float4 c2 = *reinterpret_cast<const float4*>(s_cs + 256 + t * 4), d2 = *reinterpret_cast<const float4*>(s_cs + 384 + t * 4);
-        *reinterpret_cast<float4*>(g.part + (size_t)gridDim.x * g.Kx * 128 + (size_t)blockIdx.x * 128 + t * 4) =
-            make_float4((a.x + b.x) + (c2.x + d2.x), (a.y + b.y) + (c2.y + d2.y), (a.z + b.z) + (c2.z + d2.z), (a.w + b.w) + (c2.w + d2.w));
-      }
-    }
-  } else if (warp == 8) {
-    // ============================== MMA issuer ==============================
-    if (lane == 0) {
-      const uint32_t idesc = make_idesc(kBlockM, g.Kx, 1, 1);  // both operands MN-major
-      const uint32_t rbase = smem_u32(sRaw), lbase = smem_u32(sLo);
-      uint32_t it = 0, fl = 0;
-      for (int64_t c = c_beg; c < c_end; ++fl) {
-        const int acc = fl & 1;
-        mbar_wait(&tempty[acc], ((fl >> 1) & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t d = tmem_base + acc * acc_cols, dc = d + g.Kx;
-        const int64_t c_stop = min(c_end, c + kFlush);
-        for (int first = 1; c < c_stop; ++c, ++it) {
-          const int r = it % Rr, s = it % S;
-          mbar_wait(&op_full[s], (it / S) & 1);
-          tc_fence_after();
-          const uint32_t a_hi = rbase + r * raw_stage, b_hi = a_hi + rawA, a_lo = lbase + s * raw_stage, b_lo = a_lo + rawA;
-#pragma unroll
-          for (int kk = 0; kk < kChunkK / 8; ++kk) {  // two 4-row groups per MMA
-            const uint64_t dAh = make_desc_mn_sw128(a_hi + kk * 1024), dBh = make_desc_mn_sw128(b_hi + kk * 1024);
-            umma_tf32(d, dAh, dBh, idesc, !first);
-            umma_tf32(dc, make_desc_mn_sw128(a_lo + kk * 1024), dBh, idesc, !first);
-            umma_tf32(dc, dAh, make_desc_mn_sw128(b_lo + kk * 1024), idesc, 1);
-            first = 0;
-          }
-          umma_commit(&raw_empty[r]);
-          umma_commit(&op_empty[s]);
-        }
-        umma_commit(&tfull[acc]);
-      }
-    }
-    __syncwarp();
-  } else {
-    // ============================== epilogue warps (as in k_tc_wgrad) ==============================
-    constexpr int kMaxCols = 128;
-    float sum[kMaxCols];
-#pragma unroll
-    for (int j = 0; j < kMaxCols; ++j) sum[j] = 0.f;
-    const int64_t n_flush = (c_end - c_beg + kFlush - 1) / kFlush;
-    for (int64_t fl = 0; fl < n_flush; ++fl) {
-      const int acc = fl & 1;
-      mbar_wait(&tfull[acc], (fl >> 1) & 1);
-      tc_fence_after();
-      const uint32_t t0 = tmem_base + ((uint32_t)(warp * 32) << 16) + acc * acc_cols;
-#pragma unroll
-      for (int c0 = 0; c0 < kMaxCols; c0 += 32) {
-        if (c0 < g.Kx) {
-          float v[32];
-          tmem_ld32(t0 + c0, v);
-#pragma unroll
-          for (int j = 0; j < 32; ++j) sum[c0 + j] += v[j];
-          tmem_ld32(t0 + g.Kx + c0, v);
-#pragma unroll
-          for (int j = 0; j < 32; ++j) sum[c0 + j] += v[j];
-        }
-      }
-      tc_fence_before();
-      mbar_arrive(&tempty[acc]);
-    }
-    const int n = warp * 32 + lane;
-    float* pp = g.part + (size_t)blockIdx.x * g.Kx * 128 + n;
 #pragma unroll
     for (int j = 0; j < kMaxCols; ++j)
       if (j < g.Kx) pp[(size_t)j * 128] = sum[j];
@@ -1453,10 +1082,6 @@ int lcao_tc_rows(const float* A, int64_t lda, const float* W, int64_t ldw, int b
   g.x3 = x3;
   g.wide_store = ((reinterpret_cast<uintptr_t>(Y) | (uintptr_t)(ldy * 4)) & 31u) == 0 &&
                  (!pre || ((reinterpret_cast<uintptr_t>(pre) | (uintptr_t)(ldp * 4)) & 31u) == 0);
-  static const int dbg = getenv("LCAO_TC_DEBUG") ? atoi(getenv("LCAO_TC_DEBUG")) : 0;
-  g.debug = dbg;
-  static const int one_acc = getenv("LCAO_TC_ONEACC") ? atoi(getenv("LCAO_TC_ONEACC")) : 0;
-  g.one_acc = x3 ? one_acc : 0;
   // the 3xTF32 weight (hi + lo) takes 128 KB at K = N = 128: 6 operand stages of 16 KB remain -> 3 hi + 3 lo
   int lo_stages = x3 ? 3 : 0;
   int stages = 8;
@@ -1471,43 +1096,34 @@ int lcao_tc_rows(const float* A, int64_t lda, const float* W, int64_t ldw, int b
   const size_t smem = rows_smem(Kc, Nb, stages, lo_stages);
   static bool attr_set = false;
   if (!attr_set) {
-    LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
     attr_set = true;
   }
-  static const int rp = getenv("LCAO_TC_RP") ? atoi(getenv("LCAO_TC_RP")) : 0;
   const int64_t nblocks = (M + kBlockM - 1) / kBlockM;
   const unsigned grid = (unsigned)(nblocks < num_sms() ? nblocks : num_sms());
   // eight epilogue warps pay when a CTA has a single tile (node- and table-sized layers: the drain is on the critical
   // path, 20.5 -> 18.4 us); with many tiles per CTA the drain overlaps the next tile's MMAs and they do not (85 -> 88 us)
-  static const int epi8_env = getenv("LCAO_TC_EPI8") ? atoi(getenv("LCAO_TC_EPI8")) : -1;
-  const bool epi8 = epi8_env >= 0 ? epi8_env != 0 : nblocks <= num_sms();
+  const bool epi8 = nblocks <= num_sms();
   // many tiles per CTA in 3xTF32 mode: the A-operand-in-tensor-memory kernel (twice the bytes in flight)
-  static const int ta_env = getenv("LCAO_TC_TA") ? atoi(getenv("LCAO_TC_TA")) : 1;
-  if (ta_env && x3 && !rp && nblocks >= 2 * num_sms() && Nb <= 128 && Kc % kChunkK == 0 &&
+  if (x3 && nblocks >= 2 * num_sms() && Nb <= 128 && Kc % kChunkK == 0 &&
       2 * (size_t)(Kc / kChunkK) * Nb * 128 + 3 * kStageBytes + 512 + 1024 <= kMaxSmem) {
     static bool ta_attr = false;
     if (!ta_attr) {
-      LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows_ta<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-      LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows_ta<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+      LCAO_CUDA(cudaFuncSetAttribute(k_tc_rows_ta, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
       ta_attr = true;
     }
     const size_t halfB = (size_t)(Kc / kChunkK) * Nb * 128;
-    static const int cps_env = getenv("LCAO_TC_TA_CPS") ? atoi(getenv("LCAO_TC_TA_CPS")) : 1;  // (2 measured slower in the step: 9.47 vs 9.34 ms)
-    const int cps = (cps_env == 2 && Kc % (2 * kChunkK) == 0) ? 2 : 1;
     int R = 8;
-    while (R > 2 && 2 * halfB + (size_t)R * cps * kStageBytes + 512 + 1024 > kMaxSmem) --R;
+    while (R > 2 && 2 * halfB + (size_t)R * kStageBytes + 512 + 1024 > kMaxSmem) --R;
     g.stages = R;
-    const size_t smem_ta = 2 * halfB + (size_t)R * cps * kStageBytes + 512 + 1024;
-    if (cps == 2) LCAO_CUDA(launch_pdl(k_tc_rows_ta<2>, grid, kTaThreads, smem_ta, st, g));
-    else LCAO_CUDA(launch_pdl(k_tc_rows_ta<1>, grid, kTaThreads, smem_ta, st, g));
+    const size_t smem_ta = 2 * halfB + (size_t)R * kStageBytes + 512 + 1024;
+    LCAO_CUDA(launch_pdl(k_tc_rows_ta, grid, kTaThreads, smem_ta, st, g));
     LCAO_LAUNCH_CHECK();
     return LCAO_OK;
   }
-  if (rp) LCAO_CUDA(launch_pdl(k_tc_rows<true, false>, grid, kRowsThreads, smem, st, g));
-  else if (epi8) LCAO_CUDA(launch_pdl(k_tc_rows<false, true>, grid, kRowsThreads + 128, smem, st, g));
-  else LCAO_CUDA(launch_pdl(k_tc_rows<false, false>, grid, kRowsThreads, smem, st, g));
+  if (epi8) LCAO_CUDA(launch_pdl(k_tc_rows<true>, grid, kRowsThreads + 128, smem, st, g));
+  else LCAO_CUDA(launch_pdl(k_tc_rows<false>, grid, kRowsThreads, smem, st, g));
   LCAO_LAUNCH_CHECK();
   return LCAO_OK;
 }
@@ -1537,10 +1153,6 @@ int lcao_tc_wgrad(const float* dY, int64_t ldy, const float* X, int64_t ldx, flo
   WgradArgs g{};
   g.dY = dY; g.ldy = ldy; g.X = X; g.ldx = ldx; g.dW = dW; g.ldw = ldw; g.db = db; g.part = part;
   g.M = M; g.Kx = Kx; g.x3 = x3;
-  static const int one_acc_w = getenv("LCAO_TC_ONEACC") ? atoi(getenv("LCAO_TC_ONEACC")) : 0;
-  g.one_acc = x3 ? one_acc_w : 0;
-  static const int dbg_w = getenv("LCAO_TC_DEBUG") ? atoi(getenv("LCAO_TC_DEBUG")) : 0;
-  g.debug_timing = (dbg_w & 64) != 0;
   g.op_stages = 2;
   int raw_stages = 6;
   while (raw_stages > 2 && wgrad_smem(Kx, x3, raw_stages, g.op_stages) > kMaxSmem) --raw_stages;
@@ -1551,23 +1163,6 @@ int lcao_tc_wgrad(const float* dY, int64_t ldy, const float* X, int64_t ldx, flo
     attr_set = true;
   }
   const unsigned grid = wgrad_grid(M);
-  static const int mn_env = getenv("LCAO_TC_WGRAD_MN") ? atoi(getenv("LCAO_TC_WGRAD_MN")) : 0;  // (experiment: correct, 91-95 us vs 85 us at E rows)
-  if (mn_env && x3 && Kx % 32 == 0) {
-    // MN-major operands: raw stages (dY + X chunk) are the `hi` operands, lo stages beside them
-    static bool mn_attr = false;
-    if (!mn_attr) {
-      LCAO_CUDA(cudaFuncSetAttribute(k_tc_wgrad_mn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-      mn_attr = true;
-    }
-    const size_t stage = (size_t)kChunkK * (512 + Kx * 4);
-    static const int s_env = getenv("LCAO_TC_WGRAD_S") ? atoi(getenv("LCAO_TC_WGRAD_S")) : 3;
-    int S = s_env >= 2 && s_env <= 4 ? s_env : 3, Rr = 8;
-    while (Rr > 2 && (size_t)(Rr + S) * stage + 2048 + 1024 + 1024 > kMaxSmem) --Rr;
-    if (Rr < 3) { S = 2; Rr = 8; while (Rr > 2 && (size_t)(Rr + S) * stage + 2048 + 1024 + 1024 > kMaxSmem) --Rr; }
-    g.raw_stages = Rr;
-    g.op_stages = S;
-    LCAO_CUDA(launch_pdl(k_tc_wgrad_mn, grid, kRowsThreads, (size_t)(Rr + S) * stage + 2048 + 1024 + 1024, st, g));
-  } else
   LCAO_CUDA(launch_pdl(k_tc_wgrad, grid, kRowsThreads, wgrad_smem(Kx, x3, raw_stages, g.op_stages), st, g));
   LCAO_LAUNCH_CHECK();
   if (defer_desc) {  // stage 2 is left to lcao_wgrad_reduce_batch: {part, dW, db, ldw, ncta, Kx}

@@ -14,7 +14,10 @@
 // (the reference's (T,O,C) gather, cos(theta), Y_l(T,O)) exists; cos(theta) = unit[e].unit[e'] and Y_l
 // are recomputed per (e,e') pair by one thread and broadcast through shared memory.
 //
-// Thread mapping: lane <-> float4 channel column (C = 128 -> 32 lanes), warp <-> 8 out-edges of a node
+// These FP32-pipe kernels serve 128 < C <= 256; C <= 128 goes to threebody_mma.cu (forward) and threebody_staged.cu
+// (backward).  Both entry points require 16-byte-aligned B, gate and d_tbw: every kernel reads them in float4 rows.
+//
+// Thread mapping: lane <-> float4 channel columns (lane and lane + 32), warp <-> 8 out-edges of a node
 // (forward: 8 register accumulators) or one in-edge (backward).  Warps are independent: B / gate / d_tbw
 // rows are read straight from global memory (L1/L2 serve the re-reads by the sibling warps of the same
 // node), the per-pair coefficients are computed by the lanes of the warp itself (one pair per lane)
@@ -24,8 +27,6 @@
 // written once: no atomics, deterministic.
 //
 // `gate` is sigmoid(xk) per NODE (N x C, computed once per layer by lcao_sigmoid_rows).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tb_common.cuh"
 
@@ -35,6 +36,8 @@ constexpr int kFwdWarps = 2;   // forward CTA: 2 warps x 8 out-edges per pass
 constexpr int kBwdWarps = 4;   // backward CTA: 4 warps, one in-edge per warp at a time (2 measured slower: 168 vs 128 registers)
 constexpr int kR = 8;          // forward: out-edge accumulators per warp
 constexpr int kIB = 4;         // forward: in-edges per coefficient batch (kR * kIB = 32 pairs = one per lane)
+constexpr int kV4 = 2;         // float4 channel columns per lane: these kernels serve 128 < C <= 256
+constexpr int kFwdCtasPerSm = 48, kBwdCtasPerSm = 24;  // grid caps (grid-stride over the centre nodes)
 
 // (Packed FP32 pairs — fma.rn.f32x2 / FFMA2 — were tried for the FMA blocks: same FP32 pipe rate (measured 36.8 vs
 // 36.2 TFMA/s, scripts/micro/ffma2.cu) and the forward kernel ran 2x SLOWER with them; see profiles/r01_notes.md.)
@@ -48,31 +51,31 @@ constexpr int kIB = 4;         // forward: in-edges per coefficient batch (kR * 
 // FMA block of in-edges beyond the tail, per-row guards — removed up to 30 % of the issued FMAs and did not make the
 // kernel faster: it is bound by the latency of each warp's dependent chain, not by issue slots; profiles/r01_notes.md.)
 
-// One block of nr <= R out-edges (positions ob + jb ..) of a node against all its dI in-edges.
-template <int NL, int V4, bool FULL, int R, bool TGUARD, int HB>
+// One block of nr <= kR out-edges (positions ob + jb ..) of a node against all its dI in-edges.
+template <int NL>
 __device__ __forceinline__ void tb_fwd_block(const float* __restrict__ B, int NG, const double* __restrict__ gram,
                                              const float* __restrict__ unit, const float* __restrict__ gate, int64_t ldg,
                                              const int32_t* __restrict__ in_edge, const int32_t* __restrict__ in_src,
                                              const int32_t* __restrict__ out_edge, int C, float* __restrict__ tbw,
-                                             float* sa, int lane, const bool (&okc)[V4], int ib, int dI, int ob, int jb,
+                                             float* sa, int lane, const bool (&okc)[kV4], int ib, int dI, int ob, int jb,
                                              int nr) {
   constexpr int NP = NL * (NL + 1) / 2;
-  const int r_mine = lane % R, t_mine = lane / R;  // coefficient duty: pair (in-edge t, out-edge r); lanes with t >= kIB idle
+  const int r_mine = lane % kR, t_mine = lane / kR;  // coefficient duty: pair (in-edge t, out-edge r)
   // lane (r, t) keeps out-edge r of this block: id and direction
   const int e_mine = out_edge[ob + jb + min(r_mine, nr - 1)];
   const float ux = unit[3 * (int64_t)e_mine], uy = unit[3 * (int64_t)e_mine + 1], uz = unit[3 * (int64_t)e_mine + 2];
-  float4 acc[R][V4];
+  float4 acc[kR][kV4];
 #pragma unroll
-  for (int r = 0; r < R; ++r)
+  for (int r = 0; r < kR; ++r)
 #pragma unroll
-    for (int v = 0; v < V4; ++v) acc[r][v] = zero4();
+    for (int v = 0; v < kV4; ++v) acc[r][v] = zero4();
 
   for (int ic = 0; ic < dI; ic += 32) {  // the node's in-edge ids, 32 at a time, one per lane
     const int nI = min(32, dI - ic);
     const int my_ep = in_edge[ib + ic + min(lane, nI - 1)];
     const int my_k = in_src[ib + ic + min(lane, nI - 1)];
     for (int i0 = 0; i0 < nI; i0 += kIB) {
-      // ---- coefficients of the R x 4 pairs of this batch, one per lane
+      // ---- coefficients of the kR x kIB pairs of this batch, one per lane
       const int ep_c = __shfl_sync(0xffffffffu, my_ep, min(i0 + t_mine, nI - 1));
       float4 a = zero4();
       {
@@ -87,52 +90,45 @@ __device__ __forceinline__ void tb_fwd_block(const float* __restrict__ B, int NG
         a = make_float4(w * Y[0], w * Y[1], w * Y[2], w * Y[3]);
       }
       __syncwarp();  // previous batch's readers are done
-      if (R == 8 || t_mine < kIB) st4(sa + (t_mine * 8 + r_mine) * 4, a);
+      st4(sa + (t_mine * 8 + r_mine) * 4, a);
       __syncwarp();
-      // ---- rows of the batch: issue every load first, then the FMAs (HB in-edges at a time: HB = 2 halves the row
-      //      registers, which buys resident warps)
-#pragma unroll 1
-      for (int h0 = 0; h0 < kIB; h0 += HB) {
-        if (TGUARD && h0 > 0 && i0 + h0 >= nI) break;  // warp-uniform
-        float4 gb[HB][NL][V4];
+      // ---- rows of the batch: issue every load first, then the FMAs
+      float4 gb[kIB][NL][kV4];
 #pragma unroll
-        for (int t = 0; t < HB; ++t) {
-          const int src = min(i0 + h0 + t, nI - 1);
-          const int ep = __shfl_sync(0xffffffffu, my_ep, src);
-          const int k = __shfl_sync(0xffffffffu, my_k, src);
+      for (int t = 0; t < kIB; ++t) {
+        const int src = min(i0 + t, nI - 1);
+        const int ep = __shfl_sync(0xffffffffu, my_ep, src);
+        const int k = __shfl_sync(0xffffffffu, my_k, src);
 #pragma unroll
-          for (int v = 0; v < V4; ++v) {
-            const int c = (lane + 32 * v) * 4;
-            const float4 gt = okc[v] ? ldg4(gate + (int64_t)k * ldg + c) : zero4();
+        for (int v = 0; v < kV4; ++v) {
+          const int c = (lane + 32 * v) * 4;
+          const float4 gt = okc[v] ? ldg4(gate + (int64_t)k * ldg + c) : zero4();
 #pragma unroll
-            for (int l = 0; l < NL; ++l) gb[t][l][v] = okc[v] ? mul4(gt, ldg4(B + ((int64_t)ep * NG + l) * C + c)) : zero4();
-          }
+          for (int l = 0; l < NL; ++l) gb[t][l][v] = okc[v] ? mul4(gt, ldg4(B + ((int64_t)ep * NG + l) * C + c)) : zero4();
         }
+      }
 #pragma unroll
-        for (int t = 0; t < HB; ++t) {
-          if (!TGUARD || t == 0 || i0 + h0 + t < nI) {  // warp-uniform
+      for (int t = 0; t < kIB; ++t) {
 #pragma unroll
-            for (int r = 0; r < R; ++r) {
-              const float4 ar = lds4(sa + ((h0 + t) * 8 + r) * 4);
+        for (int r = 0; r < kR; ++r) {
+          const float4 ar = lds4(sa + (t * 8 + r) * 4);
 #pragma unroll
-              for (int v = 0; v < V4; ++v) {
-                acc[r][v] = fma4(ar.x, gb[t][0][v], acc[r][v]);
-                if (NL > 1) acc[r][v] = fma4(ar.y, gb[t][1][v], acc[r][v]);
-                if (NL > 2) acc[r][v] = fma4(ar.z, gb[t][2][v], acc[r][v]);
-                if (NL > 3) acc[r][v] = fma4(ar.w, gb[t][3][v], acc[r][v]);
-              }
-            }
+          for (int v = 0; v < kV4; ++v) {
+            acc[r][v] = fma4(ar.x, gb[t][0][v], acc[r][v]);
+            if (NL > 1) acc[r][v] = fma4(ar.y, gb[t][1][v], acc[r][v]);
+            if (NL > 2) acc[r][v] = fma4(ar.z, gb[t][2][v], acc[r][v]);
+            if (NL > 3) acc[r][v] = fma4(ar.w, gb[t][3][v], acc[r][v]);
           }
         }
       }
     }
   }
 #pragma unroll
-  for (int r = 0; r < R; ++r) {
-    const int e = __shfl_sync(0xffffffffu, e_mine, r % R);
+  for (int r = 0; r < kR; ++r) {
+    const int e = __shfl_sync(0xffffffffu, e_mine, r);
     if (r < nr) {
 #pragma unroll
-      for (int v = 0; v < V4; ++v) {
+      for (int v = 0; v < kV4; ++v) {
         const int c = (lane + 32 * v) * 4;
         if (okc[v]) st4(tbw + (int64_t)e * C + c, acc[r][v]);
       }
@@ -140,12 +136,7 @@ __device__ __forceinline__ void tb_fwd_block(const float* __restrict__ B, int NG
   }
 }
 
-// L2 prefetch of `bytes` (multiple of 16) starting at the 16-byte aligned global address p: one instruction per row group
-__device__ __forceinline__ void prefetch_l2(const void* p, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
-
-template <int NL, int V4, bool FULL>
+template <int NL>
 __global__ void __launch_bounds__(kFwdWarps * 32, 8) k_threebody_fwd(
     const float* __restrict__ B, int NG, const double* __restrict__ gram, const float* __restrict__ unit,
     const float* __restrict__ gate, int64_t ldg, const int32_t* __restrict__ in_ptr,
@@ -155,15 +146,12 @@ __global__ void __launch_bounds__(kFwdWarps * 32, 8) k_threebody_fwd(
   __shared__ __align__(16) float s_a[kFwdWarps][32 * 4];  // per-warp coefficient scratch: pair (t, r) at slot t*8 + r
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* sa = s_a[warp];
-  bool okc[V4];
+  bool okc[kV4];
 #pragma unroll
-  for (int v = 0; v < V4; ++v) okc[v] = FULL || (lane + 32 * v) * 4 < C;
-  constexpr bool TG = false, PF = false;  // measured without effect (profiles/r01_notes.md): dead in-edge FMA blocks skipped, L2 prefetch of the next node's rows
+  for (int v = 0; v < kV4; ++v) okc[v] = (lane + 32 * v) * 4 < C;
 
-  // Grid-stride over the centre nodes as a three-deep software pipeline that takes the dependent latencies
-  // (row pointers -> edge ids -> rows) off every node's critical path: while node s is processed, the CSR row
-  // pointers of node s + 2G are fetched, and (PF) the in-edge ids of node s + G are read and its B / gate rows
-  // are pulled into L2 by bulk prefetches (one instruction per in-edge: its NL rows of B are contiguous).
+  // Grid-stride over the centre nodes as a software pipeline that takes the dependent latency of the CSR row
+  // pointers off every node's critical path: while node s is processed, the row pointers of node s + 2G are fetched.
   const int G = gridDim.x;
   int s = blockIdx.x;
   if (s >= N) return;
@@ -177,27 +165,11 @@ __global__ void __launch_bounds__(kFwdWarps * 32, 8) k_threebody_fwd(
       const int sn = s + 2 * G;
       f_ib = in_ptr[sn]; f_ie = in_ptr[sn + 1]; f_ob = out_ptr[sn]; f_oe = out_ptr[sn + 1];
     }
-    int pf_ep = -1, pf_k = 0;  // next node: in-edge lane * kFwdWarps + warp is this lane's to prefetch
-    if (PF) {
-      const int i = lane * kFwdWarps + warp;
-      if (i < n_ie - n_ib && n_oe > n_ob) { pf_ep = in_edge[n_ib + i]; pf_k = in_src[n_ib + i]; }
-    }
     // the node's out-edges are split into ceil(dO / 8) blocks of (almost) equal size <= 8, one block per warp and pass
     const int nblk = (dO + kR - 1) / kR, per = nblk ? (dO + nblk - 1) / nblk : 0;
     for (int blk = warp; blk < nblk; blk += kFwdWarps) {
       const int jb = blk * per, nr = min(per, dO - jb);
-#define TB_BLOCK(R) \
-  tb_fwd_block<NL, V4, FULL, R, TG, kIB>(B, NG, gram, unit, gate, ldg, in_edge, in_src, out_edge, C, tbw, sa, lane, okc, ib, dI, ob, jb, nr)
-      TB_BLOCK(8);
-#undef TB_BLOCK
-      if (PF && blk == warp && pf_ep >= 0) {
-        prefetch_l2(B + (int64_t)pf_ep * NG * C, (uint32_t)(NL * C * 4));
-        prefetch_l2(gate + (int64_t)pf_k * ldg, (uint32_t)(C * 4));
-      }
-    }
-    if (PF && warp >= nblk && pf_ep >= 0) {  // this warp had no block of the node
-      prefetch_l2(B + (int64_t)pf_ep * NG * C, (uint32_t)(NL * C * 4));
-      prefetch_l2(gate + (int64_t)pf_k * ldg, (uint32_t)(C * 4));
+      tb_fwd_block<NL>(B, NG, gram, unit, gate, ldg, in_edge, in_src, out_edge, C, tbw, sa, lane, okc, ib, dI, ob, jb, nr);
     }
     c_ib = n_ib; c_ie = n_ie; c_ob = n_ob; c_oe = n_oe;
     n_ib = f_ib; n_ie = f_ie; n_ob = f_ob; n_oe = f_oe;
@@ -213,7 +185,7 @@ __global__ void __launch_bounds__(kFwdWarps * 32, 8) k_threebody_fwd(
 //   FORCES: dc = Gt[j,:] . sum_l (w Y'_l) GB[i,l,:] - w^2 dot sum_l Y'_l (G Y)_l ;  d unit[e_j] += dc unit[e_i] and v.v.
 // Same clamping convention as the forward: dead slots read a valid row and carry zero coefficients.
 // ---------------------------------------------------------------------------------------------
-template <int NL, int V4, bool FORCES, bool FULL, bool GUARD>
+template <int NL, bool FORCES, bool FULL>
 __global__ void __launch_bounds__(kBwdWarps * 32) k_threebody_bwd(
     const float* __restrict__ B, int NG, const double* __restrict__ gram, const float* __restrict__ unit,
     const float* __restrict__ gate, int64_t ldg, const int32_t* __restrict__ in_ptr,
@@ -267,16 +239,16 @@ __global__ void __launch_bounds__(kBwdWarps * 32) k_threebody_bwd(
   float* sa = s_a[warp];
   float* sf = s_f[warp];
   const int jsub = bfly8_index(lane);
-  bool okc[V4];
+  bool okc[kV4];
 #pragma unroll
-  for (int v = 0; v < V4; ++v) okc[v] = FULL || (lane + 32 * v) * 4 < C;
+  for (int v = 0; v < kV4; ++v) okc[v] = FULL || (lane + 32 * v) * 4 < C;
 
   for (int i = warp; i < dI; i += kBwdWarps) {  // one in-edge per warp at a time
     const int ep = in_edge[ib + i], k = in_src[ib + i];
-    float4 gb[NL][V4], dacc[NL][V4], gt[V4];
+    float4 gb[NL][kV4], dacc[NL][kV4], gt[kV4];
     float h[NP];
 #pragma unroll
-    for (int v = 0; v < V4; ++v) {
+    for (int v = 0; v < kV4; ++v) {
       const int c = (lane + 32 * v) * 4;
       gt[v] = okc[v] ? ldg4(gate + (int64_t)k * ldg + c) : zero4();
 #pragma unroll
@@ -316,18 +288,14 @@ __global__ void __launch_bounds__(kBwdWarps * 32) k_threebody_bwd(
       __syncwarp();
       for (int j0 = 0; j0 < nO; j0 += 8) {
         const int nj = min(8, nO - j0);
-        // ---- d_tbw rows of the batch (all loads first).  GUARD: dead slots (jj >= nj) are SKIPPED by warp-uniform
-        //      branches (a clamped slot costs as many issue slots as a live one) and the coefficients are fetched one
-        //      slot ahead, so that no block starts by waiting on shared memory; !GUARD: dead slots read a clamped row
-        //      and carry zero coefficients (branch-free)
-        float4 gr[8][V4];
+        // ---- d_tbw rows of the batch (all loads first); dead slots (jj >= nj) read a clamped row and carry zero
+        //      coefficients (branch-free)
+        float4 gr[8][kV4];
 #pragma unroll
         for (int jj = 0; jj < 8; ++jj) {
-          if (!GUARD || jj < nj) {
-            const int e = __shfl_sync(0xffffffffu, my_ej, GUARD ? j0 + jj : min(j0 + jj, nO - 1));
+          const int e = __shfl_sync(0xffffffffu, my_ej, min(j0 + jj, nO - 1));
 #pragma unroll
-            for (int v = 0; v < V4; ++v) gr[jj][v] = okc[v] ? ldg4(d_tbw + (int64_t)e * C + (lane + 32 * v) * 4) : zero4();
-          }
+          for (int v = 0; v < kV4; ++v) gr[jj][v] = okc[v] ? ldg4(d_tbw + (int64_t)e * C + (lane + 32 * v) * 4) : zero4();
         }
         // FORCES needs two contractions of Gt with the in-edge's rows per pair (weights w Y_l and w Y'_l): instead of
         // forming both combined rows, the NL dots D_l = Gt . GB_l are taken once (NL FMAs per channel) and both scalars
@@ -336,42 +304,34 @@ __global__ void __launch_bounds__(kBwdWarps * 32) k_threebody_bwd(
         float4 ar = lds4(sa + j0 * 4);
 #pragma unroll
         for (int jj = 0; jj < 8; ++jj) {
-          if constexpr (FORCES) {
+          const float4 ar_next = lds4(sa + (j0 + jj + 1) * 4);  // (one slot ahead: no block starts by waiting on shared memory)
+          float d = 0.f, dl[NL];
 #pragma unroll
-            for (int l = 0; l < NL; ++l) partD[l][jj] = 0.f;
-          } else {
-            part[jj] = 0.f;
-          }
-          if (!GUARD || jj < nj) {
-            const float4 ar_next = lds4(sa + (j0 + jj + 1) * 4);
-            float d = 0.f, dl[NL];
+          for (int l = 0; l < NL; ++l) dl[l] = 0.f;
 #pragma unroll
-            for (int l = 0; l < NL; ++l) dl[l] = 0.f;
-#pragma unroll
-            for (int v = 0; v < V4; ++v) {
-              if constexpr (FORCES) {
-#pragma unroll
-                for (int l = 0; l < NL; ++l) dl[l] += dot4(gb[l][v], gr[jj][v]);
-              } else {
-                float4 t = scale4(ar.x, gb[0][v]);
-                if (NL > 1) t = fma4(ar.y, gb[1][v], t);
-                if (NL > 2) t = fma4(ar.z, gb[2][v], t);
-                if (NL > 3) t = fma4(ar.w, gb[3][v], t);
-                d += dot4(t, gr[jj][v]);
-              }
-              dacc[0][v] = fma4(ar.x, gr[jj][v], dacc[0][v]);
-              if (NL > 1) dacc[1][v] = fma4(ar.y, gr[jj][v], dacc[1][v]);
-              if (NL > 2) dacc[2][v] = fma4(ar.z, gr[jj][v], dacc[2][v]);
-              if (NL > 3) dacc[3][v] = fma4(ar.w, gr[jj][v], dacc[3][v]);
-            }
+          for (int v = 0; v < kV4; ++v) {
             if constexpr (FORCES) {
 #pragma unroll
-              for (int l = 0; l < NL; ++l) partD[l][jj] = dl[l];
+              for (int l = 0; l < NL; ++l) dl[l] += dot4(gb[l][v], gr[jj][v]);
             } else {
-              part[jj] = d;
+              float4 t = scale4(ar.x, gb[0][v]);
+              if (NL > 1) t = fma4(ar.y, gb[1][v], t);
+              if (NL > 2) t = fma4(ar.z, gb[2][v], t);
+              if (NL > 3) t = fma4(ar.w, gb[3][v], t);
+              d += dot4(t, gr[jj][v]);
             }
-            ar = ar_next;
+            dacc[0][v] = fma4(ar.x, gr[jj][v], dacc[0][v]);
+            if (NL > 1) dacc[1][v] = fma4(ar.y, gr[jj][v], dacc[1][v]);
+            if (NL > 2) dacc[2][v] = fma4(ar.z, gr[jj][v], dacc[2][v]);
+            if (NL > 3) dacc[3][v] = fma4(ar.w, gr[jj][v], dacc[3][v]);
           }
+          if constexpr (FORCES) {
+#pragma unroll
+            for (int l = 0; l < NL; ++l) partD[l][jj] = dl[l];
+          } else {
+            part[jj] = d;
+          }
+          ar = ar_next;
         }
         // ---- per pair scalars: the quad `jsub` of the warp finishes pair (out j0 + jsub, this in-edge)
         float dotv, dot2v = 0.f;
@@ -454,7 +414,7 @@ __global__ void __launch_bounds__(kBwdWarps * 32) k_threebody_bwd(
         for (int y = x; y < NL; ++y) { H[x][y] = h[p]; H[y][x] = h[p]; ++p; }
     }
 #pragma unroll
-    for (int v = 0; v < V4; ++v) {
+    for (int v = 0; v < kV4; ++v) {
       const int c = (lane + 32 * v) * 4;
       if (okc[v]) {
         float4 b[NL];
@@ -490,41 +450,27 @@ __global__ void __launch_bounds__(kBwdWarps * 32) k_threebody_bwd(
   }
 }
 
-// tuning knob read once from the environment (benchmark sweeps); falls back to the default when out of range
-int tile_in(const char* env, int dflt, int lo, int hi) {
-  const char* s = getenv(env);
-  const int v = s ? atoi(s) : dflt;
-  return (v < lo || v > hi) ? dflt : v;
-}
-
 }  // namespace
 
-// warp-level tensor-core formulation with bulk-copy staging (threebody_mma.cu): the default forward for C <= 128
+// warp-level tensor-core formulation with bulk-copy staging (threebody_mma.cu): the forward for C <= 128
 int lcao_tb_mma_fwd(const float* B, int32_t NG, const double* gram, const float* unit, const float* gate, int64_t ldg,
                     const int32_t* in_ptr, const int32_t* in_edge, const int32_t* in_src, const int32_t* out_ptr,
                     const int32_t* out_edge, int64_t N, int32_t C, int32_t NL, float* tbw, cudaStream_t st);
-// staged backward (threebody_staged.cu): bulk-copy staging + producer warp, the default backward for C <= 128
+// staged backward (threebody_staged.cu): bulk-copy staging + producer warp, the backward for C <= 128
 int lcao_tb_staged_bwd(const float* B, int32_t NG, const double* gram, const float* unit, const float* gate, int64_t ldg,
                        const int32_t* in_ptr, const int32_t* in_edge, const int32_t* in_src, const int32_t* out_ptr,
                        const int32_t* out_edge, int64_t N, int32_t C, int32_t NL, const float* d_tbw, const float* dP,
                        float* dB, float* q, float* du_ks, float* du_st, cudaStream_t st);
-// LCAO_TB_IMPL=simt forces the FP32-pipe forward kernel of this file (A/B measurements); it also serves C > 128 and
-// buffers that are not 16-byte aligned (the bulk copies need that)
-static bool use_mma(int C, const void* B, const void* gate, int64_t ldg) {
-  static const bool simt = [] { const char* s = getenv("LCAO_TB_IMPL"); return s && s[0] == 's'; }();
-  return !simt && C <= 128 && ((reinterpret_cast<uintptr_t>(B) | reinterpret_cast<uintptr_t>(gate)) & 15u) == 0 && ldg % 4 == 0;
-}
 
-#define TB_DISPATCH(NL, V4, CALL)   \
-  switch ((NL) * 10 + (V4)) {       \
-    case 11: { CALL(1, 1); } break; \
-    case 12: { CALL(1, 2); } break; \
-    case 21: { CALL(2, 1); } break; \
-    case 22: { CALL(2, 2); } break; \
-    case 31: { CALL(3, 1); } break; \
-    case 32: { CALL(3, 2); } break; \
-    case 41: { CALL(4, 1); } break; \
-    default: { CALL(4, 2); } break; \
+// every kernel reads these rows with 16-byte loads or bulk copies
+static bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+#define TB_DISPATCH(NL, CALL)     \
+  switch (NL) {                   \
+    case 1: { CALL(1); } break;   \
+    case 2: { CALL(2); } break;   \
+    case 3: { CALL(3); } break;   \
+    default: { CALL(4); } break;  \
   }
 
 extern "C" int lcao_threebody_fwd(const float* B, int32_t NG, const double* gram, const float* unit, const float* gate,
@@ -536,15 +482,15 @@ extern "C" int lcao_threebody_fwd(const float* B, int32_t NG, const double* gram
                "lcao_threebody_fwd: null buffer");
   LCAO_REQUIRE(C % 4 == 0 && C > 0 && C <= 256 && NL >= 1 && NL <= 4 && NG >= NL && ldg % 4 == 0,
                "lcao_threebody_fwd: need C %% 4 == 0, C <= 256, 1 <= NL <= 4, NG >= NL (C=%d NL=%d NG=%d)", C, NL, NG);
+  LCAO_REQUIRE(al16(B) && al16(gate), "lcao_threebody_fwd: B and gate must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
-  if (use_mma(C, B, gate, ldg)) return lcao_tb_mma_fwd(B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr, out_edge, N, C, NL, tbw, st);
-  const int V4 = C <= 128 ? 1 : 2;
-  static const int per_sm_f = tile_in("LCAO_TB_GRID_FWD", 48, 1, 64);
-  const unsigned grid = (unsigned)(N < 148ll * per_sm_f ? N : 148ll * per_sm_f);
-  // (the predicate-free specialisation FULL measured SLOWER in the forward: 0.291 vs 0.260 ms)
-#define TB_FWD_ARGS B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr, out_edge, (int)N, C, tbw
-#define CALL(nl, v4) k_threebody_fwd<nl, v4, false><<<grid, kFwdWarps * 32, 0, st>>>(TB_FWD_ARGS)
-  TB_DISPATCH(NL, V4, CALL)
+  if (C <= 128) return lcao_tb_mma_fwd(B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr, out_edge, N, C, NL, tbw, st);
+  const unsigned grid = (unsigned)(N < 148ll * kFwdCtasPerSm ? N : 148ll * kFwdCtasPerSm);
+  // (unlike the backward, the forward has no predicate-free C == 256 specialisation: it measured SLOWER, 0.291 vs 0.260 ms)
+#define CALL(nl)                                                                                                   \
+  k_threebody_fwd<nl><<<grid, kFwdWarps * 32, 0, st>>>(B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr, \
+                                                        out_edge, (int)N, C, tbw)
+  TB_DISPATCH(NL, CALL)
 #undef CALL
   LCAO_LAUNCH_CHECK();
   return LCAO_OK;
@@ -562,30 +508,25 @@ extern "C" int lcao_threebody_bwd(const float* B, int32_t NG, const double* gram
                "lcao_threebody_bwd: need C %% 4 == 0, C <= 256, 1 <= NL <= 4, NG >= NL");
   LCAO_REQUIRE((d_unit_ks == nullptr) == (d_unit_st == nullptr), "lcao_threebody_bwd: pass both d_unit buffers or neither");
   LCAO_REQUIRE(NG <= NL + 1, "lcao_threebody_bwd: at most one valence group (NG <= NL + 1)");
+  LCAO_REQUIRE(al16(B) && al16(gate) && al16(d_tbw), "lcao_threebody_bwd: B, gate and d_tbw must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   const bool forces = d_unit_ks != nullptr;
-  if (use_mma(C, B, gate, ldg) && (reinterpret_cast<uintptr_t>(d_tbw) & 15u) == 0)
+  if (C <= 128)
     return lcao_tb_staged_bwd(B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr, out_edge, N, C, NL, d_tbw, dP, dB,
                               q, d_unit_ks, d_unit_st, st);
-  const int V4 = C <= 128 ? 1 : 2;
-  const bool full = C == 128 * V4;
-  static const int per_sm_b = tile_in("LCAO_TB_GRID_BWD", 24, 1, 64);
-  static const bool guard = tile_in("LCAO_TB_BWD_GUARD", 0, 0, 1) != 0;
-  const unsigned grid = (unsigned)(N < 148ll * per_sm_b ? N : 148ll * per_sm_b);
+  const bool full = C == 128 * kV4;
+  const unsigned grid = (unsigned)(N < 148ll * kBwdCtasPerSm ? N : 148ll * kBwdCtasPerSm);
 #define TB_BWD_ARGS B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr, out_edge, (int)N, C, d_tbw, dP, dB, q
-#define CALL(nl, v4)                                                                                              \
-  if (forces && guard)                                                                                            \
-    k_threebody_bwd<nl, v4, true, false, true><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, d_unit_ks, d_unit_st);  \
-  else if (forces)                                                                                                \
-    k_threebody_bwd<nl, v4, true, false, false><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, d_unit_ks, d_unit_st); \
-  else if (full && guard)                                                                                         \
-    k_threebody_bwd<nl, v4, false, true, true><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, nullptr, nullptr);   \
-  else if (full)                                                                                                  \
-    k_threebody_bwd<nl, v4, false, true, false><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, nullptr, nullptr);  \
-  else                                                                                                            \
-    k_threebody_bwd<nl, v4, false, false, false><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, nullptr, nullptr)
-  TB_DISPATCH(NL, V4, CALL)
+#define CALL(nl)                                                                                            \
+  if (forces)                                                                                               \
+    k_threebody_bwd<nl, true, false><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, d_unit_ks, d_unit_st);  \
+  else if (full)                                                                                            \
+    k_threebody_bwd<nl, false, true><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, nullptr, nullptr);      \
+  else                                                                                                      \
+    k_threebody_bwd<nl, false, false><<<grid, kBwdWarps * 32, 0, st>>>(TB_BWD_ARGS, nullptr, nullptr)
+  TB_DISPATCH(NL, CALL)
 #undef CALL
+#undef TB_BWD_ARGS
   LCAO_LAUNCH_CHECK();
   return LCAO_OK;
 }

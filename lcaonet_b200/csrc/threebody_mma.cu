@@ -26,8 +26,6 @@
 // Sums over triplets stay in accumulator registers and are written once: no atomics (forces: see kJS), deterministic.
 //
 // C <= 128 (one 128-channel accumulator block per warp); wider layers take the FP32-pipe kernels in threebody.cu.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tb_common.cuh"
 #include "tb_async.cuh"
@@ -279,11 +277,7 @@ __global__ void __launch_bounds__(160) k_tb_fwd_mma(
 //  FP32-pipe kernel, but 168 registers + spills, 10 resident warps per SM and a 240 KB instruction footprint made it
 //  2x SLOWER (0.97 ms against 0.46 ms at config 2).  It is not shipped; profiles/r02_notes.md has the numbers.)
 
-int grid_knob(const char* env, int dflt, int lo, int hi) {
-  const char* s = getenv(env);
-  const int v = s ? atoi(s) : dflt;
-  return (v < lo || v > hi) ? dflt : v;
-}
+constexpr int kFwdCtasPerSm = 40;  // grid cap per SM; each CTA takes a contiguous range of nodes
 
 }  // namespace
 
@@ -291,9 +285,8 @@ int grid_knob(const char* env, int dflt, int lo, int hi) {
 int lcao_tb_mma_fwd(const float* B, int32_t NG, const double* gram, const float* unit, const float* gate, int64_t ldg,
                     const int32_t* in_ptr, const int32_t* in_edge, const int32_t* in_src, const int32_t* out_ptr,
                     const int32_t* out_edge, int64_t N, int32_t C, int32_t NL, float* tbw, cudaStream_t st) {
-  static const int per_sm = grid_knob("LCAO_TBM_GRID_FWD", 40, 1, 128);
   const int64_t want = (N + 1) / 2;  // at least two nodes per CTA
-  const unsigned grid = (unsigned)(want < 148ll * per_sm ? (want > 0 ? want : 1) : 148ll * per_sm);
+  const unsigned grid = (unsigned)(want < 148ll * kFwdCtasPerSm ? (want > 0 ? want : 1) : 148ll * kFwdCtasPerSm);
   const size_t smem = sizeof(float) * (size_t)fwd_plan(C, NL).total;
 #define CALL(nl)                                                                                                     \
   {                                                                                                                  \

@@ -17,8 +17,6 @@
 //     zero-filled once), so the loop is branch-free.
 // Results are identical in structure to threebody.cu (same per-pair formulas, sums in registers, no atomics except the
 // out-degree > kJS overflow of d_unit); C <= 128 only — wider layers keep the register kernels.
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "common.cuh"
@@ -30,7 +28,7 @@ namespace {
 constexpr int kSlots = 4;   // in-edges per item = consumer warps
 constexpr int kJC = 32;     // out-edges per chunk (lane <-> out-edge in the coefficient phase)
 constexpr int kGtBufs = 2;  // resident d_tbw chunks
-constexpr bool kForces4 = false;  // forces variant with pair groups of 4 only (96 registers): measured 0.64 vs 0.575 ms, the CTA count stays at three (shared memory)
+constexpr int kCtasPerSm = 16;  // grid cap per SM; each CTA takes a contiguous range of nodes
 enum { kFirst = 1, kLast = 2, kEnd = 4, kNodeFirst = 8, kNodeLast = 16 };
 
 // Shared-memory plan (floats).  [0, 128 B): mbarriers full_in[4] | empty_in[4] | full_gt[2].
@@ -79,7 +77,7 @@ __device__ __forceinline__ int bfly4_index(int lane) { return ((lane >> 4) & 1) 
 __device__ __forceinline__ void consumer_bar() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
 
 template <int NL, bool FORCES, int CT>
-__global__ void __launch_bounds__(160, (FORCES && !kForces4) ? 3 : 4) k_tb_bwd_staged(
+__global__ void __launch_bounds__(160, FORCES ? 3 : 4) k_tb_bwd_staged(
     const float* __restrict__ B, int NG, const double* __restrict__ gram, const float* __restrict__ unit,
     const float* __restrict__ gate, int64_t ldg, const int32_t* __restrict__ in_ptr, const int32_t* __restrict__ in_edge,
     const int32_t* __restrict__ in_src, const int32_t* __restrict__ out_ptr, const int32_t* __restrict__ out_edge, int N,
@@ -402,12 +400,8 @@ __global__ void __launch_bounds__(160, (FORCES && !kForces4) ? 3 : 4) k_tb_bwd_s
           }
         };
         int j0 = 0;
-        if constexpr (FORCES && kForces4) {  // (groups of 4 only: 32 fewer registers, see launch_bwd)
-          for (; j0 < nO; j0 += 4) group(std::integral_constant<int, 4>{}, j0);
-        } else {
-          for (; j0 + 4 < nO; j0 += 8) group(std::integral_constant<int, 8>{}, j0);
-          if (j0 < nO) group(std::integral_constant<int, 4>{}, j0);
-        }
+        for (; j0 + 4 < nO; j0 += 8) group(std::integral_constant<int, 8>{}, j0);
+        if (j0 < nO) group(std::integral_constant<int, 4>{}, j0);
       }
       if (flags & kLast) {
         // ---- finish this in-edge
@@ -475,25 +469,16 @@ __global__ void __launch_bounds__(160, (FORCES && !kForces4) ? 3 : 4) k_tb_bwd_s
   }
 }
 
-int knob(const char* env, int dflt, int lo, int hi) {
-  const char* s = getenv(env);
-  const int v = s ? atoi(s) : dflt;
-  return (v < lo || v > hi) ? dflt : v;
-}
-
 template <int NL, bool FORCES, int CT>
 int launch_bwd(const float* B, int NG, const double* gram, const float* unit, const float* gate, int64_t ldg,
                const int32_t* in_ptr, const int32_t* in_edge, const int32_t* in_src, const int32_t* out_ptr,
                const int32_t* out_edge, int64_t N, int C, const float* d_tbw, const float* dP, float* dB, float* q,
                float* du_ks, float* du_st, cudaStream_t st) {
-  static const int per_sm = knob("LCAO_TBS_GRID", 16, 1, 128);
-  static const int nst_env = knob("LCAO_TBS_STAGES", 0, 2, 4);
   // ring depth: as many stages (<= 4) as keep four CTAs (energy path: 96 registers) or three (forces: 128) resident per
   // SM (227 KB of shared memory, 1 KB reserved per CTA).  Four CTAs with a two-stage ring measured 0.402 ms against
   // 0.428 ms for three with four stages; the forces variant spills at 96 registers and stays at three.
   int nst = 4;
-  while (nst > 2 && sizeof(float) * (size_t)bwd_plan(C, NL, FORCES, nst).total > ((FORCES && !kForces4) ? 74 : 55) * 1024) --nst;
-  if (nst_env) nst = nst_env;
+  while (nst > 2 && sizeof(float) * (size_t)bwd_plan(C, NL, FORCES, nst).total > (FORCES ? 74 : 55) * 1024) --nst;
   const size_t smem = sizeof(float) * (size_t)bwd_plan(C, NL, FORCES, nst).total;
   static bool attr_done = false;
   if (!attr_done) {
@@ -501,7 +486,7 @@ int launch_bwd(const float* B, int NG, const double* gram, const float* unit, co
     attr_done = true;
   }
   const int64_t want = (N + 1) / 2;  // at least two nodes per CTA
-  const unsigned grid = (unsigned)(want < 148ll * per_sm ? (want > 0 ? want : 1) : 148ll * per_sm);
+  const unsigned grid = (unsigned)(want < 148ll * kCtasPerSm ? (want > 0 ? want : 1) : 148ll * kCtasPerSm);
   LCAO_CUDA(launch_pdl(k_tb_bwd_staged<NL, FORCES, CT>, grid, 160, smem, st, B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr,
                                                           out_edge, (int)N, C, nst, d_tbw, dP, dB, q, du_ks, du_st));
   LCAO_LAUNCH_CHECK();

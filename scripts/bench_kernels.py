@@ -113,7 +113,7 @@ def edge():
     T = gi.num_triplets()
     bf = E * (4 * NL * C + 48 + 12 + 8 + 4 * C) + N * (4 * C + 8)
     bb = E * (4 * NL * C + 48 + 4 * C + 12 + 8 + 4 * NL * C + 4 * C) + N * (4 * C + 8)
-    print(f"threebody N={N} E={E} T={T} TI={os.environ.get('LCAO_TB_TI', 'dflt')}/{os.environ.get('LCAO_TB_TI_BWD', 'dflt')}: "
+    print(f"threebody N={N} E={E} T={T}: "
           f"fwd {t_f:.3f} ms ({bf/t_f/1e6:.0f} GB/s, {T/t_f/1e6:.2f} Gtriplets/s) | "
           f"bwd {t_b:.3f} ms ({bb/t_b/1e6:.0f} GB/s, {T/t_b/1e6:.2f} Gtriplets/s) | bwd+forces {t_bf:.3f} ms", flush=True)
     t_i = timeit(lambda: ops.GraphIndex(g["edge_index"], N))
@@ -154,10 +154,9 @@ def tb():
         bf = E * (4 * NL * C + 48 + 12 + 8 + 4 * C) + N * (4 * C + 8)
         bb = E * (4 * NL * C + 48 + 4 * C + 12 + 8 + 4 * NL * C + 4 * C) + N * (4 * C + 8)
         peak = 6556.5
-        print(f"threebody[{os.environ.get('LCAO_TB_IMPL', 'mma')}] {name}: N={N} E={E} T={T}: fwd {t_f:.3f} ms ({bf/t_f/1e6:.0f} GB/s, "
+        print(f"threebody {name}: N={N} E={E} T={T}: fwd {t_f:.3f} ms ({bf/t_f/1e6:.0f} GB/s, "
               f"{bf/t_f/1e6/peak:.2f}) | bwd {t_b:.3f} ms ({bb/t_b/1e6:.0f} GB/s, {bb/t_b/1e6/peak:.2f}) | bwd+forces {t_bf:.3f} ms "
               f"({bb/t_bf/1e6/peak:.2f})", flush=True)
-        # checksums for A/B comparisons between implementations (LCAO_TB_IMPL=simt)
         print(f"  checksums: tbw {float(tbw.double().abs().sum()):.9e} dB {float(dB.double().abs().sum()):.9e} q "
               f"{float(q.double().abs().sum()):.9e} du {float((du1 + du2).double().abs().sum()):.9e}", flush=True)
 

@@ -1,5 +1,5 @@
 """E-sized dense layer (M = 252 798, K = N = 128, 3xTF32): the A-in-tensor-memory kernel, forward and dgrad.
-Usage: [LCAO_TC_TA=0|1] [LCAO_TC_TA_EPI8=1] [LCAO_TC_DEBUG=bits] python scripts/micro/gemm_ta.py"""
+Usage: python scripts/micro/gemm_ta.py"""
 import os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
@@ -13,10 +13,4 @@ m = ops.GEMM_MODES["tf32x3"]
 t0 = timeit(lambda: ops._call("lcao_linear_fwd", P(x), K, P(w), None, P(y), N, None, N, M, K, N, 0, m, st()), reps=9)
 t1 = timeit(lambda: ops._call("lcao_linear_fwd", P(x), K, P(w), None, P(y), N, P(pre), N, M, K, N, 1, m, st()), reps=9)
 t2 = timeit(lambda: ops._call("lcao_linear_dgrad", P(y), N, None, 0, 0, P(w), P(x), K, M, K, N, 0, m, None, st()), reps=9)
-env = {k: v for k, v in os.environ.items() if k.startswith("LCAO_TC")}
-print(f"{env}: fwd {t0*1e3:.1f} us | fwd+pre+silu {t1*1e3:.1f} us | dgrad {t2*1e3:.1f} us", flush=True)
-if int(os.environ.get("LCAO_TC_DEBUG", "0")) & 64:
-    ops._call("lcao_linear_fwd", P(x), K, P(w), None, P(y), N, None, N, M, K, N, 0, m, st())
-    torch.cuda.synchronize()
-    t = y.flatten()[: 2 * 148].reshape(148, 2).mean(0)
-    print(f"  epilogue warp 0, per tile: waits for the tile {float(t[0]):.0f} cycles, drains it in {float(t[1]):.0f} cycles", flush=True)
+print(f"fwd {t0*1e3:.1f} us | fwd+pre+silu {t1*1e3:.1f} us | dgrad {t2*1e3:.1f} us", flush=True)

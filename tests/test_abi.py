@@ -3,6 +3,9 @@ import ctypes
 import os
 import re
 
+import pytest
+import torch
+
 from lcaonet_b200 import _lib
 from lcaonet_b200.csrc.build import build
 
@@ -48,3 +51,15 @@ def test_argument_errors_are_reported_without_a_gpu():
     assert rc == -1 and b"null buffer" in lib.lcao_last_error()
     rc = lib.lcao_threebody_fwd(1, 3, 1, 1, 1, 8, 1, 1, 1, 1, 1, 4, 4, 130, 3, 1, None)
     assert rc == -1 and b"C % 4" in lib.lcao_last_error()
+
+
+@pytest.mark.skipif(torch.cuda.is_available(), reason="without the check, a GPU would run the kernels on these addresses")
+def test_threebody_rejects_unaligned_rows():
+    # pointer values only: every kernel reads B, gate and d_tbw with 16-byte loads or bulk copies
+    lib = _lib.load()
+    a, odd = 16, 4
+    rc = lib.lcao_threebody_fwd(odd, 3, a, a, a, 128, a, a, a, a, a, 4, 4, 128, 3, a, None)
+    assert rc == -1 and b"aligned" in lib.lcao_last_error()
+    for B, d_tbw in ((odd, a), (a, odd)):
+        rc = lib.lcao_threebody_bwd(B, 3, a, a, a, 128, a, a, a, a, a, 4, 4, 128, 3, d_tbw, None, a, a, None, None, None)
+        assert rc == -1 and b"aligned" in lib.lcao_last_error()
