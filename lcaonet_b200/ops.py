@@ -76,17 +76,17 @@ def _call(name, *args):
     call(name, *args)
 
 
-def _rows(x: Tensor) -> Tensor:
-    """2-D view with unit inner stride (copy only if needed)."""
+def _rows(x: Tensor, packed: bool = False) -> Tensor:
+    """2-D view with unit inner stride and rows that do not overlap (`packed`: no gap between them either); copies only
+    if needed.  The launch helpers pass `stride(0)` as the leading dimension, so a single row, whose stride torch leaves
+    as it finds it (0 for an expanded gradient), gets the width instead."""
     if x.dim() != 2:
         x = x.reshape(-1, x.shape[-1])
-    if x.stride(1) != 1 or (x.shape[0] > 1 and x.stride(0) < x.shape[1]):
+    if packed or x.stride(1) != 1 or (x.shape[0] > 1 and x.stride(0) < x.shape[1]):
         x = x.contiguous()
+    if x.shape[0] <= 1 and x.stride(0) != max(x.shape[1], 1):
+        x = x.as_strided(x.shape, (max(x.shape[1], 1), 1))
     return x
-
-
-def _ld(x: Tensor) -> int:
-    return x.stride(0) if x.shape[0] > 1 else max(x.shape[1], 1)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -245,6 +245,93 @@ def geom_basis(pos, shift, lattice, batch, gi, spec, n_orb, strain=None, seg=Non
 # ------------------------------------------------------------------------------------------------
 # dense layers
 # ------------------------------------------------------------------------------------------------
+# Every C-ABI entry point is launched from one place: its only user, or a launch helper (`_lin_*`, `_act_bwd`,
+# `_pair_contract_*`, ...) shared by the op-level Functions and `_InteractionLayer`.  A helper allocates the outputs its
+# caller does not pass, spells the argument list and sizes the scratch.  Matrices are 2-D tensors with unit inner stride,
+# strided views included; their `stride(0)` is the leading dimension.  `st` is the raw CUDA stream.
+def _lin_fwd(x, w, bias, st, act=ACT_NONE, need_pre=False):
+    """(y, pre): y = act(x W^T + b), and its pre-activation when `need_pre` and there is an activation (else None)."""
+    M, (Nout, K) = x.shape[0], w.shape
+    y = torch.empty(M, Nout, device=w.device)
+    pre = torch.empty(M, Nout, device=w.device) if (need_pre and act != ACT_NONE) else None
+    _call("lcao_linear_fwd", ptr(x), x.stride(0), ptr(w), ptr(bias), ptr(y), Nout, ptr(pre), Nout, M, K, Nout, act,
+          _gemm_mode, st)
+    return y, pre
+
+
+def _lin_dgrad(dy, w, st, dx=None, accumulate=0):
+    """dx = dy W (dx += dy W with `accumulate`); dx is allocated unless the caller passes it."""
+    M, (Nout, K) = dy.shape[0], w.shape
+    if dx is None:
+        dx = torch.empty(M, K, device=w.device)
+    _call("lcao_linear_dgrad", ptr(dy), dy.stride(0), None, 0, ACT_NONE, ptr(w), ptr(dx), dx.stride(0), M, K, Nout,
+          accumulate, _gemm_mode, None, st)
+    return dx
+
+
+def _lin_dgrad_act(dy, w, pre_in, act, st):
+    """dx = (dy W) * act'(pre_in): data gradient chained through the activation that produced the layer's input."""
+    M, (Nout, K) = dy.shape[0], w.shape
+    dx = torch.empty(M, K, device=w.device)
+    _call("lcao_linear_dgrad_act", ptr(dy), dy.stride(0), ptr(w), ptr(pre_in), pre_in.stride(0), act, ptr(dx), K, M, K,
+          Nout, _gemm_mode, st)
+    return dx
+
+
+# Weight gradients that go straight into the parameters' .grad buffers (gradient sinks) are only read by the optimizer /
+# the all-reduce, so the second stage of the tcgen05 weight-gradient kernel (the sum of its per-CTA partial tiles) is
+# deferred: the descriptors pile up here and ONE batched launch at the end of the backward pass (an autograd engine
+# callback) finishes them all.
+_pending_wgrad = {"desc": [], "keep": [], "queued": False, "stream": None}
+
+
+def flush_wgrad():
+    """Finish the deferred weight gradients (runs by itself at the end of every backward pass that deferred any)."""
+    p = _pending_wgrad
+    p["queued"] = False
+    if p["desc"]:
+        arr = (ctypes.c_int64 * len(p["desc"]))(*p["desc"])
+        _call("lcao_wgrad_reduce_batch", arr, len(p["desc"]) // 6, p["stream"])
+    p["desc"], p["keep"], p["stream"] = [], [], None
+
+
+def _lin_wgrad(dy, x, w, has_bias, st, dw_sink=None, db_sink=None):
+    """dW (+ db) of one layer.  With sinks (the parameters' .grad buffers) the kernels accumulate straight into them
+    — the C ABI's `dW +=` contract — and (None, None) is returned: no zero-fill, no separate accumulation pass."""
+    M, (Nout, K), ldy, ldx = dy.shape[0], w.shape, dy.stride(0), x.stride(0)
+    dw = dw_sink if dw_sink is not None else torch.zeros(Nout, K, device=w.device)
+    db = (db_sink if db_sink is not None else torch.zeros(Nout, device=w.device)) if has_bias else None
+    n_scr = int(_lib.load().lcao_linear_bwd_scratch(ptr(dy), ldy, None, 0, ACT_NONE, None, ptr(x), ldx, None, 0, M, K, Nout,
+                                                    _gemm_mode))
+    if dw_sink is not None and (db_sink is not None or not has_bias) and n_scr:
+        passes = (Nout + 127) // 128
+        scr = torch.empty(n_scr * passes, device=w.device)
+        desc, nd = (ctypes.c_int64 * (6 * passes))(), ctypes.c_int32(0)
+        _call("lcao_linear_wgrad_deferred", ptr(dy), ldy, ptr(x), ldx, ptr(dw), ptr(db), M, K, Nout, _gemm_mode, ptr(scr),
+              desc, ctypes.byref(nd), st)
+        if nd.value:
+            p = _pending_wgrad
+            p["desc"].extend(desc[: 6 * nd.value])
+            p["keep"].append((scr, dw, db))  # the partial tiles and their targets stay alive until the flush
+            p["stream"] = st
+            if not p["queued"]:
+                torch.autograd.Variable._execution_engine.queue_callback(flush_wgrad)
+                p["queued"] = True
+        return None, None
+    scr = torch.empty(n_scr, device=w.device) if n_scr else None
+    _call("lcao_linear_wgrad", ptr(dy), ldy, None, 0, ACT_NONE, ptr(x), ldx, ptr(dw), ptr(db), M, K, Nout, _gemm_mode,
+          ptr(scr), st)
+    return (None if dw_sink is not None else dw), (None if (db_sink is not None or not has_bias) else db)
+
+
+def _act_bwd(dy, pre, act, st):
+    """dH = dY * act'(pre)"""
+    M, C = dy.shape
+    out = torch.empty(M, C, device=dy.device)
+    _call("lcao_act_bwd", ptr(dy), dy.stride(0), ptr(pre), pre.stride(0), ptr(out), C, M, C, act, st)
+    return out
+
+
 class _Linear(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, weight, bias, act: int):
@@ -252,15 +339,10 @@ class _Linear(torch.autograd.Function):
         shape = x.shape
         x2 = _rows(x)
         w = weight.contiguous()
-        M, K, Nout = x2.shape[0], x2.shape[1], w.shape[0]
-        y = torch.empty(M, Nout, device=x.device)
-        need_pre = act != ACT_NONE and any(ctx.needs_input_grad)
-        pre = torch.empty(M, Nout, device=x.device) if need_pre else None
-        _call("lcao_linear_fwd", ptr(x2), _ld(x2), ptr(w), ptr(bias), ptr(y), Nout, ptr(pre), Nout, M, K, Nout, act,
-              _gemm_mode, stream_ptr())
+        y, pre = _lin_fwd(x2, w, bias, stream_ptr(), act, any(ctx.needs_input_grad))
         ctx.act, ctx.shape, ctx.has_bias = act, shape, bias is not None
         ctx.save_for_backward(x2, w, pre, x, weight, bias)
-        return y.reshape(*shape[:-1], Nout)
+        return y.reshape(*shape[:-1], w.shape[0])
 
     @staticmethod
     def backward(ctx, dy):
@@ -274,29 +356,14 @@ class _Linear(torch.autograd.Function):
                     wanted[1] = wanted[2] = False
                 gx, gw, gb = second_order.grads_with_graph([y], ins, [dy], wanted)
             return gx, gw, gb, None
-        M, K, Nout = x2.shape[0], x2.shape[1], w.shape[0]
         dy2 = _rows(dy)
         st = stream_ptr()
         need_dx = ctx.needs_input_grad[0]
         need_dw = (ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2])) and not positions_only.active
         if ctx.act != ACT_NONE:  # dH = dY * act'(pre), shared by the data and the weight gradient
-            dh = torch.empty(M, Nout, device=dy.device)
-            _call("lcao_act_bwd", ptr(dy2), _ld(dy2), ptr(pre), Nout, ptr(dh), Nout, M, Nout, ctx.act, st)
-            dy2 = dh
-        dx = dw = db = None
-        if need_dx:
-            dx = torch.empty(M, K, device=dy.device)
-            _call("lcao_linear_dgrad", ptr(dy2), _ld(dy2), None, 0, ACT_NONE, ptr(w), ptr(dx), K, M, K, Nout, 0,
-                  _gemm_mode, None, st)
-            dx = dx.reshape(ctx.shape)
-        if need_dw:
-            dw = torch.zeros(Nout, K, device=dy.device)
-            db = torch.zeros(Nout, device=dy.device) if ctx.has_bias else None
-            n_scr = int(_lib.load().lcao_linear_bwd_scratch(ptr(dy2), _ld(dy2), None, 0, ACT_NONE, None, ptr(x2), _ld(x2),
-                                                            None, 0, M, K, Nout, _gemm_mode))
-            scr = torch.empty(n_scr, device=dy.device) if n_scr else None
-            _call("lcao_linear_wgrad", ptr(dy2), _ld(dy2), None, 0, ACT_NONE, ptr(x2), _ld(x2), ptr(dw), ptr(db), M,
-                  K, Nout, _gemm_mode, ptr(scr), st)
+            dy2 = _act_bwd(dy2, pre, ctx.act, st)
+        dx = _lin_dgrad(dy2, w, st).reshape(ctx.shape) if need_dx else None
+        dw, db = _lin_wgrad(dy2, x2, w, ctx.has_bias, st) if need_dw else (None, None)
         return dx, dw, db, None
 
 
@@ -349,6 +416,35 @@ def coeff_contract(cst1, rb, vmask, lgrp, NL, C):
     return _CoeffContract.apply(cst1, rb.contiguous(), vmask, lgrp, NL, C)
 
 
+def _pair_contract_fwd(tab, pair, rb, vmask, lgrp, NL, C, st, with_psum=False):
+    """(B, gram, psum) from the (P, O, C') table: psum = [sum_l B_l | valence slot] only `with_psum` (else None)."""
+    E, O, dev = pair.numel(), tab.shape[1], tab.device
+    valence = 1 if vmask is not None else 0
+    B = torch.empty(E, NL + valence, C, device=dev)
+    gram = torch.empty(E, NL * (NL + 1) // 2, dtype=torch.float64, device=dev)
+    psum = torch.empty(E, 1 + valence, C, device=dev) if with_psum else None
+    _call("lcao_pair_contract_fwd", ptr(tab), ptr(pair), ptr(rb), ptr(vmask), ptr(lgrp), E, O, C, NL, valence, ptr(B),
+          ptr(gram), ptr(psum), st)
+    return B, gram, psum
+
+
+def _pair_contract_bwd(tab, pair, grouping, rb, vmask, lgrp, dB, NL, C, need_tab, need_rb, st):
+    """(d tab, d rb) of B = pair_contract(tab, rb), None where not needed."""
+    (P, O, _), E = tab.shape, pair.numel()
+    valence = 1 if vmask is not None else 0
+    d_tab = torch.empty_like(tab) if need_tab else None
+    d_rb = torch.empty(E, O, device=tab.device) if need_rb else None
+    if need_tab or (need_rb and E > 0):  # (an edge-less batch has no d rb to write)
+        kptr, kperm = _grouping(grouping, pair, P)
+        scratch = None
+        if need_tab:
+            nbytes = int(_lib.load().lcao_pair_contract_bwd_scratch(E, P, O, C, valence))
+            scratch = torch.empty((nbytes + 15) // 16 * 4, dtype=torch.int32, device=tab.device)
+        _call("lcao_pair_contract_bwd", ptr(tab), ptr(pair), ptr(kptr), ptr(kperm), ptr(rb), ptr(vmask), ptr(lgrp), ptr(dB),
+              E, P, O, C, NL, valence, ptr(d_tab), ptr(d_rb), ptr(scratch), st)
+    return d_tab, d_rb
+
+
 class _PairContract(torch.autograd.Function):
     """B and its Gram matrices from the species-pair coefficient table (see lcao_pair_contract_fwd)."""
 
@@ -356,16 +452,9 @@ class _PairContract(torch.autograd.Function):
     def forward(ctx, tab, pair, grouping, rb, vmask, lgrp, NL: int, C: int):
         require_cuda(tab, pair, rb)
         tab = tab.contiguous()
-        P, O, Cp = tab.shape
-        E = pair.numel()
-        valence = 1 if vmask is not None else 0
-        assert Cp == C * (1 + valence) and pair.dtype == torch.int64
-        NG = NL + valence
-        B = torch.empty(E, NG, C, device=tab.device)
-        gram = torch.empty(E, NL * (NL + 1) // 2, dtype=torch.float64, device=tab.device)
-        _call("lcao_pair_contract_fwd", ptr(tab), ptr(pair), ptr(rb), ptr(vmask), ptr(lgrp), E, O, C, NL, valence, ptr(B),
-              ptr(gram), None, stream_ptr())
-        ctx.dims, ctx.grouping = (E, P, O, C, NL, valence), grouping
+        assert tab.shape[2] == C * (1 + (vmask is not None)) and pair.dtype == torch.int64
+        B, gram, _ = _pair_contract_fwd(tab, pair, rb, vmask, lgrp, NL, C, stream_ptr())
+        ctx.NL, ctx.C, ctx.grouping = NL, C, grouping
         ctx.save_for_backward(tab, pair, rb, vmask, lgrp)
         ctx.mark_non_differentiable(gram)
         return B, gram
@@ -374,15 +463,8 @@ class _PairContract(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, dB, _dgram):
         tab, pair, rb, vmask, lgrp = ctx.saved_tensors
-        E, P, O, C, NL, valence = ctx.dims
-        kptr, kperm = _grouping(ctx.grouping, pair, P)
-        dB = dB.contiguous()
-        d_tab = torch.empty_like(tab)
-        d_rb = torch.empty_like(rb) if ctx.needs_input_grad[3] else None
-        nbytes = int(_lib.load().lcao_pair_contract_bwd_scratch(E, P, O, C, valence))
-        scratch = torch.empty((nbytes + 15) // 16 * 4, dtype=torch.int32, device=tab.device)
-        _call("lcao_pair_contract_bwd", ptr(tab), ptr(pair), ptr(kptr), ptr(kperm), ptr(rb), ptr(vmask), ptr(lgrp), ptr(dB),
-              E, P, O, C, NL, valence, ptr(d_tab), ptr(d_rb), ptr(scratch), stream_ptr())
+        d_tab, d_rb = _pair_contract_bwd(tab, pair, ctx.grouping, rb, vmask, lgrp, dB.contiguous(), ctx.NL, ctx.C, True,
+                                         ctx.needs_input_grad[3], stream_ptr())
         return d_tab, None, None, d_rb, None, None, None, None
 
 
@@ -427,19 +509,38 @@ class BodyLink:
         self.consumed = False
 
 
+def _threebody_fwd(B, gram, unit, xk, gi, NL, st):
+    """(tbw, gate): the gate sigmoid(xk) once per node, then the three-body kernel."""
+    E, NG, C = B.shape
+    gate = torch.empty(gi.N, C, device=B.device)
+    _call("lcao_sigmoid_rows", ptr(xk), xk.stride(0), ptr(gate), C, gi.N, C, st)
+    tbw = torch.empty(E, C, device=B.device)
+    _call("lcao_threebody_fwd", ptr(B), NG, ptr(gram), ptr(unit), ptr(gate), C, ptr(gi.in_ptr), ptr(gi.in_edge),
+          ptr(gi.in_src), ptr(gi.out_ptr), ptr(gi.out_edge), gi.N, E, C, NL, ptr(tbw), st)
+    return tbw, gate
+
+
+def _threebody_bwd(B, gram, unit, gate, gi, NL, d_tbw, dP, q, d_xk, forces, st):
+    """(dB, d unit) of tbw = threebody(B, unit, xk); d unit is None unless `forces`.  The kernel leaves the gradient of
+    the gate's input per edge in `q` (E, C), whose sum over each node's out-edges goes into the caller's `d_xk`."""
+    E, NG, C = B.shape
+    dB = torch.empty_like(B)
+    du_ks = torch.empty(E, 3, device=B.device) if forces else None
+    du_st = torch.empty(E, 3, device=B.device) if forces else None
+    _call("lcao_threebody_bwd", ptr(B), NG, ptr(gram), ptr(unit), ptr(gate), C, ptr(gi.in_ptr), ptr(gi.in_edge),
+          ptr(gi.in_src), ptr(gi.out_ptr), ptr(gi.out_edge), gi.N, E, C, NL, ptr(d_tbw), ptr(dP), ptr(dB), ptr(q),
+          ptr(du_ks), ptr(du_st), st)
+    _segment_sum(q, gi.out_ptr, gi.out_edge, gi.N, st, out=d_xk)
+    return dB, (du_ks + du_st) if forces else None
+
+
 class _ThreeBody(torch.autograd.Function):
     @staticmethod
     def forward(ctx, B, gram, unit, xk, gi: GraphIndex, NL: int, link):
         require_cuda(B, unit, xk)
         B, unit = B.contiguous(), unit.contiguous()
-        E, NG, C = B.shape
         assert xk.stride(1) == 1 and gram.dtype == torch.float64 and gram.is_contiguous()
-        st = stream_ptr()
-        gate = torch.empty(gi.N, C, device=B.device)  # sigmoid(xk) once per node
-        _call("lcao_sigmoid_rows", ptr(xk), xk.stride(0), ptr(gate), C, gi.N, C, st)
-        tbw = torch.empty(E, C, device=B.device)
-        _call("lcao_threebody_fwd", ptr(B), NG, ptr(gram), ptr(unit), ptr(gate), C, ptr(gi.in_ptr),
-              ptr(gi.in_edge), ptr(gi.in_src), ptr(gi.out_ptr), ptr(gi.out_edge), gi.N, E, C, NL, ptr(tbw), st)
+        tbw, gate = _threebody_fwd(B, gram, unit, xk, gi, NL, stream_ptr())
         ctx.gi, ctx.NL, ctx.link = gi, NL, link
         ctx.save_for_backward(B, gram, unit, gate)
         return tbw
@@ -448,24 +549,15 @@ class _ThreeBody(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, d_tbw):
         B, gram, unit, gate = ctx.saved_tensors
-        gi, NL, link = ctx.gi, ctx.NL, ctx.link
-        E, NG, C = B.shape
-        d_tbw = d_tbw.contiguous()
-        dB = torch.empty_like(B)
-        q = torch.empty(E, C, device=B.device)
-        st = stream_ptr()
-        forces = ctx.needs_input_grad[2]
-        du_ks = torch.empty(E, 3, device=B.device) if forces else None
-        du_st = torch.empty(E, 3, device=B.device) if forces else None
+        gi, link = ctx.gi, ctx.link
+        E, _, C = B.shape
         dP = None
         if link is not None:
             dP, link.dP, link.consumed = link.dP, None, True
-        _call("lcao_threebody_bwd", ptr(B), NG, ptr(gram), ptr(unit), ptr(gate), C, ptr(gi.in_ptr),
-              ptr(gi.in_edge), ptr(gi.in_src), ptr(gi.out_ptr), ptr(gi.out_edge), gi.N, E, C, NL, ptr(d_tbw), ptr(dP),
-              ptr(dB), ptr(q), ptr(du_ks), ptr(du_st), st)
-        d_xk = torch.empty(gi.N, C, device=B.device)
-        _call("lcao_segment_sum", ptr(q), C, None, 0, ptr(gi.out_ptr), ptr(gi.out_edge), gi.N, C, 0, ptr(d_xk), C, st)
-        return dB, None, (du_ks + du_st) if forces else None, d_xk, None, None, None
+        q, d_xk = torch.empty(E, C, device=B.device), torch.empty(gi.N, C, device=B.device)
+        dB, d_unit = _threebody_bwd(B, gram, unit, gate, gi, ctx.NL, d_tbw.contiguous(), dP, q, d_xk,
+                                    ctx.needs_input_grad[2], stream_ptr())
+        return dB, None, d_unit, d_xk, None, None, None
 
 
 def threebody(B, unit, xk, gi, NL, gram=None, link: BodyLink | None = None):
@@ -475,14 +567,28 @@ def threebody(B, unit, xk, gi, NL, gram=None, link: BodyLink | None = None):
     return _ThreeBody.apply(B, gram, unit, xk, gi, NL, link)
 
 
+def _twobody_fwd(B, g, NL, valence, st):
+    E, NG, C = B.shape
+    lw = torch.empty(E, C, device=B.device)
+    _call("lcao_twobody_fwd", ptr(B), NG, ptr(g), E, C, NL, valence, ptr(lw), st)
+    return lw
+
+
+def _twobody_bwd(B, g, d_lw, NL, valence, compact, st):
+    """(dB, dg); `compact`: dB is the (E, 1 + valence, C) gradient of [sum_l B_l | valence slot]."""
+    E, NG, C = B.shape
+    dB = torch.empty(E, 1 + valence, C, device=B.device) if compact else torch.empty_like(B)
+    dg = torch.empty_like(g)
+    _call("lcao_twobody_bwd", ptr(B), NG, ptr(g), ptr(d_lw), E, C, NL, valence, int(compact), ptr(dB), ptr(dg), st)
+    return dB, dg
+
+
 class _TwoBody(torch.autograd.Function):
     @staticmethod
     def forward(ctx, B, g, NL: int, valence: int, link):
         require_cuda(B, g)
-        E, NG, C = B.shape
         g = g.contiguous()
-        lw = torch.empty(E, C, device=B.device)
-        _call("lcao_twobody_fwd", ptr(B), NG, ptr(g), E, C, NL, valence, ptr(lw), stream_ptr())
+        lw = _twobody_fwd(B, g, NL, valence, stream_ptr())
         ctx.dims, ctx.link = (NL, valence), link
         ctx.save_for_backward(B, g)
         return lw
@@ -492,13 +598,9 @@ class _TwoBody(torch.autograd.Function):
     def backward(ctx, d_lw):
         B, g = ctx.saved_tensors
         NL, valence = ctx.dims
-        E, NG, C = B.shape
         link = ctx.link
         compact = link is not None and not link.consumed
-        dB = torch.empty(E, 1 + valence, C, device=B.device) if compact else torch.empty_like(B)
-        dg = torch.empty_like(g)
-        _call("lcao_twobody_bwd", ptr(B), NG, ptr(g), ptr(d_lw.contiguous()), E, C, NL, valence, 1 if compact else 0,
-              ptr(dB), ptr(dg), stream_ptr())
+        dB, dg = _twobody_bwd(B, g, d_lw.contiguous(), NL, valence, compact, stream_ptr())
         if compact:  # handed to the three-body backward kernel, which adds it to the dB it writes
             link.dP = dB
             return None, dg, None, None, None
@@ -513,81 +615,6 @@ def twobody(B, g, NL, valence, link: BodyLink | None = None):
 # ------------------------------------------------------------------------------------------------
 # one interaction block as ONE autograd node
 # ------------------------------------------------------------------------------------------------
-def _lin_fwd(x, ldx, M, w, bias, act, st, need_pre):
-    """y (M, Nout) [, pre] = act(x W^T + b) on raw row views; returns (y, pre)."""
-    Nout, K = w.shape
-    y = torch.empty(M, Nout, device=w.device)
-    pre = torch.empty(M, Nout, device=w.device) if (need_pre and act != ACT_NONE) else None
-    _call("lcao_linear_fwd", ptr(x), ldx, ptr(w), ptr(bias), ptr(y), Nout, ptr(pre), Nout, M, K, Nout, act, _gemm_mode, st)
-    return y, pre
-
-
-def _lin_dgrad(dy, ldy, M, w, dx, ldx, accumulate, st):
-    Nout, K = w.shape
-    _call("lcao_linear_dgrad", ptr(dy), ldy, None, 0, ACT_NONE, ptr(w), ptr(dx), ldx, M, K, Nout, accumulate, _gemm_mode, None, st)
-
-
-def _lin_dgrad_act(dy, ldy, M, w, pre_in, dx, ldx, st, act=ACT_SILU):
-    """dx = (dy W) * act'(pre_in): data gradient chained through the activation that produced the layer's input."""
-    Nout, K = w.shape
-    _call("lcao_linear_dgrad_act", ptr(dy), ldy, ptr(w), ptr(pre_in), K, act, ptr(dx), ldx, M, K, Nout, _gemm_mode, st)
-
-
-# Weight gradients that go straight into the parameters' .grad buffers (gradient sinks) are only read by the optimizer /
-# the all-reduce, so the second stage of the tcgen05 weight-gradient kernel (the sum of its per-CTA partial tiles) is
-# deferred: the descriptors pile up here and ONE batched launch at the end of the backward pass (an autograd engine
-# callback) finishes them all.  `defer_wgrad = False` restores one reduction launch per layer.
-defer_wgrad = True
-_pending_wgrad = {"desc": [], "keep": [], "queued": False, "stream": None}
-
-
-def flush_wgrad():
-    """Finish the deferred weight gradients (runs by itself at the end of every backward pass that deferred any)."""
-    p = _pending_wgrad
-    p["queued"] = False
-    if p["desc"]:
-        import ctypes as C
-        arr = (C.c_int64 * len(p["desc"]))(*p["desc"])
-        _call("lcao_wgrad_reduce_batch", arr, len(p["desc"]) // 6, p["stream"])
-    p["desc"], p["keep"], p["stream"] = [], [], None
-
-
-def _lin_wgrad(dy, ldy, x, ldx, M, w, has_bias, st, dw_sink=None, db_sink=None):
-    """dW (+ db) of one layer.  With sinks (the parameters' .grad buffers) the kernels accumulate straight into them
-    — the C ABI's `dW +=` contract — and (None, None) is returned: no zero-fill, no separate accumulation pass."""
-    Nout, K = w.shape
-    dw = dw_sink if dw_sink is not None else torch.zeros(Nout, K, device=w.device)
-    db = (db_sink if db_sink is not None else torch.zeros(Nout, device=w.device)) if has_bias else None
-    n_scr = int(_lib.load().lcao_linear_bwd_scratch(ptr(dy), ldy, None, 0, ACT_NONE, None, ptr(x), ldx, None, 0, M, K, Nout,
-                                                    _gemm_mode))
-    if defer_wgrad and dw_sink is not None and (db_sink is not None or not has_bias) and n_scr:
-        import ctypes as C
-        passes = (Nout + 127) // 128
-        scr = torch.empty(n_scr * passes, device=w.device)
-        desc, nd = (C.c_int64 * (6 * passes))(), C.c_int32(0)
-        _call("lcao_linear_wgrad_deferred", ptr(dy), ldy, ptr(x), ldx, ptr(dw), ptr(db), M, K, Nout, _gemm_mode, ptr(scr), desc,
-              C.byref(nd), st)
-        if nd.value:
-            p = _pending_wgrad
-            p["desc"].extend(desc[: 6 * nd.value])
-            p["keep"].append((scr, dw, db))  # the partial tiles and their targets stay alive until the flush
-            p["stream"] = st
-            if not p["queued"]:
-                torch.autograd.Variable._execution_engine.queue_callback(flush_wgrad)
-                p["queued"] = True
-        return None, None
-    scr = torch.empty(n_scr, device=w.device) if n_scr else None
-    _call("lcao_linear_wgrad", ptr(dy), ldy, None, 0, ACT_NONE, ptr(x), ldx, ptr(dw), ptr(db), M, K, Nout, _gemm_mode,
-          ptr(scr), st)
-    return (None if dw_sink is not None else dw), (None if (db_sink is not None or not has_bias) else db)
-
-
-def _act_bwd(dy, pre, M, C, st, act=ACT_SILU):
-    out = torch.empty(M, C, device=dy.device)
-    _call("lcao_act_bwd", ptr(dy), C, ptr(pre), C, ptr(out), C, M, C, act, st)
-    return out
-
-
 class _InteractionLayer(torch.autograd.Function):
     """LCAOInteraction.forward (reference lcaonet.py:130-216) as a single autograd node.
 
@@ -603,58 +630,44 @@ class _InteractionLayer(torch.autograd.Function):
         pair, grouping, vmask, lgrp, gi, NL, C, sinks, act = aux
         require_cuda(x, table, rb, unit)
         st = stream_ptr()
-        dev = x.device
-        N, H = x.shape
-        E = gi.E
-        P, O, K = table.shape
+        N = x.shape[0]
+        P, O, _ = table.shape
         valence = 1 if vmask is not None else 0
-        Cp, NG = C * (1 + valence), NL + valence
         grad = any(ctx.needs_input_grad)  # (grad mode is always off inside Function.forward)
-        x, table, rb, unit = x.contiguous(), table.contiguous(), rb.contiguous(), unit.contiguous()
+        x, table, rb, unit = _rows(x, True), table.contiguous(), rb.contiguous(), unit.contiguous()
         # node side: nw = [xc | xk]
-        nw, _ = _lin_fwd(x, H, N, w_n, b_n, ACT_NONE, st, False)
+        nw, _ = _lin_fwd(x, w_n, b_n, st)
         # f_coeffs on the species-pair table
-        t1, pre1 = _lin_fwd(table, K, P * O, w_c0, None, act, st, grad)
-        tab, pre2 = _lin_fwd(t1, C, P * O, w_c2, None, act, st, grad)
-        B = torch.empty(E, NG, C, device=dev)
-        gram = torch.empty(E, NL * (NL + 1) // 2, dtype=torch.float64, device=dev)
-        psum = torch.empty(E, 1 + valence, C, device=dev)  # [sum_l B_l | valence slot]: the two-body weight's view of B
-        _call("lcao_pair_contract_fwd", ptr(tab), ptr(pair), ptr(rb), ptr(vmask), ptr(lgrp), E, O, C, NL, valence, ptr(B),
-              ptr(gram), ptr(psum), st)
+        t1, pre1 = _lin_fwd(_rows(table, True), w_c0, None, st, act, grad)
+        tab, pre2 = _lin_fwd(t1, w_c2, None, st, act, grad)
+        tab = tab.view(P, O, -1)
+        # psum = [sum_l B_l | valence slot]: the two-body weight's view of B
+        B, gram, psum = _pair_contract_fwd(tab, pair, rb, vmask, lgrp, NL, C, st, with_psum=True)
         # three-body
-        gate = torch.empty(N, C, device=dev)
-        _call("lcao_sigmoid_rows", nw.data_ptr() + 4 * C, 2 * C, ptr(gate), C, N, C, st)
-        tbw = torch.empty(E, C, device=dev)
-        _call("lcao_threebody_fwd", ptr(B), NG, ptr(gram), ptr(unit), ptr(gate), C, ptr(gi.in_ptr), ptr(gi.in_edge),
-              ptr(gi.in_src), ptr(gi.out_ptr), ptr(gi.out_edge), N, E, C, NL, ptr(tbw), st)
-        g, _ = _lin_fwd(tbw, C, E, w_3, None, ACT_NONE, st, False)
+        xc, xk = nw.chunk(2, 1)
+        tbw, gate = _threebody_fwd(B, gram, unit, xk, gi, NL, st)
+        g, _ = _lin_fwd(tbw, w_3, None, st)
         # two-body weight and message
-        lw = torch.empty(E, C, device=dev)
-        _call("lcao_twobody_fwd", ptr(psum), 1 + valence, ptr(g), E, C, 1, valence, ptr(lw), st)
-        bw, _ = _lin_fwd(lw, C, E, w_b, None, ACT_NONE, st, False)
+        lw = _twobody_fwd(psum, g, 1, valence, st)
+        bw, _ = _lin_fwd(lw, w_b, None, st)
         w_1cat = torch.cat([w_1[:, :C], w_1[:, C:]], dim=0)  # (2C, C): [W1a ; W1b] acting on x_s / x_t per NODE
-        u, _ = _lin_fwd(nw, 2 * C, N, w_1cat, None, ACT_NONE, st, False)  # reads xc = nw[:, :C]
-        a1 = torch.empty(E, C, device=dev)
-        pre_a = torch.empty(E, C, device=dev) if grad else None
-        _call("lcao_edge_pair_fwd", ptr(u), 2 * C, u.data_ptr() + 4 * C, 2 * C, ptr(b_1), ptr(gi.src32), ptr(gi.dst32), E, C,
-              act, ptr(a1), ptr(pre_a), st)
+        u, _ = _lin_fwd(xc, w_1cat, None, st)
+        a1, pre_a = _edge_pair_fwd(*u.chunk(2, 1), b_1, gi, act, grad, st)
         # h = SiLU(pre_h) is never stored: the message sum and its backward apply the activation on the fly, which takes
         # one E x C write off the f_node GEMM and one E x C read off each consumer
-        pre_h, _ = _lin_fwd(a1, C, E, w_2, b_2, ACT_NONE, st, False)
-        agg = torch.empty(N, C, device=dev)
-        _call("lcao_segment_sum", ptr(bw), C, ptr(pre_h), C, ptr(gi.out_ptr), ptr(gi.out_edge), N, C, 2 | (act << 4), ptr(agg), C,
-              st)
-        y, _ = _lin_fwd(agg, C, N, w_o, None, ACT_NONE, st, False)
+        pre_h, _ = _lin_fwd(a1, w_2, b_2, st)
+        agg = _segment_sum(bw, gi.out_ptr, gi.out_edge, N, st, y=pre_h, mode=2 | (act << 4))
+        y, _ = _lin_fwd(agg, w_o, None, st)
         out = x + y
         if grad:
             ctx.aux = aux
-            ctx.save_for_backward(x, table, rb, unit, w_n, w_c0, w_c2, w_3, w_b, w_1cat, w_2, w_o, nw, t1, pre1, tab, pre2,
+            ctx.save_for_backward(x, table, rb, unit, w_n, w_c0, w_c2, w_3, w_b, w_1cat, w_2, w_o, xc, t1, pre1, tab, pre2,
                                   B, gram, gate, tbw, g, lw, bw, a1, pre_a, pre_h, agg, psum, b_n, w_1, b_1, b_2)
         return out
 
     @staticmethod
     def backward(ctx, d_out):
-        (x, table, rb, unit, w_n, w_c0, w_c2, w_3, w_b, w_1cat, w_2, w_o, nw, t1, pre1, tab, pre2, B, gram, gate, tbw, g,
+        (x, table, rb, unit, w_n, w_c0, w_c2, w_3, w_b, w_1cat, w_2, w_o, xc, t1, pre1, tab, pre2, B, gram, gate, tbw, g,
          lw, bw, a1, pre_a, pre_h, agg, psum, b_n, w_1, b_1, b_2) = ctx.saved_tensors
         pair, grouping, vmask, lgrp, gi, NL, C, sinks, act = ctx.aux
         if torch.is_grad_enabled():
@@ -676,39 +689,34 @@ class _InteractionLayer(torch.autograd.Function):
         # gradient sinks: the parameters' own .grad buffers (order: w_n, b_n, w_c0, w_c2, w_3, w_b, w_1, b_1, w_2, b_2, w_o)
         s_wn, s_bn, s_wc0, s_wc2, s_w3, s_wb, s_w1, s_b1, s_w2, s_b2, s_wo = sinks if sinks is not None else (None,) * 11
         st = stream_ptr()
-        dev = x.device
-        N, H = x.shape
-        E = gi.E
+        (N, _), E = x.shape, gi.E
         P, O, K = table.shape
         valence = 1 if vmask is not None else 0
-        Cp, NG = C * (1 + valence), NL + valence
         need_rb, need_unit = ctx.needs_input_grad[2], ctx.needs_input_grad[3]
-        d_out = d_out.contiguous()
+        d_out = _rows(d_out, True)
         dw_n = db_n = dw_c0 = dw_c2 = dw_3 = dw_b = dw_1 = db_1 = dw_2 = db_2 = dw_o = d_table = None
         # x_out = x + out_weight(agg)
         if wg:
-            dw_o, _ = _lin_wgrad(d_out, H, agg, C, N, w_o, False, st, s_wo)
-        d_agg = torch.empty(N, C, device=dev)
-        _lin_dgrad(d_out, H, N, w_o, d_agg, C, 0, st)
+            dw_o, _ = _lin_wgrad(d_out, agg, w_o, False, st, s_wo)
+        d_agg = _lin_dgrad(d_out, w_o, st)
         # agg[s] = sum_{e in out(s)} bw[e] * h[e]
-        d_bw, d_preh = torch.empty(E, C, device=dev), torch.empty(E, C, device=dev)
+        d_bw, d_preh = torch.empty(E, C, device=x.device), torch.empty(E, C, device=x.device)
         _call("lcao_msg_bwd", ptr(d_agg), C, ptr(gi.src32), None, ptr(bw), ptr(pre_h), E, C, act, ptr(d_bw), ptr(d_preh), st)
         # h = silu(f_node.2(a1)) ; a1 = silu(u_a[s] + u_b[t] + b1)
         if wg:
-            dw_2, db_2 = _lin_wgrad(d_preh, C, a1, C, E, w_2, True, st, s_w2, s_b2)
+            dw_2, db_2 = _lin_wgrad(d_preh, a1, w_2, True, st, s_w2, s_b2)
         # d_prea = d_a1 * SiLU'(pre_a) is never materialised: the two segment sums over it apply the factor on the fly
-        d_a1 = torch.empty(E, C, device=dev)
-        _lin_dgrad(d_preh, C, E, w_2, d_a1, C, 0, st)
-        d_u = torch.empty(N, 2 * C, device=dev)
-        _call("lcao_segment_sum", ptr(d_a1), C, ptr(pre_a), C, ptr(gi.out_ptr), ptr(gi.out_edge), N, C, 4 | (act << 4), ptr(d_u),
-              2 * C, st)
-        _call("lcao_segment_sum", ptr(d_a1), C, ptr(pre_a), C, ptr(gi.in_ptr), ptr(gi.in_edge), N, C, 4 | (act << 4),
-              d_u.data_ptr() + 4 * C, 2 * C, st)
-        d_nw = torch.empty(N, 2 * C, device=dev)
-        _lin_dgrad(d_u, 2 * C, N, w_1cat, d_nw, 2 * C, 0, st)  # writes d_xc = d_nw[:, :C]
+        d_a1 = _lin_dgrad(d_preh, w_2, st)
+        d_u = torch.empty(N, 2 * C, device=x.device)
+        d_ua, d_ub = d_u.chunk(2, 1)
+        _segment_sum(d_a1, gi.out_ptr, gi.out_edge, N, st, y=pre_a, mode=4 | (act << 4), out=d_ua)
+        _segment_sum(d_a1, gi.in_ptr, gi.in_edge, N, st, y=pre_a, mode=4 | (act << 4), out=d_ub)
+        d_nw = torch.empty(N, 2 * C, device=x.device)
+        d_xc, d_xk = d_nw.chunk(2, 1)
+        _lin_dgrad(d_u, w_1cat, st, d_xc)
         if wg:
             # the bias b_1 enters once per edge through the u_a half: d b_1 = column sums of d_u[:, :C]
-            dw_1cat, db_cat = _lin_wgrad(d_u, 2 * C, nw, 2 * C, N, w_1cat, True, st)
+            dw_1cat, db_cat = _lin_wgrad(d_u, xc, w_1cat, True, st)
             dw_1, db_1 = torch.cat([dw_1cat[:C], dw_1cat[C:]], dim=1), db_cat[:C]
             if s_w1 is not None:
                 s_w1.add_(dw_1)
@@ -718,52 +726,27 @@ class _InteractionLayer(torch.autograd.Function):
                 db_1 = None
         # bw = basis_weight(lw) ; lw = twobody(B, g) ; g = f_three(tbw) ; tbw = threebody(B, ...)
         if wg:
-            dw_b, _ = _lin_wgrad(d_bw, C, lw, C, E, w_b, False, st, s_wb)
-        d_lw = d_preh  # reuse
-        _lin_dgrad(d_bw, C, E, w_b, d_lw, C, 0, st)
-        dP = torch.empty(E, 1 + valence, C, device=dev)
-        d_g = torch.empty(E, Cp, device=dev)
-        _call("lcao_twobody_bwd", ptr(psum), 1 + valence, ptr(g), ptr(d_lw), E, C, 1, valence, 1, ptr(dP), ptr(d_g), st)
+            dw_b, _ = _lin_wgrad(d_bw, lw, w_b, False, st, s_wb)
+        d_lw = _lin_dgrad(d_bw, w_b, st, d_preh)  # (reuses d_preh)
+        dP, d_g = _twobody_bwd(psum, g, d_lw, 1, valence, True, st)
         if wg:
-            dw_3, _ = _lin_wgrad(d_g, Cp, tbw, C, E, w_3, False, st, s_w3)
-        d_tbw = d_bw  # reuse
-        _lin_dgrad(d_g, Cp, E, w_3, d_tbw, C, 0, st)
-        dB = torch.empty(E, NG, C, device=dev)
-        q = d_a1  # reuse
-        du_ks = torch.empty(E, 3, device=dev) if need_unit else None
-        du_st = torch.empty(E, 3, device=dev) if need_unit else None
-        _call("lcao_threebody_bwd", ptr(B), NG, ptr(gram), ptr(unit), ptr(gate), C, ptr(gi.in_ptr), ptr(gi.in_edge),
-              ptr(gi.in_src), ptr(gi.out_ptr), ptr(gi.out_edge), N, E, C, NL, ptr(d_tbw), ptr(dP), ptr(dB), ptr(q),
-              ptr(du_ks), ptr(du_st), st)
-        _call("lcao_segment_sum", ptr(q), C, None, 0, ptr(gi.out_ptr), ptr(gi.out_edge), N, C, 0, d_nw.data_ptr() + 4 * C,
-              2 * C, st)  # d_xk = d_nw[:, C:]
+            dw_3, _ = _lin_wgrad(d_g, tbw, w_3, False, st, s_w3)
+        d_tbw = _lin_dgrad(d_g, w_3, st, d_bw)  # (reuses d_bw)
+        dB, d_unit = _threebody_bwd(B, gram, unit, gate, gi, NL, d_tbw, dP, d_a1, d_xk, need_unit, st)  # (q reuses d_a1)
         # B = pair_contract(tab, rb) ; tab = f_coeffs(table)
         need_tab = wg and (ctx.needs_input_grad[1] or any(ctx.needs_input_grad[6:8]))
-        d_rb = torch.empty(E, O, device=dev) if need_rb else None
-        if need_tab or (need_rb and E > 0):  # (an edge-less batch has no d rb to write)
-            kptr, kperm = _grouping(grouping, pair, P)
-            d_tab = torch.empty(P, O, Cp, device=dev) if need_tab else None
-            scratch = None
-            if need_tab:
-                nbytes = int(_lib.load().lcao_pair_contract_bwd_scratch(E, P, O, C, valence))
-                scratch = torch.empty((nbytes + 15) // 16 * 4, dtype=torch.int32, device=dev)
-            _call("lcao_pair_contract_bwd", ptr(tab), ptr(pair), ptr(kptr), ptr(kperm), ptr(rb), ptr(vmask), ptr(lgrp), ptr(dB), E,
-                  P, O, C, NL, valence, ptr(d_tab), ptr(d_rb), ptr(scratch), st)
+        d_tab, d_rb = _pair_contract_bwd(tab, pair, grouping, rb, vmask, lgrp, dB, NL, C, need_tab, need_rb, st)
         if need_tab:
-            d_pre2 = _act_bwd(d_tab, pre2, P * O, Cp, st, act)
-            dw_c2, _ = _lin_wgrad(d_pre2, Cp, t1, C, P * O, w_c2, False, st, s_wc2)
-            d_pre1 = torch.empty(P * O, C, device=dev)
-            _lin_dgrad_act(d_pre2, Cp, P * O, w_c2, pre1, d_pre1, C, st, act)
-            dw_c0, _ = _lin_wgrad(d_pre1, C, table, K, P * O, w_c0, False, st, s_wc0)
+            d_pre2 = _act_bwd(d_tab.view(P * O, -1), pre2, act, st)
+            dw_c2, _ = _lin_wgrad(d_pre2, t1, w_c2, False, st, s_wc2)
+            d_pre1 = _lin_dgrad_act(d_pre2, w_c2, pre1, act, st)
+            dw_c0, _ = _lin_wgrad(d_pre1, _rows(table, True), w_c0, False, st, s_wc0)
             if ctx.needs_input_grad[1]:
-                d_table = torch.empty(P, O, K, device=dev)
-                _lin_dgrad(d_pre1, C, P * O, w_c0, d_table, K, 0, st)
+                d_table = _lin_dgrad(d_pre1, w_c0, st).view(P, O, K)
         # nw = node_weight(x) ; residual
         if wg:
-            dw_n, db_n = _lin_wgrad(d_nw, 2 * C, x, H, N, w_n, True, st, s_wn, s_bn)
-        dx = d_out.clone()
-        _lin_dgrad(d_nw, 2 * C, N, w_n, dx, H, 1, st)
-        d_unit = (du_ks + du_st) if need_unit else None
+            dw_n, db_n = _lin_wgrad(d_nw, x, w_n, True, st, s_wn, s_bn)
+        dx = _lin_dgrad(d_nw, w_n, st, d_out.clone(), accumulate=1)
         return dx, d_table, d_rb, d_unit, dw_n, db_n, dw_c0, dw_c2, dw_3, dw_b, dw_1, db_1, dw_2, db_2, dw_o, None
 
 
@@ -849,17 +832,43 @@ def pair_outer(fe, za, zb):
 # ------------------------------------------------------------------------------------------------
 # gathers / segment sums
 # ------------------------------------------------------------------------------------------------
+def _segment_sum(x, seg_ptr, seg_perm, R, st, y=None, mode=0, out=None):
+    """out[r] = sum of x[i] over the items i of segment r (`mode` bit 0: the mean); with `y`, of x[i] * y[i], or with
+    bit 1 / bit 2 set of x[i] * act(y[i]) / x[i] * act'(y[i]) for the activation in bits 4+.  out is allocated (R, C)
+    unless the caller passes it."""
+    C = x.shape[1]
+    if out is None:
+        out = torch.empty(R, C, device=x.device)
+    _call("lcao_segment_sum", ptr(x), x.stride(0), ptr(y), y.stride(0) if y is not None else 0, ptr(seg_ptr),
+          ptr(seg_perm), R, C, mode, ptr(out), out.stride(0), st)
+    return out
+
+
+def _gather_rows(table, idx, st, mul=None):
+    """out[i] = table[idx[i]] (* mul[i]) for every entry of idx (int32 or int64)."""
+    n, W = idx.numel(), table.shape[1]
+    out = torch.empty(n, W, device=table.device)
+    _call("lcao_gather_rows", ptr(table), table.stride(0), ptr(idx), 1 if idx.dtype == torch.int64 else 0, ptr(mul),
+          mul.stride(0) if mul is not None else 0, n, W, ptr(out), W, st)
+    return out
+
+
+def _edge_pair_fwd(a, b, bias, gi, act, need_pre, st):
+    """(out, pre): out = act(pre), pre = a[s_e] + b[t_e] + bias, kept only when `need_pre` (else None)."""
+    C = a.shape[1]
+    out = torch.empty(gi.E, C, device=a.device)
+    pre = torch.empty(gi.E, C, device=a.device) if need_pre else None
+    _call("lcao_edge_pair_fwd", ptr(a), a.stride(0), ptr(b), b.stride(0), ptr(bias), ptr(gi.src32), ptr(gi.dst32), gi.E,
+          C, act, ptr(out), ptr(pre), st)
+    return out, pre
+
+
 class _EdgePair(torch.autograd.Function):
     @staticmethod
     def forward(ctx, a, b, bias, gi: GraphIndex, act: int):
         require_cuda(a, b)
         assert a.stride(1) == 1 and b.stride(1) == 1
-        C = a.shape[1]
-        out = torch.empty(gi.E, C, device=a.device)
-        need_pre = act != ACT_NONE and any(ctx.needs_input_grad)
-        pre = torch.empty(gi.E, C, device=a.device) if need_pre else None
-        _call("lcao_edge_pair_fwd", ptr(a), a.stride(0), ptr(b), b.stride(0), ptr(bias), ptr(gi.src32), ptr(gi.dst32),
-              gi.E, C, act, ptr(out), ptr(pre), stream_ptr())
+        out, pre = _edge_pair_fwd(a, b, bias, gi, act, act != ACT_NONE and any(ctx.needs_input_grad), stream_ptr())
         ctx.gi, ctx.act, ctx.has_bias = gi, act, bias is not None
         ctx.save_for_backward(pre)
         return out
@@ -869,17 +878,12 @@ class _EdgePair(torch.autograd.Function):
     def backward(ctx, d_out):
         (pre,) = ctx.saved_tensors
         gi = ctx.gi
-        d_out = d_out.contiguous()
-        E, C = d_out.shape
+        d_out = _rows(d_out, True)
         st = stream_ptr()
         if ctx.act != ACT_NONE:
-            dh = torch.empty_like(d_out)
-            _call("lcao_act_bwd", ptr(d_out), C, ptr(pre), C, ptr(dh), C, E, C, ctx.act, st)
-            d_out = dh
-        da = torch.empty(gi.N, C, device=d_out.device)
-        db = torch.empty(gi.N, C, device=d_out.device)
-        _call("lcao_segment_sum", ptr(d_out), C, None, 0, ptr(gi.out_ptr), ptr(gi.out_edge), gi.N, C, 0, ptr(da), C, st)
-        _call("lcao_segment_sum", ptr(d_out), C, None, 0, ptr(gi.in_ptr), ptr(gi.in_edge), gi.N, C, 0, ptr(db), C, st)
+            d_out = _act_bwd(d_out, pre, ctx.act, st)
+        da = _segment_sum(d_out, gi.out_ptr, gi.out_edge, gi.N, st)
+        db = _segment_sum(d_out, gi.in_ptr, gi.in_edge, gi.N, st)
         dbias = da.sum(0) if ctx.has_bias else None
         return da, db, dbias, None, None
 
@@ -895,11 +899,8 @@ class _MulSegSum(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, y, gi: GraphIndex):
         require_cuda(x, y)
-        x, y = x.contiguous(), y.contiguous()
-        C = x.shape[1]
-        out = torch.empty(gi.N, C, device=x.device)
-        _call("lcao_segment_sum", ptr(x), C, ptr(y), C, ptr(gi.out_ptr), ptr(gi.out_edge), gi.N, C, 0, ptr(out), C,
-              stream_ptr())
+        x, y = _rows(x, True), _rows(y, True)
+        out = _segment_sum(x, gi.out_ptr, gi.out_edge, gi.N, stream_ptr(), y=y)
         ctx.gi = gi
         ctx.save_for_backward(x, y)
         return out
@@ -908,14 +909,8 @@ class _MulSegSum(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, d_out):
         x, y = ctx.saved_tensors
-        gi = ctx.gi
-        d_out = d_out.contiguous()
-        E, C = x.shape
-        st = stream_ptr()
-        dx, dy = torch.empty_like(x), torch.empty_like(y)
-        _call("lcao_gather_rows", ptr(d_out), C, ptr(gi.src32), 0, ptr(y), C, E, C, ptr(dx), C, st)
-        _call("lcao_gather_rows", ptr(d_out), C, ptr(gi.src32), 0, ptr(x), C, E, C, ptr(dy), C, st)
-        return dx, dy, None
+        d_out, st = _rows(d_out, True), stream_ptr()
+        return _gather_rows(d_out, ctx.gi.src32, st, mul=y), _gather_rows(d_out, ctx.gi.src32, st, mul=x), None
 
 
 def mul_segment_sum(x, y, gi):
@@ -929,12 +924,8 @@ class _SegmentReduce(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, seg_ptr, seg_perm, seg_of_item, mean: bool):
         require_cuda(x)
-        x2 = _rows(x)
-        R, C = seg_ptr.numel() - 1, x2.shape[1]
-        out = torch.empty(R, C, device=x.device)
-        _call("lcao_segment_sum", ptr(x2), _ld(x2), None, 0, ptr(seg_ptr), ptr(seg_perm), R, C, 1 if mean else 0,
-              ptr(out), C, stream_ptr())
-        ctx.mean, ctx.n = mean, x2.shape[0]
+        out = _segment_sum(_rows(x), seg_ptr, seg_perm, seg_ptr.numel() - 1, stream_ptr(), mode=1 if mean else 0)
+        ctx.mean = mean
         ctx.save_for_backward(seg_ptr, seg_of_item, x)
         return out
 
@@ -947,15 +938,11 @@ class _SegmentReduce(torch.autograd.Function):
                 out = second_order.segment_reduce(x_, seg_of_item, seg_ptr.numel() - 1, ctx.mean)
                 (gx,) = second_order.grads_with_graph([out], [x_], [d_out], [True])
             return gx, None, None, None, None
-        d_out = d_out.contiguous()
+        d_out = _rows(d_out, True)
         if ctx.mean:
             cnt = (seg_ptr[1:] - seg_ptr[:-1]).clamp(min=1).to(d_out.dtype)
             d_out = d_out / cnt.unsqueeze(-1)
-        C = d_out.shape[1]
-        dx = torch.empty(ctx.n, C, device=d_out.device)
-        _call("lcao_gather_rows", ptr(d_out), C, ptr(seg_of_item), 1 if seg_of_item.dtype == torch.int64 else 0, None,
-              0, ctx.n, C, ptr(dx), C, stream_ptr())
-        return dx, None, None, None, None
+        return _gather_rows(d_out, seg_of_item, stream_ptr()), None, None, None, None
 
 
 def segment_reduce(x, seg_ptr, seg_perm, seg_of_item, mean=False):
@@ -970,13 +957,10 @@ class _GatherRows(torch.autograd.Function):
         require_cuda(table, idx)
         t2 = table.reshape(table.shape[0], -1)
         assert t2.stride(1) == 1
-        n, W = idx.numel(), t2.shape[1]
-        out = torch.empty(n, W, device=table.device)
-        _call("lcao_gather_rows", ptr(t2), t2.stride(0), ptr(idx), 1 if idx.dtype == torch.int64 else 0, None, 0, n, W,
-              ptr(out), W, stream_ptr())
+        out = _gather_rows(t2, idx, stream_ptr())
         ctx.tshape = table.shape
         ctx.save_for_backward(key_ptr, key_perm)
-        return out.reshape(n, *table.shape[1:])
+        return out.reshape(idx.numel(), *table.shape[1:])
 
     @staticmethod
     @once_differentiable

@@ -165,18 +165,20 @@ def test_device_collated_stream_feeds_fresh_batches():
                 assert rel_l2(q.grad, p.grad) < 2e-5, (step, n)
 
 
-def test_deferred_weight_gradient_reduction_is_bitwise_the_same(monkeypatch):
+def test_deferred_weight_gradient_reduction_is_bitwise_the_same_as_per_layer_reduction():
     """With gradient sinks the second stage of the tcgen05 weight gradients is deferred to one batched launch at the end
-    of the backward pass (ops.defer_wgrad); same partial tiles, same summation order: the flat gradient bucket must be
-    bitwise equal to the one-reduction-per-layer path (interaction blocks), and nothing may be left pending."""
+    of the backward pass; same partial tiles, same summation order: the flat gradient bucket must be bitwise equal to
+    the one-reduction-per-layer path that the interaction blocks take without sinks (their gradients then come back
+    through autograd into the same zeroed bucket), and nothing may be left pending."""
     g = qm9_like_batch(96, seed=3).to(DEV)
     flats = []
-    for defer in (True, False):
-        monkeypatch.setattr(ops, "defer_wgrad", defer)
+    for in_place in (True, False):
         torch.manual_seed(5)
         model = LCAONet(cutoff=5.0, cutoff_net="polynomial").to(DEV).train()
         model.side_effect_keys = False
         bucket = FlatGradBucket(model)
+        for layer in model.int_layers:
+            layer.grads_in_place = in_place
         for _ in range(2):
             bucket.zero()
             out = model(g)
