@@ -273,13 +273,17 @@ int lcao_reduce_by_key(const float* x, int64_t ldx, const int32_t* kptr, const i
                        int64_t n, int32_t W, float* acc, void* stream);
 
 /* ---- dense layers (nn/base.py:11-81 = nn.Linear; sites listed in SURVEY.md §8 a-7) ------------- */
-/* Y = act(X W^T + bias); X (M,K) ldx, W (Nout,K) contiguous, Y (M,Nout) ldy; pre (nullable) gets X W^T + bias */
+/* Y = act(X W^T + bias); X (M,K) ldx, W (Nout,K) contiguous, Y (M,Nout) ldy; pre (nullable) gets X W^T + bias.
+ * The tcgen05 kernels split W into shared memory while the previous kernel of the stream may still run (programmatic
+ * dependent launch), so W must not be written by this library's immediately preceding launch on the same stream (a
+ * layer's weight is a parameter: no kernel of the pass writes it). */
 int lcao_linear_fwd(const float* X, int64_t ldx, const float* W, const float* bias, float* Y, int64_t ldy,
                     float* pre, int64_t ldp, int64_t M, int32_t K, int32_t Nout, int32_t act, int32_t mode,
                     void* stream);
 /* dX = (dY * act'(H)) W   (accumulate=1: dX += ...).  H (M,Nout) = the layer's pre-activation, or NULL /
- * act = NONE for a plain dY.  The tcgen05 path fuses the act' factor into its operand prologue; the
- * CUDA-core path needs `scratch` (M*Nout floats, may be NULL when act == NONE). */
+ * act = NONE for a plain dY.  dY * act'(H) is first formed in `scratch` (lcao_linear_bwd_scratch() floats: M*Nout;
+ * may be NULL when act == NONE).  W must not be written by this library's
+ * immediately preceding launch on the same stream (see lcao_linear_fwd); nor for lcao_linear_dgrad_act. */
 int lcao_linear_dgrad(const float* dY, int64_t ldy, const float* H, int64_t ldh, int32_t act, const float* W, float* dX,
                       int64_t ldx, int64_t M, int32_t K, int32_t Nout, int32_t accumulate, int32_t mode, float* scratch,
                       void* stream);
@@ -306,7 +310,7 @@ int lcao_wgrad_reduce_batch(const int64_t* desc, int32_t n, void* stream);
 int64_t lcao_linear_bwd_scratch(const float* dY, int64_t ldy, const float* H, int64_t ldh, int32_t act, const float* W,
                                 const float* X, int64_t ldx, const float* dX, int64_t lddx, int64_t M, int32_t K,
                                 int32_t Nout, int32_t mode);
-/* dH = dY * act'(H)  elementwise over (M,C) with row strides (in place allowed: dH == dY) */
+/* dH = dY * act'(H)  elementwise over (M,C) with row strides (in place allowed: dH == dY); any alignment and width */
 int lcao_act_bwd(const float* dY, int64_t ldy, const float* H, int64_t ldh, float* dH, int64_t ldd, int64_t M,
                  int32_t C, int32_t act, void* stream);
 /* Y = act(X) elementwise over (M,C) with row strides (in place allowed).  lcao_linear_fwd's tcgen05 epilogue fuses

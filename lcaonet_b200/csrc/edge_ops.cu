@@ -353,6 +353,21 @@ __global__ void k_act_bwd(const float* __restrict__ dY, int64_t ldy, const float
   st4(dH + i * ldd + c, g);
 }
 
+// the same, one element per thread, for rows that are not 16-byte aligned or widths / strides that are not multiples of 4
+// (the CUDA-core fallback of lcao_linear_dgrad_act applies the factor in place with the caller's G and dX)
+__global__ void k_act_bwd_any(const float* dY, int64_t ldy, const float* __restrict__ H, int64_t ldh, float* dH,
+                              int64_t ldd, int64_t M, int C, int act) {
+  pdl_trigger();
+  pdl_wait();
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= M * C) return;
+  const int64_t i = t / C;
+  const int c = (int)(t - i * C);
+  float g = dY[i * ldy + c];
+  if (act != LCAO_ACT_NONE) g *= act_gradf(act, __ldg(H + i * ldh + c));
+  dH[i * ldd + c] = g;
+}
+
 // backward of  agg[s] = sum_{e in out(s)} bw[e] * h[e]  with  h = SiLU(pre_h):
 //   d_bw[e] = d_agg[src[e]] * h[e] ;  d_pre_h[e] = d_agg[src[e]] * bw[e] * SiLU'(pre_h[e])
 template <bool GEN>
@@ -549,8 +564,14 @@ extern "C" int lcao_act_bwd(const float* dY, int64_t ldy, const float* H, int64_
                             int64_t M, int32_t C, int32_t act, void* stream) {
   if (M == 0 || C == 0) return LCAO_OK;
   LCAO_REQUIRE(dY && dH && (act == LCAO_ACT_NONE || H), "lcao_act_bwd: null buffer");
-  LCAO_REQUIRE(C % 4 == 0 && ldy % 4 == 0 && ldd % 4 == 0 && (act == LCAO_ACT_NONE || ldh % 4 == 0),
-               "lcao_act_bwd: need C and strides multiples of 4");
+  const bool vec = C % 4 == 0 && ldy % 4 == 0 && ldd % 4 == 0 && aligned16(dY) && aligned16(dH) &&
+                   (act == LCAO_ACT_NONE || (ldh % 4 == 0 && aligned16(H)));
+  if (!vec) {
+    LCAO_CUDA(launch_pdl(k_act_bwd_any, (unsigned)ceil_div64(M * C, 256), 256, 0, (cudaStream_t)stream, dY, ldy, H, ldh, dH,
+                         ldd, M, C, act));
+    LCAO_LAUNCH_CHECK();
+    return LCAO_OK;
+  }
   const unsigned grid = (unsigned)ceil_div64(M * (C / 4), 256);
   if (act <= LCAO_ACT_SILU) LCAO_CUDA(launch_pdl(k_act_bwd<false>, grid, 256, 0, (cudaStream_t)stream, dY, ldy, H, ldh, dH, ldd, M, C / 4, act));
   else LCAO_CUDA(launch_pdl(k_act_bwd<true>, grid, 256, 0, (cudaStream_t)stream, dY, ldy, H, ldh, dH, ldd, M, C / 4, act));
