@@ -217,7 +217,8 @@ int lcao_pair_outer_bwd(const float* dpre, const float* fe, const float* za, con
 int lcao_sigmoid_rows(const float* x, int64_t ldx, float* out, int64_t ldo, int64_t M, int32_t C, void* stream);
 /* tbw[e,:] = sum_{e' in in(s_e), e' != e} normalize( sum_l Y_l(unit[e].unit[e']) B[e',l,:] ) * gate[src[e'],:]
  * B has NG groups per edge (row stride NG*C); gram = its per-edge Gram matrices (|v|^2 = Y^T G Y);
- * gate (N,C) with row stride ldg.  B, gate (and d_tbw for the backward) must be 16-byte aligned: LCAO_E_ARG otherwise. */
+ * gate (N,C) with row stride ldg.  B, gate and tbw (and d_tbw, dP, dB and q for the backward) must be 16-byte aligned:
+ * LCAO_E_ARG otherwise. */
 int lcao_threebody_fwd(const float* B, int32_t NG, const double* gram, const float* unit, const float* gate,
                        int64_t ldg, const int32_t* in_ptr, const int32_t* in_edge, const int32_t* in_src,
                        const int32_t* out_ptr, const int32_t* out_edge, int64_t N, int64_t E, int32_t C,

@@ -15,7 +15,8 @@
 // are recomputed per (e,e') pair by one thread and broadcast through shared memory.
 //
 // These FP32-pipe kernels serve 128 < C <= 256; C <= 128 goes to threebody_mma.cu (forward) and threebody_staged.cu
-// (backward).  Both entry points require 16-byte-aligned B, gate and d_tbw: every kernel reads them in float4 rows.
+// (backward).  Both entry points require 16-byte-aligned B, gate and d_tbw (read in float4 rows or by bulk copies)
+// and tbw, dB, q and dP (written or read in float4 rows).
 //
 // Thread mapping: lane <-> float4 channel columns (lane and lane + 32), warp <-> 8 out-edges of a node
 // (forward: 8 register accumulators) or one in-edge (backward).  Warps are independent: B / gate / d_tbw
@@ -462,7 +463,7 @@ int lcao_tb_staged_bwd(const float* B, int32_t NG, const double* gram, const flo
                        const int32_t* out_edge, int64_t N, int32_t C, int32_t NL, const float* d_tbw, const float* dP,
                        float* dB, float* q, float* du_ks, float* du_st, cudaStream_t st);
 
-// every kernel reads these rows with 16-byte loads or bulk copies
+// every kernel reads or writes these rows with 16-byte accesses or bulk copies
 static bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 #define TB_DISPATCH(NL, CALL)     \
@@ -482,7 +483,7 @@ extern "C" int lcao_threebody_fwd(const float* B, int32_t NG, const double* gram
                "lcao_threebody_fwd: null buffer");
   LCAO_REQUIRE(C % 4 == 0 && C > 0 && C <= 256 && NL >= 1 && NL <= 4 && NG >= NL && ldg % 4 == 0,
                "lcao_threebody_fwd: need C %% 4 == 0, C <= 256, 1 <= NL <= 4, NG >= NL (C=%d NL=%d NG=%d)", C, NL, NG);
-  LCAO_REQUIRE(al16(B) && al16(gate), "lcao_threebody_fwd: B and gate must be 16-byte aligned");
+  LCAO_REQUIRE(al16(B) && al16(gate) && al16(tbw), "lcao_threebody_fwd: B, gate and tbw must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   if (C <= 128) return lcao_tb_mma_fwd(B, NG, gram, unit, gate, ldg, in_ptr, in_edge, in_src, out_ptr, out_edge, N, C, NL, tbw, st);
   const unsigned grid = (unsigned)(N < 148ll * kFwdCtasPerSm ? N : 148ll * kFwdCtasPerSm);
@@ -508,7 +509,8 @@ extern "C" int lcao_threebody_bwd(const float* B, int32_t NG, const double* gram
                "lcao_threebody_bwd: need C %% 4 == 0, C <= 256, 1 <= NL <= 4, NG >= NL");
   LCAO_REQUIRE((d_unit_ks == nullptr) == (d_unit_st == nullptr), "lcao_threebody_bwd: pass both d_unit buffers or neither");
   LCAO_REQUIRE(NG <= NL + 1, "lcao_threebody_bwd: at most one valence group (NG <= NL + 1)");
-  LCAO_REQUIRE(al16(B) && al16(gate) && al16(d_tbw), "lcao_threebody_bwd: B, gate and d_tbw must be 16-byte aligned");
+  LCAO_REQUIRE(al16(B) && al16(gate) && al16(d_tbw) && al16(dB) && al16(q) && al16(dP),
+               "lcao_threebody_bwd: B, gate, d_tbw, dP, dB and q must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   const bool forces = d_unit_ks != nullptr;
   if (C <= 128)

@@ -55,11 +55,17 @@ def test_argument_errors_are_reported_without_a_gpu():
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="without the check, a GPU would run the kernels on these addresses")
 def test_threebody_rejects_unaligned_rows():
-    # pointer values only: every kernel reads B, gate and d_tbw with 16-byte loads or bulk copies
+    # pointer values only: every kernel reads B, gate, d_tbw and dP and writes tbw, dB and q with 16-byte accesses or
+    # bulk copies.  Each case misaligns one pointer; C = 128 and C = 256 reach both kernel families' entry points.
     lib = _lib.load()
     a, odd = 16, 4
-    rc = lib.lcao_threebody_fwd(odd, 3, a, a, a, 128, a, a, a, a, a, 4, 4, 128, 3, a, None)
-    assert rc == -1 and b"aligned" in lib.lcao_last_error()
-    for B, d_tbw in ((odd, a), (a, odd)):
-        rc = lib.lcao_threebody_bwd(B, 3, a, a, a, 128, a, a, a, a, a, 4, 4, 128, 3, d_tbw, None, a, a, None, None, None)
-        assert rc == -1 and b"aligned" in lib.lcao_last_error()
+    for C in (128, 256):
+        for B, gate, tbw in ((odd, a, a), (a, odd, a), (a, a, odd)):
+            rc = lib.lcao_threebody_fwd(B, 3, a, a, gate, C, a, a, a, a, a, 4, 4, C, 3, tbw, None)
+            assert rc == -1 and b"aligned" in lib.lcao_last_error(), (C, B, gate, tbw)
+        bwd = dict(B=a, gate=a, d_tbw=a, dP=a, dB=a, q=a)
+        for name in bwd:
+            p = dict(bwd, **{name: odd})
+            rc = lib.lcao_threebody_bwd(p["B"], 3, a, a, p["gate"], C, a, a, a, a, a, 4, 4, C, 3, p["d_tbw"], p["dP"], p["dB"],
+                                        p["q"], None, None, None)
+            assert rc == -1 and b"aligned" in lib.lcao_last_error(), (C, name)
