@@ -127,7 +127,8 @@ int lcao_neighbor_fill(const float* pos, const int64_t* batch, const int32_t* gr
                        void* stream);
 
 /* ---- geometry + radial basis (base.py:27-43, rbf.py:92-103,129-142, cutoff.py:32-67) --------- */
-/* dist (E), unit (E,3), rb (E,O), optional drb (E,O) = d rb / d r (for autograd forces). */
+/* dist (E), unit (E,3), rb (E,O), optional drb (E,O) = d rb / d r (for autograd forces).  An unknown
+ * spec->cutoff_kind or spec->rbf_kind is LCAO_E_ARG. */
 int lcao_geom_basis_fwd(const float* pos, const float* shift, const float* lattice, const int64_t* batch,
                         const int32_t* src32, const int32_t* dst32, int64_t E, const lcao_basis_spec* spec_host,
                         float* dist, float* unit, float* rb, float* drb, void* stream);
@@ -158,10 +159,12 @@ int lcao_geom_cell_bwd(const float* pos, const float* shift, const float* lattic
 /* ---- orbital contraction (the einsum "ed,edh->eh" sites lcaonet.py:180-183,200-203) ----------- */
 /* B[e,l,:]  = sum_{o: l(o)=l} rb[e,o] * (A[e,o,:] + m[e,o] V[e,o,:])        l = 0..NL-1
  * B[e,NL,:] = sum_o rb[e,o] m[e,o] V[e,o,:]                                  (only if valence)
- * with cst1 (E,O,Cp) = [A | V], Cp = C or 2C; lgrp (O) = l of each orbital; vmask (E,O) 0/1 floats. */
+ * with cst1 (E,O,Cp) = [A | V], Cp = C or 2C; lgrp (O) = l of each orbital; vmask (E,O) 0/1 floats.
+ * cst1 and B must be 16-byte aligned: LCAO_E_ARG otherwise. */
 int lcao_coeff_contract_fwd(const float* cst1, const float* rb, const float* vmask, const int32_t* lgrp,
                             int64_t E, int32_t O, int32_t C, int32_t NL, int32_t valence, float* B, void* stream);
-/* d_cst1 (E,O,Cp) from dB (E,NG,C); d_rb (E,O) written if non-NULL. */
+/* d_cst1 (E,O,Cp) from dB (E,NG,C); d_rb (E,O) written if non-NULL.  dB, d_cst1 and, when d_rb is given, cst1 must
+ * be 16-byte aligned: LCAO_E_ARG otherwise. */
 int lcao_coeff_contract_bwd(const float* cst1, const float* rb, const float* vmask, const int32_t* lgrp,
                             const float* dB, int64_t E, int32_t O, int32_t C, int32_t NL, int32_t valence,
                             float* d_cst1, float* d_rb, void* stream);
@@ -174,14 +177,16 @@ int lcao_coeff_contract_bwd(const float* cst1, const float* rb, const float* vma
  * with tab (P,O,Cp) = [A | V].  gram (nullable): (E, NL(NL+1)/2) FP64 upper triangle of B[e,l,:].B[e,l',:]
  * over the first NL groups (consumed by lcao_threebody_*).  psum (nullable): (E, 1 + valence, C) =
  * [sum_{l<NL} B[e,l,:] | B[e,NL,:]] — the only part of B the two-body weight needs; lcao_twobody_fwd/bwd accept it
- * in place of B with NG = 1 + valence, NL = 1 (a third of the bytes). */
+ * in place of B with NG = 1 + valence, NL = 1 (a third of the bytes).  tab, B and psum must be 16-byte aligned:
+ * LCAO_E_ARG otherwise. */
 int lcao_pair_contract_fwd(const float* tab, const int64_t* pair, const float* rb, const float* vmask,
                            const int32_t* lgrp, int64_t E, int32_t O, int32_t C, int32_t NL, int32_t valence,
                            float* B, double* gram, float* psum, void* stream);
 /* d_tab (P,O,Cp) = keyed reduction of rb[e,o] dB[e,l(o),:] over the edges of each pair, deterministic
  * (two stages, no atomics); (kptr (P+1), kperm (E)) = edges grouped by pair (lcao_bucket_sort).
  * d_rb (E,O) written if non-NULL (autograd forces); d_tab may be NULL when only d_rb is wanted (the positions-only
- * pass of autograd forces).  scratch: lcao_pair_contract_bwd_scratch() BYTES. */
+ * pass of autograd forces).  scratch: lcao_pair_contract_bwd_scratch() BYTES.  dB, d_tab, scratch and, when d_rb is
+ * given, tab must be 16-byte aligned: LCAO_E_ARG otherwise (every argument is checked before the first launch). */
 int lcao_pair_contract_bwd(const float* tab, const int64_t* pair, const int32_t* kptr, const int32_t* kperm,
                            const float* rb, const float* vmask, const int32_t* lgrp, const float* dB, int64_t E,
                            int64_t P, int32_t O, int32_t C, int32_t NL, int32_t valence, float* d_tab, float* d_rb,

@@ -432,7 +432,7 @@ extern "C" int lcao_coeff_contract_fwd(const float* cst1, const float* rb, const
   LCAO_REQUIRE(cst1 && rb && lgrp && B && (!valence || vmask), "lcao_coeff_contract_fwd: null buffer");
   LCAO_REQUIRE(C % 4 == 0 && C > 0 && O > 0 && O <= LCAO_MAX_ORB && NL >= 1 && NL <= 4,
                "lcao_coeff_contract_fwd: need C %% 4 == 0, O <= %d, 1 <= NL <= 4 (got C=%d O=%d NL=%d)", LCAO_MAX_ORB, C, O, NL);
-  LCAO_REQUIRE(aligned16(cst1) && aligned16(B), "lcao_coeff_contract_fwd: buffers must be 16-byte aligned");
+  LCAO_REQUIRE(aligned16(cst1) && aligned16(B), "lcao_coeff_contract_fwd: cst1 and B must be 16-byte aligned");
   const unsigned grid = (unsigned)ceil_div64(E, kWarpsPerCta);
   cudaStream_t st = (cudaStream_t)stream;
   DISPATCH_NL_VAL(NL, valence != 0, k_coeff_contract_fwd, <<<grid, kWarpsPerCta * 32, 0, st>>>(cst1, rb, vmask, lgrp, E, O, C, B));
@@ -447,7 +447,8 @@ extern "C" int lcao_coeff_contract_bwd(const float* cst1, const float* rb, const
   LCAO_REQUIRE(rb && lgrp && dB && d_cst1 && (!valence || vmask) && (!d_rb || cst1), "lcao_coeff_contract_bwd: null buffer");
   LCAO_REQUIRE(C % 4 == 0 && C > 0 && O > 0 && O <= LCAO_MAX_ORB && NL >= 1 && NL <= 4,
                "lcao_coeff_contract_bwd: need C %% 4 == 0, O <= %d, 1 <= NL <= 4", LCAO_MAX_ORB);
-  LCAO_REQUIRE(aligned16(dB) && aligned16(d_cst1), "lcao_coeff_contract_bwd: buffers must be 16-byte aligned");
+  LCAO_REQUIRE(aligned16(dB) && aligned16(d_cst1) && (!d_rb || aligned16(cst1)),
+               "lcao_coeff_contract_bwd: dB, d_cst1 and (with d_rb) cst1 must be 16-byte aligned");
   const unsigned grid = (unsigned)ceil_div64(E, kWarpsPerCta);
   cudaStream_t st = (cudaStream_t)stream;
   DISPATCH_NL_VAL(NL, valence != 0, k_coeff_contract_bwd, <<<grid, kWarpsPerCta * 32, 0, st>>>(cst1, rb, vmask, lgrp, dB, E, O, C, d_cst1, d_rb));

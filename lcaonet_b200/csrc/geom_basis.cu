@@ -225,6 +225,9 @@ extern "C" int lcao_geom_basis_fwd(const float* pos, const float* shift, const f
   LCAO_REQUIRE(pos && shift && lattice && src32 && dst32 && sp && dist && unit && rb, "lcao_geom_basis_fwd: null buffer");
   LCAO_REQUIRE(sp->n_unique >= 1 && sp->n_unique <= LCAO_MAX_UNIQUE_ORB && sp->n_rep >= 1,
                "lcao_geom_basis_fwd: bad orbital count");
+  LCAO_REQUIRE(sp->cutoff_kind >= LCAO_CUT_POLYNOMIAL && sp->cutoff_kind <= LCAO_CUT_COSINE &&
+                   (sp->rbf_kind == LCAO_RBF_HYDROGEN || sp->rbf_kind == LCAO_RBF_SPHERICAL_BESSEL),
+               "lcao_geom_basis_fwd: unknown cutoff_kind %d or rbf_kind %d", sp->cutoff_kind, sp->rbf_kind);
   for (int u = 0; u < sp->n_unique; ++u)
     LCAO_REQUIRE(sp->deg[u] >= 0 && sp->deg[u] < LCAO_MAX_POLY && sp->l[u] >= 0 && sp->l[u] <= 3,
                  "lcao_geom_basis_fwd: bad orbital entry %d", u);

@@ -395,7 +395,7 @@ extern "C" int lcao_pair_contract_fwd(const float* tab, const int64_t* pair, con
   LCAO_REQUIRE(tab && pair && rb && lgrp && B && (!valence || vmask), "lcao_pair_contract_fwd: null buffer");
   LCAO_REQUIRE(C % 4 == 0 && C > 0 && O > 0 && O <= LCAO_MAX_ORB && NL >= 1 && NL <= 4,
                "lcao_pair_contract_fwd: need C %% 4 == 0, O <= %d, 1 <= NL <= 4 (got C=%d O=%d NL=%d)", LCAO_MAX_ORB, C, O, NL);
-  LCAO_REQUIRE(al16(tab) && al16(B), "lcao_pair_contract_fwd: buffers must be 16-byte aligned");
+  LCAO_REQUIRE(al16(tab) && al16(B) && al16(psum), "lcao_pair_contract_fwd: tab, B and psum must be 16-byte aligned");
   const int64_t want = ceil_div64(E, kWarps);
   const unsigned grid = (unsigned)(want < 148 * 16 ? want : 148 * 16);
   cudaStream_t st = (cudaStream_t)stream;
@@ -440,7 +440,9 @@ extern "C" int lcao_pair_contract_bwd(const float* tab, const int64_t* pair, con
   LCAO_REQUIRE(E == 0 || (kperm && rb && lgrp && dB && (!valence || vmask)), "lcao_pair_contract_bwd: null buffer");
   LCAO_REQUIRE(C % 4 == 0 && C > 0 && O > 0 && O <= LCAO_MAX_ORB && NL >= 1 && NL <= 4,
                "lcao_pair_contract_bwd: need C %% 4 == 0, O <= %d, 1 <= NL <= 4", LCAO_MAX_ORB);
-  LCAO_REQUIRE(al16(dB) && al16(d_tab) && al16(scratch), "lcao_pair_contract_bwd: buffers must be 16-byte aligned");
+  LCAO_REQUIRE(!d_rb || E == 0 || (tab && pair), "lcao_pair_contract_bwd: d_rb needs tab and pair");
+  LCAO_REQUIRE(al16(dB) && al16(d_tab) && al16(scratch) && (!d_rb || al16(tab)),
+               "lcao_pair_contract_bwd: dB, d_tab, scratch and (with d_rb) tab must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   int32_t* cptr = static_cast<int32_t*>(scratch);
   float* partial = reinterpret_cast<float*>(static_cast<char*>(scratch) + ((P + 1 + 3) / 4) * 16);
@@ -464,7 +466,6 @@ extern "C" int lcao_pair_contract_bwd(const float* tab, const int64_t* pair, con
   LCAO_LAUNCH_CHECK();
   }
   if (d_rb && E > 0) {
-    LCAO_REQUIRE(tab && pair, "lcao_pair_contract_bwd: d_rb needs tab and pair");
     if (C <= 128) {  // pair-sorted walk: table rows stay in registers across a run of equal pairs
       const unsigned grid = (unsigned)ceil_div64(ceil_div64(E, 16), kWarps);
       if (valence) k_pair_contract_drb_sorted<true><<<grid, kWarps * 32, 0, st>>>(tab, pair, kperm, vmask, lgrp, dB, E, O, C, NL, d_rb);
