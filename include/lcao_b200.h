@@ -106,7 +106,8 @@ int lcao_triplets_fill(const int32_t* src32, const int32_t* in_ptr, const int32_
                        const int32_t* tri_ptr, int64_t E, int64_t* tri_k, int64_t* e_ks, int64_t* e_st,
                        const float* unit, float* cos_out, void* stream);
 
-/* histogram of small integer keys (pair / species counts for the BatchNorm statistics) */
+/* histogram of small integer keys (pair / species counts for the BatchNorm statistics): counts (nb) = the number of
+ * keys equal to each value in [0, nb); keys outside that range are dropped.  Exact below 2^24 per bucket. */
 int lcao_histogram(const int64_t* keys, int64_t n, int64_t nb, float* counts, void* stream);
 
 /* ---- neighbour list under PBC (data/convert.py:103-172 atoms2graphdata; ase.neighborlist.neighbor_list) -------- */
@@ -200,7 +201,9 @@ int lcao_coeff_gram(const float* B, int32_t NG, int64_t E, int32_t C, int32_t NL
  * depend on the species, the coefficient rows on the species pair: DESIGN.md R6).  training != 0: batch statistics
  * (biased variance), running_mean / running_var (nullable together) updated with `momentum` and the unbiased variance,
  * *num_batches_tracked (nullable) incremented; training == 0: the running statistics normalise.  gamma / beta nullable
- * (affine=False).  save_mean / save_rstd (F) are kept for the backward pass. */
+ * (affine=False).  save_mean / save_rstd (F) are kept for the backward pass.  Training at a total count n = 1: the mean
+ * is the row itself, the variance 0 and running_var becomes NaN (0 * n/(n-1); nn.BatchNorm1d raises instead); at n = 0
+ * the batch statistics, y and the running statistics are NaN. */
 int lcao_table_norm_fwd(const float* x, const float* counts, const float* gamma, const float* beta, int64_t R, int32_t F,
                         float eps, float momentum, int32_t training, float* running_mean, float* running_var,
                         int64_t* num_batches_tracked, float* y, float* save_mean, float* save_rstd, void* stream);
@@ -254,7 +257,8 @@ int lcao_twobody_bwd(const float* B, int32_t NG, const float* g, const float* d_
 
 /* ---- edge <- node gathers and node <- edge segment sums (torch_scatter sites lcaonet.py:208,293,307;
  *      ATen index sites lcaonet.py:209) --------------------------------------------------------- */
-/* out[e,:] = act(a[src[e],:] + b[dst[e],:] + bias) ; pre[e,:] (nullable) = value before act */
+/* out[e,:] = act(a[src[e],:] + b[dst[e],:] + bias) ; pre[e,:] (nullable) = value before act.  a, b, out and, when
+ * given, bias and pre must be 16-byte aligned; act outside [LCAO_ACT_NONE, LCAO_ACT_LAST]: LCAO_E_ARG. */
 int lcao_edge_pair_fwd(const float* a, int64_t lda, const float* b, int64_t ldb, const float* bias,
                        const int32_t* src32, const int32_t* dst32, int64_t E, int32_t C, int32_t act,
                        float* out, float* pre, void* stream);
@@ -262,8 +266,8 @@ int lcao_edge_pair_fwd(const float* a, int64_t lda, const float* b, int64_t ldb,
  * `mean` is a flag word: bit 0: scale_r = 1/max(count,1) instead of 1; bit 1: y holds a pre-activation and the
  * factor is act(y) (the message sum then needs no stored copy of h = act(pre_h)); bit 2: the factor is act'(y)
  * (backward through an activation folded into the reduction that follows it); bits 4-7: the activation (LCAO_ACT_*,
- * 0 = SiLU).  Deterministic, no atomics.  x may be NULL when no segment
- * has any item (edge-less batch): out is zero-filled. */
+ * 0 = SiLU).  Bits 1 and 2 exclude each other and need y when x is given; any other bit set is LCAO_E_ARG.  Deterministic, no
+ * atomics.  x may be NULL when no segment has any item (edge-less batch): out is zero-filled. */
 int lcao_segment_sum(const float* x, int64_t ldx, const float* y, int64_t ldy, const int32_t* ptr,
                      const int32_t* perm, int64_t R, int32_t C, int32_t mean, float* out, int64_t ldo, void* stream);
 /* backward of the message sum  agg[s] = sum_{e in out(s)} bw[e] * h[e],  h = act(pre_h)  (lcaonet.py:207-214):
@@ -274,7 +278,9 @@ int lcao_msg_bwd(const float* d_agg, int64_t lda, const int32_t* src32, const fl
 /* out[i,:] = table[idx[i],:] * (mul ? mul[i,:] : 1)   (idx int64 or int32 chosen by idx_is64) */
 int lcao_gather_rows(const float* table, int64_t ldt, const void* idx, int32_t idx_is64, const float* mul, int64_t ldm,
                      int64_t n, int32_t W, float* out, int64_t ldo, void* stream);
-/* acc[key[i],:] += x[i,:]   (keys int64, few distinct values: pair / species tables; acc pre-zeroed) */
+/* acc[k,:] += sum_{j in [kptr[k], kptr[k+1])} x[kperm[j],:]   for the nkeys keys of the grouping (kptr (nkeys+1),
+ * kperm (n): lcao_bucket_sort); acc (nkeys, W) packed, W and ldx multiples of 4.  Each CTA sums 32 sorted entries and
+ * flushes every key run it holds with atomics: exact for integer-valued data, NOT bitwise reproducible otherwise. */
 int lcao_reduce_by_key(const float* x, int64_t ldx, const int32_t* kptr, const int32_t* kperm, int64_t nkeys,
                        int64_t n, int32_t W, float* acc, void* stream);
 
@@ -316,7 +322,8 @@ int lcao_wgrad_reduce_batch(const int64_t* desc, int32_t n, void* stream);
 int64_t lcao_linear_bwd_scratch(const float* dY, int64_t ldy, const float* H, int64_t ldh, int32_t act, const float* W,
                                 const float* X, int64_t ldx, const float* dX, int64_t lddx, int64_t M, int32_t K,
                                 int32_t Nout, int32_t mode);
-/* dH = dY * act'(H)  elementwise over (M,C) with row strides (in place allowed: dH == dY); any alignment and width */
+/* dH = dY * act'(H)  elementwise over (M,C) with row strides (in place allowed: dH == dY); any alignment and width.
+ * act outside [LCAO_ACT_NONE, LCAO_ACT_LAST]: LCAO_E_ARG. */
 int lcao_act_bwd(const float* dY, int64_t ldy, const float* H, int64_t ldh, float* dH, int64_t ldd, int64_t M,
                  int32_t C, int32_t act, void* stream);
 /* Y = act(X) elementwise over (M,C) with row strides (in place allowed).  lcao_linear_fwd's tcgen05 epilogue fuses

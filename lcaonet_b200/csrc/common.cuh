@@ -76,14 +76,15 @@ __device__ __forceinline__ float silu_gradf(float x) {
   return s * (1.0f + x * (1.0f - s));
 }
 // generic activation and its derivative as functions of the PRE-activation (torch semantics: F.softplus threshold 20,
-// exact-erf GELU, ELU alpha 1, LeakyReLU slope 0.01); SiLU is the hot case and comes first
+// exact-erf GELU, ELU alpha 1, LeakyReLU slope 0.01; ReLU maps NaN to NaN and passes the gradient at a NaN input, as
+// torch.relu / threshold_backward do); SiLU is the hot case and comes first
 __device__ __forceinline__ float softplusf_acc(float x) { return x > 20.0f ? x : log1pf(expf(x)); }
 __device__ __forceinline__ float act_fwdf(int act, float x) {
   switch (act) {
     case LCAO_ACT_SILU: return siluf(x);
     case LCAO_ACT_SSP: return softplusf_acc(x) - 0.69314718055994530942f;
     case LCAO_ACT_SOFTPLUS: return softplusf_acc(x);
-    case LCAO_ACT_RELU: return fmaxf(x, 0.0f);
+    case LCAO_ACT_RELU: return x < 0.0f ? 0.0f : x;
     case LCAO_ACT_TANH: return tanhf(x);
     case LCAO_ACT_SIGMOID: return sigmoidf_acc(x);
     case LCAO_ACT_GELU: return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f));
@@ -97,7 +98,7 @@ __device__ __forceinline__ float act_gradf(int act, float x) {
     case LCAO_ACT_SILU: return silu_gradf(x);
     case LCAO_ACT_SSP:
     case LCAO_ACT_SOFTPLUS: return x > 20.0f ? 1.0f : sigmoidf_acc(x);
-    case LCAO_ACT_RELU: return x > 0.0f ? 1.0f : 0.0f;
+    case LCAO_ACT_RELU: return x <= 0.0f ? 0.0f : 1.0f;
     case LCAO_ACT_TANH: { const float t = tanhf(x); return 1.0f - t * t; }
     case LCAO_ACT_SIGMOID: { const float s = sigmoidf_acc(x); return s * (1.0f - s); }
     case LCAO_ACT_GELU:

@@ -499,8 +499,10 @@ extern "C" int lcao_edge_pair_fwd(const float* a, int64_t lda, const float* b, i
                                   float* out, float* pre, void* stream) {
   if (E == 0) return LCAO_OK;
   LCAO_REQUIRE(a && b && src32 && dst32 && out, "lcao_edge_pair_fwd: null buffer");
-  LCAO_REQUIRE(C % 4 == 0 && lda % 4 == 0 && ldb % 4 == 0 && aligned16(a) && aligned16(b) && aligned16(out),
+  LCAO_REQUIRE(C % 4 == 0 && lda % 4 == 0 && ldb % 4 == 0 && aligned16(a) && aligned16(b) && aligned16(out) &&
+                   (!bias || aligned16(bias)) && (!pre || aligned16(pre)),
                "lcao_edge_pair_fwd: need C, lda, ldb multiples of 4 and 16-byte aligned buffers");
+  LCAO_REQUIRE(act >= LCAO_ACT_NONE && act <= LCAO_ACT_LAST, "lcao_edge_pair_fwd: unsupported activation %d", act);
   if (act == LCAO_ACT_NONE || act == LCAO_ACT_SILU)
     LCAO_CUDA(launch_pdl(k_edge_pair_fwd<false>, (unsigned)ceil_div64(E, kWarpsPerCta), kWarpsPerCta * 32, 0, (cudaStream_t)stream, 
         a, lda, b, ldb, bias, src32, dst32, E, C, act, out, pre));
@@ -514,6 +516,10 @@ extern "C" int lcao_edge_pair_fwd(const float* a, int64_t lda, const float* b, i
 extern "C" int lcao_segment_sum(const float* x, int64_t ldx, const float* y, int64_t ldy, const int32_t* ptr,
                                 const int32_t* perm, int64_t R, int32_t C, int32_t mean, float* out, int64_t ldo,
                                 void* stream) {
+  // flag bits 0, 1, 2 and 4-7 only; act(y) (bit 1) and act'(y) (bit 2) exclude each other and need y when there are
+  // items (x given)
+  LCAO_REQUIRE((mean & ~0xF7) == 0 && (mean & 6) != 6 && (!(mean & 6) || y || !x),
+               "lcao_segment_sum: bad flag word 0x%x (defined bits 0, 1, 2, 4-7; bits 1 and 2 exclusive, each needs y)", mean);
   if (R == 0 || C == 0) return LCAO_OK;
   // x may be NULL when there are no items at all (an edge-less batch): every segment is empty and out is zero-filled
   LCAO_REQUIRE(ptr && out, "lcao_segment_sum: null buffer");
@@ -565,6 +571,7 @@ extern "C" int lcao_act_bwd(const float* dY, int64_t ldy, const float* H, int64_
                             int64_t M, int32_t C, int32_t act, void* stream) {
   if (M == 0 || C == 0) return LCAO_OK;
   LCAO_REQUIRE(dY && dH && (act == LCAO_ACT_NONE || H), "lcao_act_bwd: null buffer");
+  LCAO_REQUIRE(act >= LCAO_ACT_NONE && act <= LCAO_ACT_LAST, "lcao_act_bwd: unsupported activation %d", act);
   const bool vec = C % 4 == 0 && ldy % 4 == 0 && ldd % 4 == 0 && aligned16(dY) && aligned16(dH) &&
                    (act == LCAO_ACT_NONE || (ldh % 4 == 0 && aligned16(H)));
   if (!vec) {

@@ -114,3 +114,27 @@ def test_edge_basis_rejects_unaligned_rows_and_unknown_kinds():
         sp.cutoff_kind, sp.rbf_kind = cut, rbf
         rc = lib.lcao_geom_basis_fwd(a, a, a, None, a, a, E, ctypes.byref(sp), a, a, a, None, None)
         assert rc == -1 and b"unknown" in lib.lcao_last_error(), (cut, rbf)
+
+
+@pytest.mark.skipif(torch.cuda.is_available(), reason="without the check, a GPU would run the kernels on these addresses")
+def test_message_entry_points_reject_bad_flags_activations_and_alignment():
+    # pointer values only: every case must be refused before the first launch
+    lib = _lib.load()
+    a, odd = 16, 4
+    R, C = 4, 128
+    for mode, y in ((2 | 4, a), (2, None), (4, None), (4 | (5 << 4), None), (8, a), (1 << 8, a), (1 << 12, a), (-1, a)):
+        rc = lib.lcao_segment_sum(a, C, y, C, a, a, R, C, mode, a, C, None)
+        assert rc == -1 and b"flag word" in lib.lcao_last_error(), (mode, y)
+    # an edge-less batch passes neither x nor y: nothing is read, so bit 1 or 2 is accepted (it then fails at the launch)
+    rc = lib.lcao_segment_sum(None, C, None, C, a, a, R, C, 2 | (1 << 4), a, C, None)
+    assert b"flag word" not in lib.lcao_last_error()
+    E = 64
+    for bias, pre in ((odd, a), (a, odd), (odd, None)):
+        rc = lib.lcao_edge_pair_fwd(a, C, a, C, bias, a, a, E, C, 1, a, pre, None)
+        assert rc == -1 and b"aligned" in lib.lcao_last_error(), (bias, pre)
+    for act in (-1, 10, 1 << 20):
+        rc = lib.lcao_edge_pair_fwd(a, C, a, C, a, a, a, E, C, act, a, a, None)
+        assert rc == -1 and b"activation" in lib.lcao_last_error(), act
+        for width in (C, 127):   # the vector and the any-alignment kernel
+            rc = lib.lcao_act_bwd(a, width, a, width, a, width, R, width, act, None)
+            assert rc == -1 and b"activation" in lib.lcao_last_error(), (act, width)
