@@ -156,6 +156,18 @@ int lcao_geom_cell_bwd(const float* pos, const float* shift, const float* lattic
                        const int32_t* dst32, const float* dvec, int64_t E, int64_t N, const int32_t* out_ptr,
                        const int32_t* out_edge, const int32_t* seg_ptr, const int32_t* seg_perm, int64_t B,
                        double* scratch, float* d_lattice, float* virial, void* stream);
+/* Per-atom virials from the same dvec (E,3) = d E / d vec, with vec_e as above:
+ *   atom_virial[i][a][c] = 1/2 sum_{e: s_e = i} vec_e[a] dvec_e[c] + 1/2 sum_{e: t_e = i} vec_e[a] dvec_e[c]    (N,3,3)
+ * = d E / d eps_i for a per-atom strain eps acting on the edges as vec_e -> vec_e + 1/2 vec_e (eps_s + eps_t); the rows
+ * of a graph sum to its virial (lcao_geom_cell_bwd), and a self-image edge (s = t) gives its atom 1/2 + 1/2.  Energy units
+ * (not divided by a volume).  One warp per node over its out-CSR then in-CSR edges (in_src = src32[in_edge], as
+ * lcao_graph_index_build writes it), any degree; vec is recomputed in FP64 by the same code as in lcao_geom_cell_bwd, the
+ * nine sums are accumulated in FP64 and rounded once, without atomics (bitwise reproducible).  batch (N, nullable = all
+ * graph 0) selects the lattice row of an edge's source.  Atoms without edges, and all atoms when E == 0, get zeros. */
+int lcao_geom_atom_virial_bwd(const float* pos, const float* shift, const float* lattice, const int64_t* batch,
+                              const int32_t* dst32, const int32_t* in_ptr, const int32_t* in_edge, const int32_t* in_src,
+                              const int32_t* out_ptr, const int32_t* out_edge, const float* dvec, int64_t E, int64_t N,
+                              float* atom_virial, void* stream);
 
 /* ---- orbital contraction (the einsum "ed,edh->eh" sites lcaonet.py:180-183,200-203) ----------- */
 /* B[e,l,:]  = sum_{o: l(o)=l} rb[e,o] * (A[e,o,:] + m[e,o] V[e,o,:])        l = 0..NL-1

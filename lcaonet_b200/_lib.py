@@ -48,6 +48,7 @@ SIGNATURES = {
     "lcao_geom_basis_fwd": [_p, _p, _p, _p, _p, _p, _i64, C.POINTER(BasisSpec), _p, _p, _p, _p, _p],
     "lcao_geom_basis_bwd": [_p, _p, _p, _p, _p, _p, _i64, _i64, _i32, _p, _p, _p, _p, _p, _p, _p],
     "lcao_geom_cell_bwd": [_p, _p, _p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p, _i64, _p, _p, _p, _p],
+    "lcao_geom_atom_virial_bwd": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i64, _p, _p],
     "lcao_coeff_contract_fwd": [_p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32, _p, _p],
     "lcao_coeff_contract_bwd": [_p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32, _p, _p, _p],
     "lcao_pair_contract_fwd": [_p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32, _p, _p, _p, _p],

@@ -112,7 +112,8 @@ __global__ void k_geom_node_bwd(const float* __restrict__ dvec, const int32_t* _
   d_pos[idx] = acc;
 }
 
-// ---- cell derivatives: d E / d lattice and the virial, per graph (lcao_geom_cell_bwd).
+// ---- cell derivatives: d E / d lattice and the virial, per graph (lcao_geom_cell_bwd), and the per-atom virials
+// (lcao_geom_atom_virial_bwd).
 // A graph's nodes (seg_perm[seg_ptr[g] .. seg_ptr[g+1]), or that range itself when seg_perm is NULL) are cut into chunks of
 // LCAO_CELL_CHUNK; chunk j of graph g owns partial slot  seg_ptr[g] / LCAO_CELL_CHUNK + g + j.  These ranges are disjoint
 // (the slots of g end at or before the first slot of g + 1), their union lies in [0, N / LCAO_CELL_CHUNK + B), and a slot
@@ -124,18 +125,90 @@ __device__ __forceinline__ int64_t cell_slot_base(const int32_t* seg_ptr, int g)
   return seg_ptr[g] / LCAO_CELL_CHUNK + g;
 }
 
-// Stage 1: CTA = one chunk; warp w takes the chunk's nodes w, w + 8, ...; lane l the out-edges l, l + 32, ... of each
-// node in out-CSR order.  Every lane accumulates shift (x) dvec and vec (x) dvec in FP64; the lanes are combined by a
-// fixed xor butterfly and the warps in warp order: the partial is a fixed function of the inputs (bitwise reproducible).
-// vec is recomputed in FP64 exactly as k_geom_basis_fwd forms it (not dist * unit: that would carry the FP32 rounding of
-// unit into the virial).
+// vec = pos[t] - pos[s] + shift . L in FP64, formed exactly as k_geom_basis_fwd forms it (not dist * unit: that would carry
+// the FP32 rounding of unit into the virial); ps = pos[s], L = the lattice of the graph of s.  Both virial reductions below
+// form vec here, so the per-atom virials of a graph add up to its virial up to the rounding of the sums.
+__device__ __forceinline__ void edge_vec(const float* __restrict__ pos, int32_t t, const double ps[3], const double sh[3],
+                                         const float* __restrict__ L, double v[3]) {
+#pragma unroll
+  for (int c = 0; c < 3; ++c)
+    v[c] = ((double)pos[3 * t + c] - ps[c]) + (sh[0] * L[c] + sh[1] * L[3 + c] + sh[2] * L[6 + c]);
+}
+
+// Per-atom virial of node n (one warp): W_n = 1/2 sum_{e: s_e = n} vec_e (x) dvec_e + 1/2 sum_{e: t_e = n} vec_e (x) dvec_e.
+// Lane l takes the node's out-edges l, l + 32, ... in out-CSR order, then its in-edges the same way in in-CSR order, so a
+// node of any degree is one warp's loop.  FP64 accumulation, a fixed xor butterfly and one rounding after the 1/2: the row
+// is a fixed function of the inputs (bitwise reproducible), and no atomics.
+__device__ __forceinline__ void atom_virial_row(
+    const float* __restrict__ pos, const float* __restrict__ shift, const float* __restrict__ lattice,
+    const int64_t* __restrict__ batch, const int32_t* __restrict__ dst32, const float* __restrict__ dvec,
+    const int32_t* __restrict__ out_ptr, const int32_t* __restrict__ out_edge, const int32_t* __restrict__ in_ptr,
+    const int32_t* __restrict__ in_edge, const int32_t* __restrict__ in_src, int64_t n, int lane,
+    float* __restrict__ atom_virial) {
+  double acc[9];
+#pragma unroll
+  for (int k = 0; k < 9; ++k) acc[k] = 0.0;
+  const int32_t o0 = out_ptr[n], o1 = out_ptr[n + 1], i0 = in_ptr[n], i1 = in_ptr[n + 1];
+  if (o0 < o1 || i0 < i1) {  // (an atom without edges reads nothing: edge buffers may be NULL when E == 0)
+    const double pn[3] = {pos[3 * n], pos[3 * n + 1], pos[3 * n + 2]};
+    const float* Ln = lattice + 9 * (batch ? batch[n] : 0);
+    for (int32_t p = o0 + lane; p < o1; p += 32) {  // s = n: vec = pos[t] - pos[n] + shift . L[batch[n]]
+      const int64_t e = out_edge[p];
+      const double sh[3] = {shift[3 * e], shift[3 * e + 1], shift[3 * e + 2]};
+      const double dv[3] = {dvec[3 * e], dvec[3 * e + 1], dvec[3 * e + 2]};
+      double v[3];
+      edge_vec(pos, dst32[e], pn, sh, Ln, v);
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) acc[3 * a + c] = fma(v[a], dv[c], acc[3 * a + c]);
+    }
+    for (int32_t p = i0 + lane; p < i1; p += 32) {  // t = n: vec = pos[n] - pos[s] + shift . L[batch[s]]
+      const int64_t e = in_edge[p];
+      const int32_t s = in_src[p];
+      const double ps[3] = {pos[3 * s], pos[3 * s + 1], pos[3 * s + 2]};
+      const double sh[3] = {shift[3 * e], shift[3 * e + 1], shift[3 * e + 2]};
+      const double dv[3] = {dvec[3 * e], dvec[3 * e + 1], dvec[3 * e + 2]};
+      double v[3];
+      edge_vec(pos, (int32_t)n, ps, sh, lattice + 9 * (batch ? batch[s] : 0), v);
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) acc[3 * a + c] = fma(v[a], dv[c], acc[3 * a + c]);
+    }
+  }
+  float out = 0.f;
+#pragma unroll
+  for (int k = 0; k < 9; ++k) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+    if (lane == k) out = (float)(0.5 * acc[k]);
+  }
+  if (lane < 9) atom_virial[9 * n + lane] = out;
+}
+
+// Two reductions of the same dvec, with the same vec (edge_vec), in one kernel:
+//  - atom_virial != NULL (lcao_geom_atom_virial_bwd): warp w of CTA b is node 8 b + w (atom_virial_row); the cell arguments
+//    (seg_ptr, seg_perm, B, partial) are unused.
+//  - otherwise, stage 1 of lcao_geom_cell_bwd: CTA = one chunk; warp w takes the chunk's nodes w, w + 8, ...; lane l the
+//    out-edges l, l + 32, ... of each node in out-CSR order.  Every lane accumulates shift (x) dvec and vec (x) dvec in
+//    FP64; the lanes are combined by a fixed xor butterfly and the warps in warp order: the partial is a fixed function of
+//    the inputs (bitwise reproducible).
 __global__ void __launch_bounds__(kCellWarps * 32) k_geom_cell_partial(
     const float* __restrict__ pos, const float* __restrict__ shift, const float* __restrict__ lattice,
     const int64_t* __restrict__ batch, const int32_t* __restrict__ dst32, const float* __restrict__ dvec,
     const int32_t* __restrict__ out_ptr, const int32_t* __restrict__ out_edge, const int32_t* __restrict__ seg_ptr,
-    const int32_t* __restrict__ seg_perm, int B, double* __restrict__ partial) {
+    const int32_t* __restrict__ seg_perm, int B, double* __restrict__ partial, const int32_t* __restrict__ in_ptr,
+    const int32_t* __restrict__ in_edge, const int32_t* __restrict__ in_src, int64_t N, float* __restrict__ atom_virial) {
   pdl_trigger();  // (programmatic dependent launch: the next kernel may start its set-up; common.cuh)
   pdl_wait();     // launched through launch_pdl: nothing of the stream's earlier work is touched before this
+  if (atom_virial) {
+    const int64_t n = blockIdx.x * (int64_t)kCellWarps + (threadIdx.x >> 5);
+    if (n < N)
+      atom_virial_row(pos, shift, lattice, batch, dst32, dvec, out_ptr, out_edge, in_ptr, in_edge, in_src, n,
+                      threadIdx.x & 31, atom_virial);
+    return;
+  }
   __shared__ double s_red[kCellWarps][kCellVals];
   const int64_t slot = blockIdx.x;
   int lo = 0, hi = B;  // the graph: last g with cell_slot_base(g) <= slot (strictly increasing in g)
@@ -164,9 +237,7 @@ __global__ void __launch_bounds__(kCellWarps * 32) k_geom_cell_partial(
       const double ps[3] = {ps0, ps1, ps2};
       const double dv[3] = {dvec[3 * e], dvec[3 * e + 1], dvec[3 * e + 2]};
       double v[3];
-#pragma unroll
-      for (int c = 0; c < 3; ++c)
-        v[c] = ((double)pos[3 * t + c] - ps[c]) + (sh[0] * L[c] + sh[1] * L[3 + c] + sh[2] * L[6 + c]);
+      edge_vec(pos, t, ps, sh, L, v);
 #pragma unroll
       for (int a = 0; a < 3; ++a)
 #pragma unroll
@@ -268,10 +339,28 @@ extern "C" int lcao_geom_cell_bwd(const float* pos, const float* shift, const fl
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t slots = N / LCAO_CELL_CHUNK + B;
   LCAO_CUDA(launch_pdl(k_geom_cell_partial, (unsigned)slots, kCellWarps * 32, 0, st, pos, shift, lattice, batch, dst32, dvec,
-                       out_ptr, out_edge, seg_ptr, seg_perm, (int)B, scratch));
+                       out_ptr, out_edge, seg_ptr, seg_perm, (int)B, scratch, (const int32_t*)nullptr,
+                       (const int32_t*)nullptr, (const int32_t*)nullptr, (int64_t)0, (float*)nullptr));
   LCAO_LAUNCH_CHECK();
   LCAO_CUDA(launch_pdl(k_geom_cell_final, (unsigned)ceil_div64(B, kCellWarps), kCellWarps * 32, 0, st, seg_ptr, (int)B,
                        (const double*)scratch, d_lattice, virial));
+  LCAO_LAUNCH_CHECK();
+  return LCAO_OK;
+}
+
+extern "C" int lcao_geom_atom_virial_bwd(const float* pos, const float* shift, const float* lattice, const int64_t* batch,
+                                         const int32_t* dst32, const int32_t* in_ptr, const int32_t* in_edge,
+                                         const int32_t* in_src, const int32_t* out_ptr, const int32_t* out_edge,
+                                         const float* dvec, int64_t E, int64_t N, float* atom_virial, void* stream) {
+  LCAO_REQUIRE(N >= 0 && N < ((int64_t)1 << 31) && E >= 0 && E < ((int64_t)1 << 31),
+               "lcao_geom_atom_virial_bwd: bad sizes (N=%lld, E=%lld)", (long long)N, (long long)E);
+  if (N == 0) return LCAO_OK;
+  LCAO_REQUIRE(in_ptr && out_ptr && atom_virial, "lcao_geom_atom_virial_bwd: null buffer");
+  LCAO_REQUIRE(E == 0 || (pos && shift && lattice && dst32 && in_edge && in_src && out_edge && dvec),
+               "lcao_geom_atom_virial_bwd: null edge buffer");
+  LCAO_CUDA(launch_pdl(k_geom_cell_partial, (unsigned)ceil_div64(N, kCellWarps), kCellWarps * 32, 0, (cudaStream_t)stream,
+                       pos, shift, lattice, batch, dst32, dvec, out_ptr, out_edge, (const int32_t*)nullptr,
+                       (const int32_t*)nullptr, 0, (double*)nullptr, in_ptr, in_edge, in_src, N, atom_virial));
   LCAO_LAUNCH_CHECK();
   return LCAO_OK;
 }

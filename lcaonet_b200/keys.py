@@ -26,5 +26,9 @@ class GraphKeys:
     Edge_idx_st_3b = "edge_idx_st_3b"  # (T)
     Angles_3b = "angles_3b"  # (T) cos(theta)
 
+    # written by LCAONet.forward when regress_atom_energy / regress_atom_virial is set (no reference counterpart)
+    Atom_energy = "atom_energy"  # (N, out_size)
+    Atom_virial = "atom_virial"  # (N, 3, 3), or (N, out_size, 3, 3)
+
 
 KEYS = [v for k, v in vars(GraphKeys).items() if not k.startswith("__")]

@@ -412,8 +412,13 @@ class LCAOOut(nn.Module):
                                                Dense(emb_size, emb_size // 2, True, weight_init), activation,
                                                Dense(emb_size // 2, 1, False, weight_init))
 
-    def forward(self, x, seg, gi, unit, pos, strain=None, lattice=None):
-        prop = ops.segment_reduce(_mlp(self.out_lin, x), *seg, mean=not self.is_extensive)
+    def forward(self, x, seg, gi, unit, pos, strain=None, lattice=None, atom_strain=None, atom_out=None):
+        """`atom_out` (a dict, optional) receives the per-node rows of out_lin under "energy" and, with the (N,3,3) probe
+        `atom_strain` (autograd forces only), the per-atom virials d E / d atom_strain under "virial" (ops.geom_basis)."""
+        e = _mlp(self.out_lin, x)
+        if atom_out is not None:
+            atom_out["energy"] = e
+        prop = ops.segment_reduce(e, *seg, mean=not self.is_extensive)
         if not self.regress_forces:
             return prop
         if self.direct_forces:
@@ -437,21 +442,28 @@ class LCAOOut(nn.Module):
         # pass: the backward kernels skip every parameter gradient inside it (ops.positions_only).
         graph = self.training if self.force_training is None else bool(self.force_training)
         graph = graph and torch.is_grad_enabled()
-        if strain is None:
+        if strain is None and atom_strain is None:
             with ops.positions_only():
                 cols = [-torch.autograd.grad(prop[:, i].sum(), pos, create_graph=graph, retain_graph=True)[0]
                         for i in range(self.out_size)]
             return prop, (cols[0] if len(cols) == 1 else torch.stack(cols, dim=1).squeeze(1))
-        # stress (LCAONet.regress_stress): the same backward pass also yields d E / d strain = the virial W (ops.geom_basis)
+        # stress (LCAONet.regress_stress) and per-atom virials (LCAONet.regress_atom_virial): the same backward pass also
+        # yields d E / d strain = the virial W and d E / d atom_strain = the per-atom virials W_i (ops.geom_basis)
+        probes = [p for p in (strain, atom_strain) if p is not None]
         with ops.positions_only():
-            grads = [torch.autograd.grad(prop[:, i].sum(), [pos, strain], create_graph=graph, retain_graph=True)
+            grads = [torch.autograd.grad(prop[:, i].sum(), [pos, *probes], create_graph=graph, retain_graph=True)
                      for i in range(self.out_size)]
         cols = [-g[0] for g in grads]
+        forces = cols[0] if len(cols) == 1 else torch.stack(cols, dim=1).squeeze(1)
+        if atom_strain is not None:
+            w = [g[-1] for g in grads]
+            atom_out["virial"] = w[0] if len(w) == 1 else torch.stack(w, dim=1)
+        if strain is None:
+            return prop, forces
         L = lattice[: strain.shape[0]].double()
         vol = (L[:, 0] * torch.linalg.cross(L[:, 1], L[:, 2], dim=-1)).sum(-1).abs().to(grads[0][1].dtype)
         sig = [g[1] / vol.view(-1, 1, 1) for g in grads]
-        return (prop, (cols[0] if len(cols) == 1 else torch.stack(cols, dim=1).squeeze(1)),
-                (sig[0] if len(sig) == 1 else torch.stack(sig, dim=1)))
+        return prop, forces, (sig[0] if len(sig) == 1 else torch.stack(sig, dim=1))
 
 
 class PostProcess(nn.Module):
@@ -474,6 +486,15 @@ class PostProcess(nn.Module):
                 m = cnt * m
             out = out + m
         return (out, *rest) if rest else out
+
+    def atom_energy(self, e, z):
+        """per-atom energies e_i = out_lin(x_i) + atomref[z_i] + mean (each offset only if set): `forward` gives their sum
+        per graph (is_extensive) or their mean (otherwise)."""
+        if self.atomref is not None:
+            e = e + self.atomref[z].to(torch.float32)
+        if self.mean is not None:
+            e = e + self.mean.unsqueeze(0)
+        return e
 
 
 # ----------------------------------------------------------------------------------------------
@@ -618,6 +639,17 @@ class LCAONet(nn.Module):
         # autograd forces: forward returns (energy, forces, stress), stress in energy units per A^3, not symmetrised; a cell
         # of zero volume gives non-finite rows.  Needs regress_forces=True, direct_forces=False.
         self.regress_stress = False
+        # write the per-atom energies  e_i = out_lin(x_i) + atomref[z_i] + mean  (N, out_size) into the batch under
+        # GraphKeys.Atom_energy (ASE's get_potential_energies, LAMMPS compute pe/atom): the energy is their sum per graph
+        # (is_extensive) or their mean.  Any model configuration; the return value of forward does not change.
+        self.regress_atom_energy = False
+        # write the per-atom virials  W_i = 1/2 sum_{e: s_e = i} vec_e (x) dvec_e + 1/2 sum_{e: t_e = i} vec_e (x) dvec_e,
+        # dvec_e = d E / d vec_e, into the batch under GraphKeys.Atom_virial: (N,3,3), or (N,out_size,3,3) when out_size > 1,
+        # same index order as the virial behind the stress, not symmetrised.  They sum per graph to that virial, i.e. to
+        # stress_g |det L_g|.  Energy units, not divided by a volume, so defined for molecules too: ASE's per-atom stresses
+        # (get_stresses) are W_i / |det L_g|.  Computed in the same backward pass as the forces (trainable in training mode,
+        # like the stress).  Needs regress_forces=True, direct_forces=False.
+        self.regress_atom_virial = False
 
         elec_info = ElecInfo(max_z, max_orb, min_orb, n_per_orb)
         if elec_info.n_orb > 64:
@@ -674,6 +706,9 @@ class LCAONet(nn.Module):
         if self.regress_stress and not autograd_forces:
             raise ValueError("regress_stress needs autograd forces: construct the model with regress_forces=True, "
                              "direct_forces=False")
+        if self.regress_atom_virial and not autograd_forces:
+            raise ValueError("regress_atom_virial needs autograd forces: construct the model with regress_forces=True, "
+                             "direct_forces=False")
         if autograd_forces:
             graph[GraphKeys.Pos].requires_grad_(True)
         batch_idx = graph.get(GraphKeys.Batch_idx)
@@ -697,8 +732,11 @@ class LCAONet(nn.Module):
         # stress: a zero strain per graph whose gradient is the virial (ops.geom_basis)
         strain = (torch.zeros(seg[0].numel() - 1, 3, 3, device=pos.device, requires_grad=True) if self.regress_stress
                   else None)
+        # per-atom virials: a zero strain per atom whose gradient is W_i (ops.geom_basis)
+        atom_strain = torch.zeros(N, 3, 3, device=pos.device, requires_grad=True) if self.regress_atom_virial else None
         # geometry + radial basis in one kernel (base.py:27-43, rbf.py:129-142)
-        dist, unit, rb = ops.geom_basis(pos, shift, lattice, batch_idx, gi, self.rbf.spec, self.rbf.n_orb, strain, seg[:2])
+        dist, unit, rb = ops.geom_basis(pos, shift, lattice, batch_idx, gi, self.rbf.spec, self.rbf.n_orb, strain, seg[:2],
+                                        atom_strain)
         graph[GraphKeys.Edge_dist], graph[GraphKeys.Edge_vec_st] = dist, unit
         if self.side_effect_keys:
             k, e_ks, e_st, cos = gi.triplets(unit.detach())
@@ -709,5 +747,10 @@ class LCAONet(nn.Module):
         vmask = self.valence_mask(z, idx_t) if self.add_valence else None
         for layer in self.int_layers:
             x = layer(x, cst, vmask, rb, unit, gi, self._lgrp, self._n_l)
-        out = self.out_layer(x, seg, gi, unit, pos, strain, lattice)
+        atom = {} if (self.regress_atom_energy or self.regress_atom_virial) else None
+        out = self.out_layer(x, seg, gi, unit, pos, strain, lattice, atom_strain, atom)
+        if self.regress_atom_energy:
+            graph[GraphKeys.Atom_energy] = self.pp_layer.atom_energy(atom["energy"], z)
+        if self.regress_atom_virial:
+            graph[GraphKeys.Atom_virial] = atom["virial"]
         return self.pp_layer(out, z, seg)

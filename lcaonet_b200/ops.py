@@ -164,7 +164,7 @@ def histogram(keys: Tensor, n_buckets: int) -> Tensor:
 # ------------------------------------------------------------------------------------------------
 class _GeomBasis(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, pos, shift, lattice, batch, gi: GraphIndex, spec, n_orb: int, strain=None, seg=None):
+    def forward(ctx, pos, shift, lattice, batch, gi: GraphIndex, spec, n_orb: int, strain=None, seg=None, atom_strain=None):
         require_cuda(pos, shift, lattice)
         pos_c, shift_c, lat_c = pos.contiguous().float(), shift.contiguous().float(), lattice.contiguous().float()
         E, dev = gi.E, pos.device
@@ -172,28 +172,29 @@ class _GeomBasis(torch.autograd.Function):
         unit = torch.empty(E, 3, device=dev)
         rb = torch.empty(E, n_orb, device=dev)
         ni = ctx.needs_input_grad
-        need_grad = ni[0] or ni[2] or ni[7]
+        need_grad = ni[0] or ni[2] or ni[7] or ni[9]
         drb = torch.empty(E, n_orb, device=dev) if need_grad else None
         _call("lcao_geom_basis_fwd", ptr(pos_c), ptr(shift_c), ptr(lat_c), ptr(batch), ptr(gi.src32), ptr(gi.dst32), E,
               ctypes.byref(spec), ptr(dist), ptr(unit), ptr(rb), ptr(drb), stream_ptr())
         ctx.gi, ctx.n_orb, ctx.spec, ctx.seg = gi, n_orb, spec, seg
-        ctx.save_for_backward(dist, unit, drb, pos, shift, lattice, batch, strain)
+        ctx.save_for_backward(dist, unit, drb, pos, shift, lattice, batch, strain, atom_strain)
         return dist, unit, rb
 
     @staticmethod
     def backward(ctx, d_dist, d_unit, d_rb):
-        dist, unit, drb, pos, shift, lattice, batch, strain = ctx.saved_tensors
+        dist, unit, drb, pos, shift, lattice, batch, strain, atom_strain = ctx.saved_tensors
         gi = ctx.gi
         if drb is None:
-            return (None,) * 9
+            return (None,) * 10
         ni = ctx.needs_input_grad
         if torch.is_grad_enabled():  # create_graph=True: this backward is itself differentiated (training on autograd forces)
             with torch.enable_grad():
-                pos_, lat_, strain_ = second_order.aliases([pos, lattice, strain])
-                outs = second_order.geom_basis(pos_, shift, lat_, batch, gi.src32, gi.dst32, ctx.spec, ctx.n_orb, strain_)
-                d_pos, d_lat, d_strain = second_order.grads_with_graph(outs, [pos_, lat_, strain_], [d_dist, d_unit, d_rb],
-                                                                       [ni[0], ni[2], ni[7]])
-            return d_pos, None, d_lat, None, None, None, None, d_strain, None
+                pos_, lat_, strain_, astrain_ = second_order.aliases([pos, lattice, strain, atom_strain])
+                outs = second_order.geom_basis(pos_, shift, lat_, batch, gi.src32, gi.dst32, ctx.spec, ctx.n_orb, strain_,
+                                               astrain_)
+                d_pos, d_lat, d_strain, d_astrain = second_order.grads_with_graph(
+                    outs, [pos_, lat_, strain_, astrain_], [d_dist, d_unit, d_rb], [ni[0], ni[2], ni[7], ni[9]])
+            return d_pos, None, d_lat, None, None, None, None, d_strain, None, d_astrain
         dev = dist.device
         dvec = torch.empty(gi.E, 3, device=dev)
         d_pos = torch.empty(gi.N, 3, device=dev)
@@ -202,10 +203,12 @@ class _GeomBasis(torch.autograd.Function):
         _call("lcao_geom_basis_bwd", ptr(dist), ptr(unit), ptr(drb), ptr(d_dist), ptr(d_unit), ptr(d_rb), gi.E, gi.N,
               ctx.n_orb, ptr(gi.in_ptr), ptr(gi.in_edge), ptr(gi.out_ptr), ptr(gi.out_edge), ptr(dvec), ptr(d_pos),
               stream_ptr())
-        d_lat = d_strain = None
+        d_lat = d_strain = d_astrain = None
         if ni[2] or ni[7]:
             d_lat, d_strain = _cell_grads(dvec, pos, shift, lattice, batch, gi, ctx.seg, ni[2], ni[7])
-        return d_pos if ni[0] else None, None, d_lat, None, None, None, None, d_strain, None
+        if ni[9]:
+            d_astrain = _atom_virial(dvec, pos, shift, lattice, batch, gi)
+        return d_pos if ni[0] else None, None, d_lat, None, None, None, None, d_strain, None, d_astrain
 
 
 def _cell_grads(dvec, pos, shift, lattice, batch, gi, seg, want_lattice: bool, want_virial: bool):
@@ -231,15 +234,28 @@ def _cell_grads(dvec, pos, shift, lattice, batch, gi, seg, want_lattice: bool, w
     return d_lat, virial
 
 
-def geom_basis(pos, shift, lattice, batch, gi, spec, n_orb, strain=None, seg=None):
+def _atom_virial(dvec, pos, shift, lattice, batch, gi):
+    """(N,3,3) per-atom virials W_i = 1/2 sum of vec_e (x) dvec_e over the edges with s_e = i and over those with t_e = i,
+    from dvec = d E / d vec (lcao_geom_atom_virial_bwd)."""
+    out = torch.empty(gi.N, 3, 3, device=dvec.device)
+    pos_c, shift_c, lat_c = pos.contiguous().float(), shift.contiguous().float(), lattice.contiguous().float()
+    _call("lcao_geom_atom_virial_bwd", ptr(pos_c), ptr(shift_c), ptr(lat_c), ptr(batch), ptr(gi.dst32), ptr(gi.in_ptr),
+          ptr(gi.in_edge), ptr(gi.in_src), ptr(gi.out_ptr), ptr(gi.out_edge), ptr(dvec), gi.E, gi.N, ptr(out), stream_ptr())
+    return out
+
+
+def geom_basis(pos, shift, lattice, batch, gi, spec, n_orb, strain=None, seg=None, atom_strain=None):
     """(dist, unit, rb) of every edge, vec_e = pos[t] - pos[s] + shift_e . lattice[batch[s]] (row vectors, base.py:27-43).
     Differentiable with respect to `pos` and `lattice` (d E / d L_g[i][j] = sum_{e in g} shift_e[i] dvec_e[j]); the
     gradient with respect to `shift` is not computed (None).
     `strain` (internal, not public API: LCAONet.regress_stress creates it) is a (B,3,3) gradient probe: zeros with
     requires_grad whose value the forward never reads, standing for eps_g in pos' = pos (I + eps), L' = L (I + eps).  Its
     gradient is the virial W_g = sum_{e in g} vec_e (x) dvec_e.  `seg` = (seg_ptr, seg_perm), the nodes grouped by
-    graph (optional: built from `batch` when a cell gradient is wanted and it is missing)."""
-    return _GeomBasis.apply(pos, shift, lattice, batch, gi, spec, n_orb, strain, seg)
+    graph (optional: built from `batch` when a cell gradient is wanted and it is missing).
+    `atom_strain` (internal, like `strain`: LCAONet.regress_atom_virial creates it) is an (N,3,3) probe eps_i acting on the
+    edges as vec_e -> vec_e + 1/2 vec_e (eps_s + eps_t).  Its gradient is the per-atom virial
+    W_i = 1/2 sum_{e: s_e = i} vec_e (x) dvec_e + 1/2 sum_{e: t_e = i} vec_e (x) dvec_e."""
+    return _GeomBasis.apply(pos, shift, lattice, batch, gi, spec, n_orb, strain, seg, atom_strain)
 
 
 # ------------------------------------------------------------------------------------------------
